@@ -291,6 +291,42 @@ int rua_segment_reduce_backward(const void* grad_out, const void* out, const voi
                                 rua_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------- */
+/* K7  per-sequence prefix scans (no counterpart in the reference; replaces the pad -> ATen scan  */
+/* along dim 1 -> unpad composition a user would write with to_left / torch.cumsum / to_cat)     */
+/* ------------------------------------------------------------------------------------------- */
+enum rua_scan { RUA_SCAN_SUM = 0, RUA_SCAN_LOGSUMEXP = 1, RUA_SCAN_MAX = 2, RUA_SCAN_MIN = 3 };
+
+/* workspace of rua_segment_scan (backward = 0) / rua_segment_scan_backward (backward = 1) over side->rows = rows rows of
+ * H elements; 0 when there is nothing to do or an argument is invalid. */
+size_t rua_segment_scan_workspace_bytes(int64_t rows, int64_t H, int32_t dtype, int32_t op, int32_t backward);
+
+/* src / dst: side->rows rows of H elements in the storage of `side` (C, L, P or R over `ragged`; len_xform must be
+ * RUA_LEN_SAME).  For token (i, t) of sequence i with length len[i] (rows from the "Row of token" formulas above):
+ *   dst(i, t) = op over src(i, 0..t)             (reverse = 0)
+ *   dst(i, t) = op over src(i, t..len[i]-1)      (reverse = 1)
+ * op = max / min also writes idx_out (same shape, int64): the position within the sequence of the selected element,
+ * ties to the later position in scan order, a NaN sticks with its own position (torch.cummax / cummin).  Rows that hold
+ * no token (L / R padding, C rows at or past off[B]) are copied through, with index 0.  max / min: side->rows < 2^31
+ * (RUA_ERR_UNSUPPORTED otherwise).  fp32 accumulation (fp64 for
+ * RUA_F64), one rounding.  Deterministic: chunk carries are combined in chunk order, never in arrival order.
+ * ws: rua_segment_scan_workspace_bytes(side->rows, H, dtype, op, 0) bytes; it is cleared by a memset on `stream`. */
+int rua_segment_scan(const void* src, void* dst, int64_t* idx_out, int64_t H, int32_t dtype, int32_t op,
+                     int32_t reverse, const rua_ragged_t* ragged, const rua_side_t* side, void* ws, size_t ws_bytes,
+                     rua_stream_t stream);
+
+/* gradient of rua_segment_scan with the same op / reverse / ragged / side: grad_in = d(loss)/d(src) from grad_out.
+ *   sum: the scan of grad_out in the other direction;
+ *   logsumexp: x = the forward input, y = the forward output; grad_in = exp(x - y) * v with v the reverse affine scan
+ *              v_k = g_k + exp(y_k - y_next) v_next (exponents <= 0); 0 where x = -inf (torch gives NaN for a leading
+ *              -inf);
+ *   max / min: idx = the forward indices; grad_in(k) = sum of grad_out(j) over the positions j whose index is k.
+ * Arguments an op does not use may be NULL.  Rows that hold no token pass grad_out through.  Every row of grad_in is
+ * written.  ws: rua_segment_scan_workspace_bytes(side->rows, H, dtype, op, 1) bytes. */
+int rua_segment_scan_backward(const void* grad_out, const void* x, const void* y, const int64_t* idx, void* grad_in,
+                              int64_t H, int32_t dtype, int32_t op, int32_t reverse, const rua_ragged_t* ragged,
+                              const rua_side_t* side, void* ws, size_t ws_bytes, rua_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------- */
 /* K5  multi-GPU output gather over NVLink peer memory (SURVEY.md 8e-3; the reference is         */
 /* single-device).  One process per GPU; the batch is sharded by sequence; every rank stores its */
 /* rows directly into the output buffers ("windows") of all ranks of the node.                   */

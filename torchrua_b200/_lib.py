@@ -17,6 +17,7 @@ MAP_SHIFT, MAP_REV, MAP_ROLL = 0, 1, 2
 PAD_FILL, PAD_ROW0, PAD_WRAP = 0, 1, 2
 F32, F64, F16, BF16 = 0, 1, 2, 3
 SUM, MEAN, PROD, MAX, MIN, LOGSUMEXP = 0, 1, 2, 3, 4, 5
+SCAN_SUM, SCAN_LOGSUMEXP, SCAN_MAX, SCAN_MIN = 0, 1, 2, 3
 
 
 class Ragged(Structure):
@@ -76,6 +77,11 @@ SIGNATURES = {
     'rua_segment_reduce_backward_workspace_bytes': (c_size_t, [c_int64, c_int64, c_int64, c_int32, c_int32]),
     'rua_segment_reduce_backward': (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64,
                                               c_int32, c_int32, c_void_p, c_void_p, c_size_t, c_void_p]),
+    'rua_segment_scan_workspace_bytes': (c_size_t, [c_int64, c_int64, c_int32, c_int32, c_int32]),
+    'rua_segment_scan': (c_int32, [c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, POINTER(Ragged),
+                                   POINTER(Side), c_void_p, c_size_t, c_void_p]),
+    'rua_segment_scan_backward': (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32,
+                                            c_int32, POINTER(Ragged), POINTER(Side), c_void_p, c_size_t, c_void_p]),
     'rua_peer_window_alloc': (c_int32, [c_size_t, POINTER(c_void_p), c_char_p]),
     'rua_peer_window_open': (c_int32, [c_char_p, POINTER(c_void_p)]),
     'rua_peer_window_close': (c_int32, [c_void_p]),

@@ -1081,7 +1081,9 @@ _STRICT_OPS = (_lib.SUM, _lib.MEAN, _lib.PROD)
 class strict_reductions:
     """``with strict_reductions():`` -- segment_sum / segment_mean / segment_prod (and .seg(...) through them)
     return exactly the bits of the reference; the default fast kernels stay within the stated tolerance of it
-    (fp32 accumulation, one rounding) and are closer to the true value for 16-bit data."""
+    (fp32 accumulation, one rounding) and are closer to the true value for 16-bit data.  The prefix scans
+    (segment_cumsum / logcumsumexp / cummax / cummin and their layout methods) are not affected: they always
+    accumulate in fp32 (fp64 for fp64) with one rounding."""
 
     def __init__(self, enabled: bool = True):
         self.enabled = enabled
@@ -1166,6 +1168,126 @@ def segment_reduce(data: Tensor, segment_sizes: Tensor, op: str) -> Tensor:
     if not (data.requires_grad and torch.is_grad_enabled()):
         return _reduce_raw(data if data.is_contiguous() else data.contiguous(), rg.off, rg.B, _OPS[op])
     return _SegmentReduce.apply(data, rg.off, rg.B, _OPS[op])
+
+
+# ------------------------------------------------------------------------------------------------
+# K6: per-sequence prefix scans (+ autograd)
+# ------------------------------------------------------------------------------------------------
+_SCAN_OPS = {'sum': _lib.SCAN_SUM, 'logsumexp': _lib.SCAN_LOGSUMEXP, 'max': _lib.SCAN_MAX, 'min': _lib.SCAN_MIN}
+
+
+def _scan_check(data: Tensor) -> None:
+    if data.dtype not in _DTYPES:
+        raise RuntimeError(f'torchrua_b200: segment scans support float16/bfloat16/float32/float64, got {data.dtype}')
+
+
+def _scan_raw(data: Tensor, rg: Ragged, side: SideSpec, op: int, reverse: bool):
+    """(out, idx or None) with out laid out like data; data: (side.rows, *feat) contiguous."""
+    lib = _lib.load()
+    H = data[0].numel() if data.shape[0] else 0
+    out = torch.empty_like(data)
+    idx = torch.empty(data.shape, dtype=torch.long, device=data.device) if op in (_lib.SCAN_MAX, _lib.SCAN_MIN) else None
+    if out.numel() == 0:
+        return out, idx
+    dt = _DTYPES[data.dtype]
+    c_rg, c_side = rg.c_struct(), side.c_struct()
+    with _on(data.device):
+        nbytes = lib.rua_segment_scan_workspace_bytes(side.rows, H, dt, op, 0)
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=data.device)
+        prof = _profile_begin()
+        _lib.check(lib.rua_segment_scan(data.data_ptr(), out.data_ptr(), _ptr(idx), H, dt, op, int(reverse),
+                                        ctypes.byref(c_rg), ctypes.byref(c_side), ws.data_ptr(), nbytes, _stream()),
+                   'rua_segment_scan')
+        if prof is not None:
+            # every row read once and written once (+ the int64 indices of max / min) + the metadata consulted
+            nb = 2 * data.numel() * data.element_size() + (8 * data.numel() if idx is not None else 0)
+            _profile_end(prof, 'segment_scan', nb + 8 * rg.B + (8 * (rg.Tp + rg.B) if side.layout == PACK else 0))
+    return out, idx
+
+
+def _scan_backward_raw(g: Tensor, x: Optional[Tensor], y: Optional[Tensor], idx: Optional[Tensor], rg: Ragged,
+                       side: SideSpec, op: int, reverse: bool) -> Tensor:
+    lib = _lib.load()
+    g = g.contiguous()
+    grad = torch.empty_like(g)   # every row is written by the kernel (non-token rows pass grad_out through)
+    if grad.numel() == 0:
+        return grad
+    H = g[0].numel()
+    dt = _DTYPES[g.dtype]
+    c_rg, c_side = rg.c_struct(), side.c_struct()
+    with _on(g.device):
+        nbytes = lib.rua_segment_scan_workspace_bytes(side.rows, H, dt, op, 1)
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=g.device)
+        prof = _profile_begin()
+        _lib.check(lib.rua_segment_scan_backward(g.data_ptr(), _ptr(x), _ptr(y), _ptr(idx), grad.data_ptr(), H, dt, op,
+                                                 int(reverse), ctypes.byref(c_rg), ctypes.byref(c_side), ws.data_ptr(),
+                                                 nbytes, _stream()), 'rua_segment_scan_backward')
+        if prof is not None:
+            nb = g.numel() * g.element_size() * (4 if op == _lib.SCAN_LOGSUMEXP else 2)
+            _profile_end(prof, 'segment_scan_backward', nb + (8 * g.numel() if idx is not None else 0) + 8 * rg.B)
+    return grad
+
+
+class _ScanSum(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, data: Tensor, rg: Ragged, side: SideSpec, reverse: bool):
+        ctx.meta = (rg, side, reverse)
+        return _scan_raw(data.detach().contiguous(), rg, side, _lib.SCAN_SUM, reverse)[0]
+
+    @staticmethod
+    def backward(ctx, grad_out: Tensor):
+        rg, side, reverse = ctx.meta
+        # the gradient of a prefix sum is the suffix sum: the differentiable call, so double backward works
+        return segment_scan(grad_out, rg, side, 'sum', not reverse)[0], None, None, None
+
+
+class _ScanLogSumExp(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, data: Tensor, rg: Ragged, side: SideSpec, reverse: bool):
+        x = data.detach().contiguous()
+        y = _scan_raw(x, rg, side, _lib.SCAN_LOGSUMEXP, reverse)[0]
+        ctx.meta = (rg, side, reverse)
+        ctx.save_for_backward(x, y)
+        return y
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_out: Tensor):
+        rg, side, reverse = ctx.meta
+        x, y = ctx.saved_tensors
+        return _scan_backward_raw(grad_out, x, y, None, rg, side, _lib.SCAN_LOGSUMEXP, reverse), None, None, None
+
+
+class _ScanExtreme(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, data: Tensor, rg: Ragged, side: SideSpec, op: int, reverse: bool):
+        out, idx = _scan_raw(data.detach().contiguous(), rg, side, op, reverse)
+        ctx.meta = (rg, side, op, reverse)
+        ctx.save_for_backward(idx)
+        ctx.mark_non_differentiable(idx)
+        return out, idx
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_out: Tensor, _grad_idx):
+        rg, side, op, reverse = ctx.meta
+        idx, = ctx.saved_tensors
+        return _scan_backward_raw(grad_out, None, None, idx, rg, side, op, reverse), None, None, None, None
+
+
+def segment_scan(data: Tensor, rg: Ragged, side: SideSpec, op: str, reverse: bool):
+    """per-sequence inclusive scan of the flattened storage ``data`` (side.rows, *feat) -> (out, idx or None)."""
+    _scan_check(data)
+    require_cuda(data)
+    code = _SCAN_OPS[op]
+    grad = data.requires_grad and torch.is_grad_enabled()
+    if not grad:
+        return _scan_raw(data if data.is_contiguous() else data.contiguous(), rg, side, code, reverse)
+    if code == _lib.SCAN_SUM:
+        return _ScanSum.apply(data, rg, side, reverse), None
+    if code == _lib.SCAN_LOGSUMEXP:
+        return _ScanLogSumExp.apply(data, rg, side, reverse), None
+    return _ScanExtreme.apply(data, rg, side, code, reverse)
 
 
 # ------------------------------------------------------------------------------------------------
