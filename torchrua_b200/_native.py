@@ -1099,13 +1099,17 @@ class strict_reductions:
         return False
 
 
-def _reduce_raw(data: Tensor, off: Tensor, S: int, op: int) -> Tensor:
+def _reduce_raw(data: Tensor, off: Tensor, S: int, op: int, rows: Optional[Tensor] = None) -> Tensor:
+    """out[s] = reduce(data[off[s]:off[s + 1]]), or with `rows` reduce(data[rows[off[s]:off[s + 1]]]) (the kernel gathers
+    the rows; no strict mode)."""
     lib = _lib.load()
     if data.dtype not in _DTYPES:
+        if rows is not None:
+            raise RuntimeError(f'torchrua_b200: scatter reductions support float16/bfloat16/float32/float64, got {data.dtype}')
         raise RuntimeError(f'torchrua_b200: segment reductions support float16/bfloat16/float32/float64, got '
                            f'{data.dtype} (the reference rejects integer data too: "_segment_reduce" not '
                            f'implemented for Long)')
-    N = data.shape[0]
+    N = data.shape[0] if rows is None else rows.numel()
     feat = tuple(data.shape[1:])
     H = 1
     for f in feat:
@@ -1114,7 +1118,7 @@ def _reduce_raw(data: Tensor, off: Tensor, S: int, op: int) -> Tensor:
     if out.numel() == 0:
         return out
     dt = _DTYPES[data.dtype]
-    if STRICT_REDUCTIONS and op in _STRICT_OPS:
+    if rows is None and STRICT_REDUCTIONS and op in _STRICT_OPS:
         with _on(data.device):
             _lib.check(lib.rua_segment_reduce_strict(_ptr(data), off.data_ptr(), N, S, H, dt, op, out.data_ptr(),
                                                      _stream()), 'rua_segment_reduce_strict')
@@ -1123,11 +1127,34 @@ def _reduce_raw(data: Tensor, off: Tensor, S: int, op: int) -> Tensor:
         nbytes = lib.rua_segment_reduce_workspace_bytes(N, S, H, dt, op)
         ws = torch.empty(nbytes, dtype=torch.uint8, device=data.device)
         prof = _profile_begin()
-        _lib.check(lib.rua_segment_reduce(_ptr(data), off.data_ptr(), N, S, H, dt, op, out.data_ptr(), ws.data_ptr(),
-                                          nbytes, _stream()), 'rua_segment_reduce')
+        if rows is None:
+            _lib.check(lib.rua_segment_reduce(_ptr(data), off.data_ptr(), N, S, H, dt, op, out.data_ptr(),
+                                              ws.data_ptr(), nbytes, _stream()), 'rua_segment_reduce')
+        else:
+            _lib.check(lib.rua_segment_reduce_gather(_ptr(data), rows.data_ptr(), off.data_ptr(), N, S, H, dt, op,
+                                                     out.data_ptr(), ws.data_ptr(), nbytes, _stream()),
+                       'rua_segment_reduce_gather')
         if prof is not None:
-            _profile_end(prof, 'segment_reduce', (N + S) * H * data.element_size() + 8 * S)
+            if rows is None:
+                _profile_end(prof, 'segment_reduce', (N + S) * H * data.element_size() + 8 * S)
+            else:
+                _profile_end(prof, 'segment_reduce_gather', (N + S) * H * data.element_size() + 8 * (S + N))
     return out
+
+
+def _reduce_backward_raw(grad_out: Tensor, out: Tensor, data: Tensor, off: Tensor, S: int, op: int,
+                         grad: Tensor) -> None:
+    """grad (the shape of data, at least one element) = gradient of out = _reduce_raw(data, off, S, op)."""
+    lib = _lib.load()
+    N = data.shape[0]
+    H = data[0].numel()
+    dt = _DTYPES[data.dtype]
+    with _on(data.device):
+        nbytes = lib.rua_segment_reduce_backward_workspace_bytes(N, S, H, dt, op)
+        ws = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=data.device)
+        _lib.check(lib.rua_segment_reduce_backward(grad_out.data_ptr(), out.data_ptr(), data.data_ptr(), off.data_ptr(),
+                                                   N, S, H, dt, op, grad.data_ptr(), ws.data_ptr(), nbytes, _stream()),
+                   'rua_segment_reduce_backward')
 
 
 class _SegmentReduce(torch.autograd.Function):
@@ -1144,21 +1171,10 @@ class _SegmentReduce(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, grad_out: Tensor):
-        lib = _lib.load()
         data, off, out = ctx.saved_tensors
-        g = grad_out.contiguous()
-        N = data.shape[0]
-        H = data[0].numel() if N else 0
         grad = torch.empty_like(data)
         if grad.numel() > 0:
-            dt = _DTYPES[data.dtype]
-            with _on(data.device):
-                nbytes = lib.rua_segment_reduce_backward_workspace_bytes(N, ctx.S, H, dt, ctx.op)
-                ws = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=data.device)
-                _lib.check(lib.rua_segment_reduce_backward(g.data_ptr(), out.data_ptr(), data.data_ptr(),
-                                                           off.data_ptr(), N, ctx.S, H, dt, ctx.op, grad.data_ptr(),
-                                                           ws.data_ptr(), nbytes, _stream()),
-                           'rua_segment_reduce_backward')
+            _reduce_backward_raw(grad_out.contiguous(), out, data, off, ctx.S, ctx.op, grad)
         return grad, None, None, None
 
 
@@ -1321,31 +1337,6 @@ def bucket_offsets(keys: Tensor, srt: Tensor, buckets: int) -> Tensor:
     return off
 
 
-def _reduce_gather_raw(data: Tensor, row_index: Tensor, off: Tensor, S: int, op: int) -> Tensor:
-    lib = _lib.load()
-    if data.dtype not in _DTYPES:
-        raise RuntimeError(f'torchrua_b200: scatter reductions support float16/bfloat16/float32/float64, got {data.dtype}')
-    N = row_index.numel()
-    feat = tuple(data.shape[1:])
-    H = 1
-    for f in feat:
-        H *= f
-    out = torch.empty((S,) + feat, dtype=data.dtype, device=data.device)
-    if out.numel() == 0:
-        return out
-    dt = _DTYPES[data.dtype]
-    with _on(data.device):
-        nbytes = lib.rua_segment_reduce_workspace_bytes(N, S, H, dt, op)
-        ws = torch.empty(nbytes, dtype=torch.uint8, device=data.device)
-        prof = _profile_begin()
-        _lib.check(lib.rua_segment_reduce_gather(_ptr(data), row_index.data_ptr(), off.data_ptr(), N, S, H, dt, op,
-                                                 out.data_ptr(), ws.data_ptr(), nbytes, _stream()),
-                   'rua_segment_reduce_gather')
-        if prof is not None:
-            _profile_end(prof, 'segment_reduce_gather', (N + S) * H * data.element_size() + 8 * (S + N))
-    return out
-
-
 class _ScatterReduce(torch.autograd.Function):
     """out[m] = reduce over {source[k] : index[k] == m}; rows of `source` are gathered in sorted-index order
     inside the kernel.  Backward: gather the rows into sorted order, run the segment-reduce backward kernel,
@@ -1356,30 +1347,21 @@ class _ScatterReduce(torch.autograd.Function):
         flat = source.detach()
         if not flat.is_contiguous():
             flat = flat.contiguous()
-        out = _reduce_gather_raw(flat, srt, off, S, op)
+        out = _reduce_raw(flat, off, S, op, rows=srt)
         ctx.op, ctx.S = op, S
         ctx.save_for_backward(flat, srt, off, out)
         return out
 
     @staticmethod
     def backward(ctx, grad_out: Tensor):
-        lib = _lib.load()
         source, srt, off, out = ctx.saved_tensors
-        g = grad_out.contiguous()
         K = srt.numel()
         H = source[0].numel() if source.shape[0] else 0
         grad = torch.zeros_like(source)
         if K > 0 and H > 0:
             ordered = _gather_rows_raw(source, srt)               # rows in sorted-index order
             grad_ordered = torch.empty_like(ordered)
-            dt = _DTYPES[source.dtype]
-            with _on(source.device):
-                nbytes = lib.rua_segment_reduce_backward_workspace_bytes(K, ctx.S, H, dt, ctx.op)
-                ws = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=source.device)
-                _lib.check(lib.rua_segment_reduce_backward(g.data_ptr(), out.data_ptr(), ordered.data_ptr(),
-                                                           off.data_ptr(), K, ctx.S, H, dt, ctx.op,
-                                                           grad_ordered.data_ptr(), ws.data_ptr(), nbytes, _stream()),
-                           'rua_segment_reduce_backward')
+            _reduce_backward_raw(grad_out.contiguous(), out, ordered, off, ctx.S, ctx.op, grad_ordered)
             scatter_rows_(grad, srt, grad_ordered)
         return grad, None, None, None, None
 
@@ -1392,7 +1374,7 @@ def segment_reduce_gathered(source: Tensor, rows: Tensor, segment_sizes: Tensor,
     rows = _i64(rows).view(-1)
     if source.requires_grad and torch.is_grad_enabled():
         return _ScatterReduce.apply(source, rows, rg.off, rg.B, _OPS[op])
-    return _reduce_gather_raw(source if source.is_contiguous() else source.contiguous(), rows, rg.off, rg.B, _OPS[op])
+    return _reduce_raw(source if source.is_contiguous() else source.contiguous(), rg.off, rg.B, _OPS[op], rows=rows)
 
 
 def scatter_reduce(source: Tensor, index: Tensor, buckets: int, op: str):
@@ -1403,5 +1385,5 @@ def scatter_reduce(source: Tensor, index: Tensor, buckets: int, op: str):
     if source.requires_grad and torch.is_grad_enabled():
         red = _ScatterReduce.apply(source, srt, off, buckets, _OPS[op])
     else:
-        red = _reduce_gather_raw(source if source.is_contiguous() else source.contiguous(), srt, off, buckets, _OPS[op])
+        red = _reduce_raw(source if source.is_contiguous() else source.contiguous(), off, buckets, _OPS[op], rows=srt)
     return red, off[1:] - off[:-1]

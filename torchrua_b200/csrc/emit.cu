@@ -7,9 +7,8 @@
 // The reference builds these from repeat_interleave (each an internal cumsum + a .item() sync),
 // arange, new_full and index_put_.  Here every output element is a closed form of (segment, within)
 // and is stored once with 16-byte coalesced stores.  HBM-write bound.
-#include <cstdlib>
-
 #include "common.cuh"
+#include "dispatch.cuh"
 #include "tile_decode.cuh"
 
 namespace rua {
@@ -317,8 +316,7 @@ int rua_emit_ptr(const int64_t* off, int64_t S, int64_t n, const int64_t* relabe
   if (blocks >= (1ll << 31)) return RUA_ERR_UNSUPPORTED;
   const uintptr_t align = (uintptr_t)which | (uintptr_t)within | (uintptr_t)flat;
   // many short segments (C.ptr / L.idx / R.idx of a large batch): a warp per 32 segments, no per-tile decode chain
-  static const int64_t ws_min = [] { const char* e = getenv("RUA_WARPSEG_MIN_S"); return e ? atoll(e) : 32768ll; }();
-  if (!relabel && S >= ws_min && n <= 256 * S) {
+  if (!relabel && warpseg_applies(n, S)) {
     const int64_t wblocks = ceil_div(S, (int64_t)kEwWarps * 32);
     if (wblocks >= (1ll << 31)) return RUA_ERR_UNSUPPORTED;
     emit_ptr_warpseg_kernel<<<(unsigned)wblocks, kEwThreads, 0, (cudaStream_t)stream>>>(off, S, n, which, within, flat,

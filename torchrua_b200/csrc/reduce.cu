@@ -19,28 +19,6 @@
 //   * the reference's `initial` quirks (SURVEY.md 8c hazard 3) cost no extra pass: the global
 //     extreme is reduced on the fly (one atomic per CTA) and a NaN is detected at emit time; a
 //     third tiny kernel patches empty segments and applies the NaN poisoning.
-#include "reduce_common.cuh"
-
-namespace rua {
-
-// narrow rows (H * elem <= 16 bytes) run on the rows-on-lanes kernels of reduce_flat.cu
-bool flat_supported(int32_t dtype, int64_t H);
-int flat_rows_per_tile(int32_t dtype, int64_t H);
-int flat_launch(int32_t dtype, int64_t H, int32_t op, const void* data, const int64_t* ridx, const int64_t* off,
-                int64_t N, int64_t S, void* out, void* head, void* tail, int64_t* tail_seg, void* hdr,
-                int vector_loads, int64_t tiles, cudaStream_t st);
-// ... or, with many short segments, on the warp-per-32-segments kernel of reduce_warpseg.cu
-bool warpseg_applies(int64_t N, int64_t S);
-int warpseg_launch(int32_t dtype, int64_t H, int32_t op, const void* data, const int64_t* off, int64_t N, int64_t S,
-                   void* out, void* hdr, cudaStream_t st);
-// ... and wide rows in very short segments on the SHORT instance of the main kernel (reduce_short.cu)
-bool short_applies(int64_t N, int64_t S, int32_t op);
-int short_launch(int32_t dtype, int32_t op, bool gather, bool packed, dim3 grid, int threads, const void* data,
-                 const int64_t* ridx, const int64_t* off, int64_t N, int64_t S, int64_t H, int R, void* out, void* head,
-                 void* tail, int64_t* tail_seg, void* hdr, int lanes_log2, int64_t chunks, cudaStream_t st);
-
-}  // namespace rua
-
 #include "reduce_kernel.cuh"
 
 namespace rua {
@@ -153,7 +131,7 @@ static RedPlan plan_reduce(int64_t N, int64_t H, int32_t dtype, int32_t op, cons
     p.part_elems = (size_t)p.chunks * (size_t)H * (op == RUA_LOGSUMEXP ? 2 : 1);
     return p;
   }
-  int full = dtype == RUA_F32 ? 4 : (dtype == RUA_F64 ? 2 : 8);
+  int full = vec_elems(dtype);
   bool aligned = (H % full == 0) && (((uintptr_t)data | (uintptr_t)out) & 15u) == 0;
   p.vec = aligned ? full : 1;
   int64_t hv = H / p.vec;
@@ -205,21 +183,22 @@ static int run_reduce(const RedPlan& p, const void* data, const int64_t* ridx, c
       rc = flat_launch(p.dtype, H, OP, data, ridx, off, N, S, out, head, tail, tail_seg, hdr, ridx ? 0 : p.vector_loads, p.chunks, st);
       if (rc) return rc;
     } else {
-#define RUA_LAUNCH_SEGREDUCE(G_, P_)                                                                              \
-  segreduce_kernel<T, V, OP, G_, P_><<<grid, p.main_threads, 0, st>>>((const T*)data, ridx, off, N, S, H, p.R, (T*)out, \
-                                                                      head, tail, tail_seg, hdr, p.lanes_log2, p.chunks)
+      auto launch = [&](auto gather, auto packed) {
+        segreduce_kernel<T, V, OP, decltype(gather)::value, decltype(packed)::value><<<grid, p.main_threads, 0, st>>>(
+            (const T*)data, ridx, off, N, S, H, p.R, (T*)out, head, tail, tail_seg, hdr, p.lanes_log2, p.chunks);
+      };
       const bool packed = (p.main_threads >> p.lanes_log2) > 1;
       if constexpr (V > 1) {   // packing exists for the vectorised instances only (V = 1 is the odd-alignment fallback)
         if (short_applies(N, S, OP)) {
           rc = short_launch(p.dtype, OP, ridx != nullptr, packed, grid, p.main_threads, data, ridx, off, N, S, H, p.R, out,
                             head, tail, tail_seg, hdr, p.lanes_log2, p.chunks, st);
           if (rc) return rc;
-        } else if (packed) { if (ridx) RUA_LAUNCH_SEGREDUCE(true, true); else RUA_LAUNCH_SEGREDUCE(false, true); }
-        else { if (ridx) RUA_LAUNCH_SEGREDUCE(true, false); else RUA_LAUNCH_SEGREDUCE(false, false); }
+        } else {
+          with_bool(ridx != nullptr, [&](auto g) { with_bool(packed, [&](auto pk) { launch(g, pk); }); });
+        }
       } else {
-        if (ridx) RUA_LAUNCH_SEGREDUCE(true, false); else RUA_LAUNCH_SEGREDUCE(false, false);
+        with_bool(ridx != nullptr, [&](auto g) { launch(g, std::false_type{}); });
       }
-#undef RUA_LAUNCH_SEGREDUCE
       if ((rc = check_launch())) return rc;
     }
     if (p.chunks > 1) {
@@ -230,27 +209,6 @@ static int run_reduce(const RedPlan& p, const void* data, const int64_t* ridx, c
   }
   segreduce_patch_kernel<T, V, OP><<<(unsigned)ceil_div(S, 256), 256, 0, st>>>(off, S, H, (T*)out, hdr);
   return check_launch();
-}
-
-template <typename T, int V>
-static int dispatch_op(int32_t op, const RedPlan& p, const void* data, const int64_t* ridx, const int64_t* off, int64_t N,
-                       int64_t S, int64_t H, void* out, void* ws, cudaStream_t st) {
-  switch (op) {
-    case RUA_SUM: return run_reduce<T, V, RUA_SUM>(p, data, ridx, off, N, S, H, out, ws, st);
-    case RUA_MEAN: return run_reduce<T, V, RUA_MEAN>(p, data, ridx, off, N, S, H, out, ws, st);
-    case RUA_PROD: return run_reduce<T, V, RUA_PROD>(p, data, ridx, off, N, S, H, out, ws, st);
-    case RUA_MAX: return run_reduce<T, V, RUA_MAX>(p, data, ridx, off, N, S, H, out, ws, st);
-    case RUA_MIN: return run_reduce<T, V, RUA_MIN>(p, data, ridx, off, N, S, H, out, ws, st);
-    case RUA_LOGSUMEXP: return run_reduce<T, V, RUA_LOGSUMEXP>(p, data, ridx, off, N, S, H, out, ws, st);
-    default: return RUA_ERR_INVALID;
-  }
-}
-
-template <typename T>
-static int dispatch_vec(int32_t op, const RedPlan& p, const void* data, const int64_t* ridx, const int64_t* off, int64_t N,
-                        int64_t S, int64_t H, void* out, void* ws, cudaStream_t st) {
-  if (p.vec == 1) return dispatch_op<T, 1>(op, p, data, ridx, off, N, S, H, out, ws, st);
-  return dispatch_op<T, Store<T>::kVec>(op, p, data, ridx, off, N, S, H, out, ws, st);
 }
 
 }  // namespace rua
@@ -265,7 +223,7 @@ size_t rua_segment_reduce_workspace_bytes(int64_t N, int64_t S, int64_t H, int32
   // the vector width may drop to 1 for misaligned views; that only changes threads/tiles, not R... be safe:
   RedPlan q = plan_reduce(N, H, dtype, op, (const void*)1, nullptr);
   size_t elems = p.part_elems > q.part_elems ? p.part_elems : q.part_elems;
-  size_t acc = dtype == RUA_F64 ? 8 : 4;
+  size_t acc = acc_bytes(dtype);
   size_t chunks = p.chunks > q.chunks ? p.chunks : q.chunks;
   return sizeof(RedHeader) + tail_seg_bytes(chunks) + 2 * elems * acc + 64;
 }
@@ -285,16 +243,17 @@ int rua_segment_reduce_gather(const void* data, const int64_t* row_index, const 
   if (op < RUA_SUM || op > RUA_LOGSUMEXP) return RUA_ERR_INVALID;
   if (dtype < RUA_F32 || dtype > RUA_BF16) return RUA_ERR_UNSUPPORTED;
   RedPlan p = plan_reduce(N, H, dtype, op, data, out);
-  size_t acc = dtype == RUA_F64 ? 8 : 4;
-  if (ws_bytes < sizeof(RedHeader) + tail_seg_bytes(p.chunks) + 2 * p.part_elems * acc) return RUA_ERR_WORKSPACE;
+  if (ws_bytes < sizeof(RedHeader) + tail_seg_bytes(p.chunks) + 2 * p.part_elems * acc_bytes(dtype)) return RUA_ERR_WORKSPACE;
   if (((uintptr_t)ws & 15u) != 0) return RUA_ERR_INVALID;
   cudaStream_t st = (cudaStream_t)stream;
-  switch (dtype) {
-    case RUA_F32: return dispatch_vec<float>(op, p, data, ridx, off, N, S, H, out, ws, st);
-    case RUA_F64: return dispatch_vec<double>(op, p, data, ridx, off, N, S, H, out, ws, st);
-    case RUA_F16: return dispatch_vec<__half>(op, p, data, ridx, off, N, S, H, out, ws, st);
-    default: return dispatch_vec<__nv_bfloat16>(op, p, data, ridx, off, N, S, H, out, ws, st);
-  }
+  return with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    return with_op(op, [&](auto o) {
+      constexpr int OP = decltype(o)::value;
+      if (p.vec == 1) return run_reduce<T, 1, OP>(p, data, ridx, off, N, S, H, out, ws, st);
+      return run_reduce<T, Store<T>::kVec, OP>(p, data, ridx, off, N, S, H, out, ws, st);
+    });
+  });
 }
 
 }  // extern "C"

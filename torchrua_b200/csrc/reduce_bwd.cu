@@ -18,12 +18,6 @@
 
 namespace rua {
 
-// narrow rows + many short segments: the warp-per-32-segments twin in reduce_warpseg.cu
-bool flat_supported(int32_t dtype, int64_t H);
-bool warpseg_applies(int64_t N, int64_t S);
-int warpseg_bwd_launch(int32_t dtype, int64_t H, int32_t op, const void* gout, const void* out, const void* data,
-                       const int64_t* off, int64_t N, int64_t S, void* grad, cudaStream_t st);
-
 constexpr int kBwdUnroll = 4;
 constexpr int kTieInlineAvg = 8;   // max / min backward: average segment length up to which the INLINE instances run
 
@@ -302,27 +296,6 @@ static int run_bwd(const void* gout, const void* out, const void* data, const in
   return check_launch();
 }
 
-template <typename T, int V>
-static int bwd_op(int32_t op, const void* gout, const void* out, const void* data, const int64_t* off, int64_t N,
-                  int64_t S, int64_t H, void* grad, void* ws, cudaStream_t st) {
-  switch (op) {
-    case RUA_SUM: return run_bwd<T, V, RUA_SUM>(gout, out, data, off, N, S, H, grad, ws, st);
-    case RUA_MEAN: return run_bwd<T, V, RUA_MEAN>(gout, out, data, off, N, S, H, grad, ws, st);
-    case RUA_PROD: return run_bwd<T, V, RUA_PROD>(gout, out, data, off, N, S, H, grad, ws, st);
-    case RUA_MAX: return run_bwd<T, V, RUA_MAX>(gout, out, data, off, N, S, H, grad, ws, st);
-    case RUA_MIN: return run_bwd<T, V, RUA_MIN>(gout, out, data, off, N, S, H, grad, ws, st);
-    case RUA_LOGSUMEXP: return run_bwd<T, V, RUA_LOGSUMEXP>(gout, out, data, off, N, S, H, grad, ws, st);
-    default: return RUA_ERR_INVALID;
-  }
-}
-
-template <typename T>
-static int bwd_vec(bool vec, int32_t op, const void* gout, const void* out, const void* data, const int64_t* off,
-                   int64_t N, int64_t S, int64_t H, void* grad, void* ws, cudaStream_t st) {
-  if (!vec) return bwd_op<T, 1>(op, gout, out, data, off, N, S, H, grad, ws, st);
-  return bwd_op<T, Store<T>::kVec>(op, gout, out, data, off, N, S, H, grad, ws, st);
-}
-
 }  // namespace rua
 
 using namespace rua;
@@ -349,22 +322,19 @@ int rua_segment_reduce_backward(const void* grad_out, const void* out, const voi
   if (dtype < RUA_F32 || dtype > RUA_BF16) return RUA_ERR_UNSUPPORTED;
   if (ws_bytes < rua_segment_reduce_backward_workspace_bytes(N, S, H, dtype, op) - 16) return RUA_ERR_WORKSPACE;
   if ((op == RUA_MAX || op == RUA_MIN) && !ws) return RUA_ERR_INVALID;
-  int full = dtype == RUA_F32 ? 4 : (dtype == RUA_F64 ? 2 : 8);
   uintptr_t a = (uintptr_t)grad_out | (uintptr_t)out | (uintptr_t)data | (uintptr_t)grad_data;
-  bool vec = (H % full == 0) && (a & 15u) == 0;
+  bool vec = (H % vec_elems(dtype) == 0) && (a & 15u) == 0;
   cudaStream_t st = (cudaStream_t)stream;
-  if (H == 1 && warpseg_applies(N, S) && (((uintptr_t)data | (uintptr_t)grad_data) & 15u) == 0) {
-    // rows no segment owns (sum of sizes < N) get no gradient; the kernel only writes rows it owns
-    int rc = check_cuda(cudaMemsetAsync(grad_data, 0, 0, st));
-    if (rc) return rc;
+  if (H == 1 && warpseg_applies(N, S) && (((uintptr_t)data | (uintptr_t)grad_data) & 15u) == 0)
     return warpseg_bwd_launch(dtype, H, op, grad_out, out, data, off, N, S, grad_data, st);
-  }
-  switch (dtype) {
-    case RUA_F32: return bwd_vec<float>(vec, op, grad_out, out, data, off, N, S, H, grad_data, ws, st);
-    case RUA_F64: return bwd_vec<double>(vec, op, grad_out, out, data, off, N, S, H, grad_data, ws, st);
-    case RUA_F16: return bwd_vec<__half>(vec, op, grad_out, out, data, off, N, S, H, grad_data, ws, st);
-    default: return bwd_vec<__nv_bfloat16>(vec, op, grad_out, out, data, off, N, S, H, grad_data, ws, st);
-  }
+  return with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    return with_op(op, [&](auto o) {
+      constexpr int OP = decltype(o)::value;
+      if (!vec) return run_bwd<T, 1, OP>(grad_out, out, data, off, N, S, H, grad_data, ws, st);
+      return run_bwd<T, Store<T>::kVec, OP>(grad_out, out, data, off, N, S, H, grad_data, ws, st);
+    });
+  });
 }
 
 }  // extern "C"

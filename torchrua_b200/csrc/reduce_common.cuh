@@ -6,6 +6,7 @@
 #include <math_constants.h>
 
 #include "common.cuh"
+#include "dispatch.cuh"
 
 namespace rua {
 
@@ -92,6 +93,12 @@ template <> struct Store<__nv_bfloat16> {
   __device__ static Acc to_acc(__nv_bfloat16 v) { return __bfloat162float(v); }
   __device__ static __nv_bfloat16 from_acc(Acc v) { return __float2bfloat16_rn(v); }
 };
+
+template <int32_t D, typename T> constexpr bool store_matches() {
+  return vec_elems(D) == Store<T>::kVec && acc_bytes(D) == sizeof(typename Store<T>::Acc) && Store<T>::kVec * sizeof(T) == 16;
+}
+static_assert(store_matches<RUA_F32, float>() && store_matches<RUA_F64, double>() && store_matches<RUA_F16, __half>() &&
+              store_matches<RUA_BF16, __nv_bfloat16>(), "vec_elems / acc_bytes (dispatch.cuh) disagree with Store<T>");
 
 // ---------------------------------------------------------------------------------------------
 // scalar math on the accumulator type
@@ -428,5 +435,25 @@ __device__ __forceinline__ void load_partial(const A* base, int64_t H, int64_t c
   }
 }
 
+// ---------------------------------------------------------------------------------------------
+// host launchers defined in one translation unit and called from another (reduce.cu, reduce_bwd.cu)
+// ---------------------------------------------------------------------------------------------
+// narrow rows (H * elem <= 16 bytes) run on the rows-on-lanes kernels of reduce_flat.cu
+bool flat_supported(int32_t dtype, int64_t H);
+int flat_rows_per_tile(int32_t dtype, int64_t H);
+int flat_launch(int32_t dtype, int64_t H, int32_t op, const void* data, const int64_t* ridx, const int64_t* off,
+                int64_t N, int64_t S, void* out, void* head, void* tail, int64_t* tail_seg, void* hdr,
+                int vector_loads, int64_t tiles, cudaStream_t st);
+// ... or, with many short segments (warpseg_applies), on the warp-per-32-segments kernels of reduce_warpseg.cu and
+// reduce_warpseg_bwd.cu
+int warpseg_launch(int32_t dtype, int64_t H, int32_t op, const void* data, const int64_t* off, int64_t N, int64_t S,
+                   void* out, void* hdr, cudaStream_t st);
+int warpseg_bwd_launch(int32_t dtype, int64_t H, int32_t op, const void* gout, const void* out, const void* data,
+                       const int64_t* off, int64_t N, int64_t S, void* grad, cudaStream_t st);
+// ... and wide rows in very short segments on the SHORT instance of the main kernel (reduce_short.cu)
+bool short_applies(int64_t N, int64_t S, int32_t op);
+int short_launch(int32_t dtype, int32_t op, bool gather, bool packed, dim3 grid, int threads, const void* data,
+                 const int64_t* ridx, const int64_t* off, int64_t N, int64_t S, int64_t H, int R, void* out, void* head,
+                 void* tail, int64_t* tail_seg, void* hdr, int lanes_log2, int64_t chunks, cudaStream_t st);
 
 }  // namespace rua

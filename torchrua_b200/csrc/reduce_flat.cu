@@ -317,63 +317,30 @@ segreduce_flat_kernel(const T* __restrict__ data, const int64_t* __restrict__ ri
   }
 }
 
-template <typename T, int HE, int OP>
-static void flat_launch3(const void* data, const int64_t* ridx, const int64_t* off, int64_t N, int64_t S, void* out, void* head, void* tail,
-                         int64_t* tail_seg, RedHeader* hdr, int vector_loads, int64_t tiles, cudaStream_t st) {
-  using A = typename Store<T>::Acc;
-  segreduce_flat_kernel<T, HE, OP><<<(unsigned)tiles, kFlatThreads, 0, st>>>(
-      (const T*)data, ridx, off, N, S, (T*)out, (A*)head, (A*)tail, tail_seg, hdr, vector_loads);
-}
-
-template <typename T, int HE>
-static int flat_launch2(int op, const void* data, const int64_t* ridx, const int64_t* off, int64_t N, int64_t S, void* out, void* head,
-                        void* tail, int64_t* tail_seg, RedHeader* hdr, int vl, int64_t tiles, cudaStream_t st) {
-  switch (op) {
-    case RUA_SUM: flat_launch3<T, HE, RUA_SUM>(data, ridx, off, N, S, out, head, tail, tail_seg, hdr, vl, tiles, st); break;
-    case RUA_MEAN: flat_launch3<T, HE, RUA_MEAN>(data, ridx, off, N, S, out, head, tail, tail_seg, hdr, vl, tiles, st); break;
-    case RUA_PROD: flat_launch3<T, HE, RUA_PROD>(data, ridx, off, N, S, out, head, tail, tail_seg, hdr, vl, tiles, st); break;
-    case RUA_MAX: flat_launch3<T, HE, RUA_MAX>(data, ridx, off, N, S, out, head, tail, tail_seg, hdr, vl, tiles, st); break;
-    case RUA_MIN: flat_launch3<T, HE, RUA_MIN>(data, ridx, off, N, S, out, head, tail, tail_seg, hdr, vl, tiles, st); break;
-    case RUA_LOGSUMEXP: flat_launch3<T, HE, RUA_LOGSUMEXP>(data, ridx, off, N, S, out, head, tail, tail_seg, hdr, vl, tiles, st); break;
-    default: return RUA_ERR_INVALID;
-  }
-  return check_launch();
-}
-
-template <typename T>
-static int flat_launch1(int he, int op, const void* data, const int64_t* ridx, const int64_t* off, int64_t N, int64_t S, void* out,
-                        void* head, void* tail, int64_t* tail_seg, RedHeader* hdr, int vl, int64_t tiles,
-                        cudaStream_t st) {
-  constexpr int E = 16 / sizeof(T);
-  if (he == 1) return flat_launch2<T, 1>(op, data, ridx, off, N, S, out, head, tail, tail_seg, hdr, vl, tiles, st);
-  if constexpr (E >= 2) if (he == 2) return flat_launch2<T, 2>(op, data, ridx, off, N, S, out, head, tail, tail_seg, hdr, vl, tiles, st);
-  if constexpr (E >= 4) if (he == 4) return flat_launch2<T, 4>(op, data, ridx, off, N, S, out, head, tail, tail_seg, hdr, vl, tiles, st);
-  if constexpr (E >= 8) if (he == 8) return flat_launch2<T, 8>(op, data, ridx, off, N, S, out, head, tail, tail_seg, hdr, vl, tiles, st);
-  return RUA_ERR_UNSUPPORTED;
-}
-
 // does a flat kernel exist for rows of `H` elements of this dtype?
 bool flat_supported(int32_t dtype, int64_t H) {
-  const int e = dtype == RUA_F32 ? 4 : (dtype == RUA_F64 ? 2 : 8);   // elements per 16 bytes
-  return H >= 1 && H <= e && (H & (H - 1)) == 0;
+  return H >= 1 && H <= vec_elems(dtype) && (H & (H - 1)) == 0;
 }
 
 int flat_rows_per_tile(int32_t dtype, int64_t H) {   // == FlatShape<T, H>::R
-  const int e = dtype == RUA_F32 ? 4 : (dtype == RUA_F64 ? 2 : 8);
-  const int g = e / (int)H;
+  const int g = vec_elems(dtype) / (int)H;
   return kFlatThreads * g * (g * 4 <= 16 ? 4 : 16 / g);
 }
 
 int flat_launch(int32_t dtype, int64_t H, int32_t op, const void* data, const int64_t* ridx, const int64_t* off,
                 int64_t N, int64_t S, void* out, void* head, void* tail, int64_t* tail_seg, void* hdr,
                 int vector_loads, int64_t tiles, cudaStream_t st) {
-  RedHeader* h = (RedHeader*)hdr;
-  switch (dtype) {
-    case RUA_F32: return flat_launch1<float>((int)H, op, data, ridx, off, N, S, out, head, tail, tail_seg, h, vector_loads, tiles, st);
-    case RUA_F64: return flat_launch1<double>((int)H, op, data, ridx, off, N, S, out, head, tail, tail_seg, h, vector_loads, tiles, st);
-    case RUA_F16: return flat_launch1<__half>((int)H, op, data, ridx, off, N, S, out, head, tail, tail_seg, h, vector_loads, tiles, st);
-    default: return flat_launch1<__nv_bfloat16>((int)H, op, data, ridx, off, N, S, out, head, tail, tail_seg, h, vector_loads, tiles, st);
-  }
+  return with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    using A = typename Store<T>::Acc;
+    return with_row_elems<T>(H, [&](auto he) {
+      return with_op(op, [&](auto o) {
+        segreduce_flat_kernel<T, decltype(he)::value, decltype(o)::value><<<(unsigned)tiles, kFlatThreads, 0, st>>>(
+            (const T*)data, ridx, off, N, S, (T*)out, (A*)head, (A*)tail, tail_seg, (RedHeader*)hdr, vector_loads);
+        return check_launch();
+      });
+    });
+  });
 }
 
 }  // namespace rua

@@ -4,8 +4,6 @@
 // long-segment instance in reduce.cu; only the walk over the 8 loaded rows differs (one visit per row with a boundary
 // test after it instead of one predicated sweep per run).  A separate translation unit so that the two families of
 // instantiations compile in parallel.
-#include <cstdlib>
-
 #include "reduce_kernel.cuh"
 
 namespace rua {
@@ -16,64 +14,30 @@ namespace rua {
 // pieces of 16: 91 > 84; logsumexp U[1,4] 56 -> 62, pieces of 8: 80 > 57 (its per-row online update costs more than
 // the batch form of the run-wise walk as soon as whole batches of 8 rows fall inside one segment).
 bool short_applies(int64_t N, int64_t S, int32_t op) {
-  static const int64_t avg = [] {
-    const char* e = getenv("RUA_SEG_SHORT_AVG");
-    return e ? (int64_t)atoll(e) : (int64_t)6;
-  }();
-  static const int64_t avg_lse = [] {
-    const char* e = getenv("RUA_SEG_SHORT_LSE_AVG");
-    return e ? (int64_t)atoll(e) : (int64_t)4;
-  }();
+  static const int64_t avg = knob("RUA_SEG_SHORT_AVG", 6);
+  static const int64_t avg_lse = knob("RUA_SEG_SHORT_LSE_AVG", 4);
   const int64_t a = op == RUA_LOGSUMEXP ? avg_lse : avg;
   return a > 0 && S > 0 && N < a * S;
-}
-
-template <typename T, int OP>
-static int short_launch_op(bool gather, bool packed, dim3 grid, int threads, const void* data, const int64_t* ridx,
-                           const int64_t* off, int64_t N, int64_t S, int64_t H, int R, void* out, void* head, void* tail,
-                           int64_t* tail_seg, void* hdr, int lanes_log2, int64_t chunks, cudaStream_t st) {
-  using A = typename Store<T>::Acc;
-  constexpr int V = Store<T>::kVec;
-#define RUA_SHORT(G_, P_)                                                                                          \
-  segreduce_kernel<T, V, OP, G_, P_, true><<<grid, threads, 0, st>>>((const T*)data, ridx, off, N, S, H, R, (T*)out, \
-                                                                     (A*)head, (A*)tail, tail_seg, (RedHeader*)hdr, \
-                                                                     lanes_log2, chunks)
-  if (packed) { if (gather) RUA_SHORT(true, true); else RUA_SHORT(false, true); }
-  else { if (gather) RUA_SHORT(true, false); else RUA_SHORT(false, false); }
-#undef RUA_SHORT
-  return check_launch();
-}
-
-template <typename T>
-static int short_launch_t(int32_t op, bool gather, bool packed, dim3 grid, int threads, const void* data,
-                          const int64_t* ridx, const int64_t* off, int64_t N, int64_t S, int64_t H, int R, void* out,
-                          void* head, void* tail, int64_t* tail_seg, void* hdr, int lanes_log2, int64_t chunks,
-                          cudaStream_t st) {
-#define RUA_SHORT_OP(OP_) \
-  case OP_: return short_launch_op<T, OP_>(gather, packed, grid, threads, data, ridx, off, N, S, H, R, out, head, tail, tail_seg, hdr, lanes_log2, chunks, st)
-  switch (op) {
-    RUA_SHORT_OP(RUA_SUM);
-    RUA_SHORT_OP(RUA_MEAN);
-    RUA_SHORT_OP(RUA_PROD);
-    RUA_SHORT_OP(RUA_MAX);
-    RUA_SHORT_OP(RUA_MIN);
-    RUA_SHORT_OP(RUA_LOGSUMEXP);
-    default: return RUA_ERR_INVALID;
-  }
-#undef RUA_SHORT_OP
 }
 
 // vectorised (16-byte column vectors) instances only; the caller keeps the V = 1 fallback on the generic kernel
 int short_launch(int32_t dtype, int32_t op, bool gather, bool packed, dim3 grid, int threads, const void* data,
                  const int64_t* ridx, const int64_t* off, int64_t N, int64_t S, int64_t H, int R, void* out, void* head,
                  void* tail, int64_t* tail_seg, void* hdr, int lanes_log2, int64_t chunks, cudaStream_t st) {
-  switch (dtype) {
-    case RUA_F32: return short_launch_t<float>(op, gather, packed, grid, threads, data, ridx, off, N, S, H, R, out, head, tail, tail_seg, hdr, lanes_log2, chunks, st);
-    case RUA_F64: return short_launch_t<double>(op, gather, packed, grid, threads, data, ridx, off, N, S, H, R, out, head, tail, tail_seg, hdr, lanes_log2, chunks, st);
-    case RUA_F16: return short_launch_t<__half>(op, gather, packed, grid, threads, data, ridx, off, N, S, H, R, out, head, tail, tail_seg, hdr, lanes_log2, chunks, st);
-    case RUA_BF16: return short_launch_t<__nv_bfloat16>(op, gather, packed, grid, threads, data, ridx, off, N, S, H, R, out, head, tail, tail_seg, hdr, lanes_log2, chunks, st);
-    default: return RUA_ERR_UNSUPPORTED;
-  }
+  return with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    using A = typename Store<T>::Acc;
+    return with_op(op, [&](auto o) {
+      with_bool(gather, [&](auto g) {
+        with_bool(packed, [&](auto pk) {
+          segreduce_kernel<T, Store<T>::kVec, decltype(o)::value, decltype(g)::value, decltype(pk)::value, true>
+              <<<grid, threads, 0, st>>>((const T*)data, ridx, off, N, S, H, R, (T*)out, (A*)head, (A*)tail, tail_seg,
+                                         (RedHeader*)hdr, lanes_log2, chunks);
+        });
+      });
+      return check_launch();
+    });
+  });
 }
 
 }  // namespace rua

@@ -70,26 +70,13 @@ segreduce_strict_kernel(const T* __restrict__ data, const int64_t* __restrict__ 
   store_vec<T, V>(out + s * H + col, acc);
 }
 
-template <typename T, int V>
-static int strict_launch(int32_t op, const void* data, const int64_t* off, int64_t S, int64_t H, void* out, cudaStream_t st) {
+template <typename T, int V, int OP>
+static int strict_launch(const void* data, const int64_t* off, int64_t S, int64_t H, void* out, cudaStream_t st) {
   const int64_t threads = S * (H / V);
   const int64_t blocks = ceil_div(threads, kStrictThreads);
   if (blocks >= (1ll << 31)) return RUA_ERR_UNSUPPORTED;
-  const unsigned nb = (unsigned)blocks;
-  switch (op) {
-    case RUA_SUM: segreduce_strict_kernel<T, V, RUA_SUM><<<nb, kStrictThreads, 0, st>>>((const T*)data, off, S, H, (T*)out); break;
-    case RUA_MEAN: segreduce_strict_kernel<T, V, RUA_MEAN><<<nb, kStrictThreads, 0, st>>>((const T*)data, off, S, H, (T*)out); break;
-    case RUA_PROD: segreduce_strict_kernel<T, V, RUA_PROD><<<nb, kStrictThreads, 0, st>>>((const T*)data, off, S, H, (T*)out); break;
-    default: return RUA_ERR_UNSUPPORTED;   // max / min are order-independent (already bit-exact); logsumexp has no exact replay
-  }
+  segreduce_strict_kernel<T, V, OP><<<(unsigned)blocks, kStrictThreads, 0, st>>>((const T*)data, off, S, H, (T*)out);
   return check_launch();
-}
-
-template <typename T>
-static int strict_dispatch(int32_t op, const void* data, const int64_t* off, int64_t S, int64_t H, void* out, cudaStream_t st) {
-  constexpr int V = Store<T>::kVec;
-  const bool vec = H % V == 0 && (((uintptr_t)data | (uintptr_t)out) & 15u) == 0;
-  return vec ? strict_launch<T, V>(op, data, off, S, H, out, st) : strict_launch<T, 1>(op, data, off, S, H, out, st);
 }
 
 }  // namespace rua
@@ -105,12 +92,19 @@ int rua_segment_reduce_strict(const void* data, const int64_t* off, int64_t N, i
   if (!off || !out || (N > 0 && !data)) return RUA_ERR_INVALID;
   if (dtype < RUA_F32 || dtype > RUA_BF16) return RUA_ERR_INVALID;
   cudaStream_t st = (cudaStream_t)stream;
-  switch (dtype) {
-    case RUA_F32: return strict_dispatch<float>(op, data, off, S, H, out, st);
-    case RUA_F64: return strict_dispatch<double>(op, data, off, S, H, out, st);
-    case RUA_F16: return strict_dispatch<__half>(op, data, off, S, H, out, st);
-    default: return strict_dispatch<__nv_bfloat16>(op, data, off, S, H, out, st);
-  }
+  return with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    constexpr int V = Store<T>::kVec;
+    const bool vec = H % V == 0 && (((uintptr_t)data | (uintptr_t)out) & 15u) == 0;
+    return with_op(op, [&](auto o) {
+      constexpr int OP = decltype(o)::value;
+      // max / min are order-independent (already bit-exact); logsumexp has no exact replay
+      if constexpr (OP == RUA_SUM || OP == RUA_MEAN || OP == RUA_PROD)
+        return vec ? strict_launch<T, V, OP>(data, off, S, H, out, st) : strict_launch<T, 1, OP>(data, off, S, H, out, st);
+      else
+        return (int)RUA_ERR_UNSUPPORTED;
+    }, RUA_ERR_UNSUPPORTED);
+  });
 }
 
 }  // extern "C"

@@ -20,8 +20,6 @@
 // Measured and dropped (round 2): 256-thread CTAs (4.4 waves at cfg5: 51 % vs 55 % of peak for 128 threads), and TWO groups of 32
 // segments per warp with both first windows in flight (43 %: the extra state costs occupancy, which is what hides the two serial
 // DRAM latencies -- offsets, then the window -- of a warp).
-#include <cstdlib>
-
 #include "warpseg_common.cuh"
 
 namespace rua {
@@ -208,53 +206,20 @@ segreduce_warpseg_kernel(const T* __restrict__ data, const int64_t* __restrict__
   }
 }
 
-template <typename T, int HE>
-static int ws_launch2(int op, const void* data, const int64_t* off, int64_t N, int64_t S, void* out, RedHeader* hdr,
-                      cudaStream_t st) {
-  const int64_t blocks = ceil_div(S, (int64_t)kWsWarps * 32);
-  if (blocks >= (1ll << 31)) return RUA_ERR_UNSUPPORTED;
-  const unsigned nb = (unsigned)blocks;
-#define RUA_WS(OP_) segreduce_warpseg_kernel<T, HE, OP_><<<nb, kWsThreads, 0, st>>>((const T*)data, off, N, S, (T*)out, hdr)
-  switch (op) {
-    case RUA_SUM: RUA_WS(RUA_SUM); break;
-    case RUA_MEAN: RUA_WS(RUA_MEAN); break;
-    case RUA_PROD: RUA_WS(RUA_PROD); break;
-    case RUA_MAX: RUA_WS(RUA_MAX); break;
-    case RUA_MIN: RUA_WS(RUA_MIN); break;
-    case RUA_LOGSUMEXP: RUA_WS(RUA_LOGSUMEXP); break;
-    default: return RUA_ERR_INVALID;
-  }
-#undef RUA_WS
-  return check_launch();
-}
-
-template <typename T>
-static int ws_launch1(int he, int op, const void* data, const int64_t* off, int64_t N, int64_t S, void* out, RedHeader* hdr,
-                      cudaStream_t st) {
-  constexpr int E = 16 / sizeof(T);
-  if (he == 1) return ws_launch2<T, 1>(op, data, off, N, S, out, hdr, st);
-  if constexpr (E >= 2) if (he == 2) return ws_launch2<T, 2>(op, data, off, N, S, out, hdr, st);
-  if constexpr (E >= 4) if (he == 4) return ws_launch2<T, 4>(op, data, off, N, S, out, hdr, st);
-  if constexpr (E >= 8) if (he == 8) return ws_launch2<T, 8>(op, data, off, N, S, out, hdr, st);
-  return RUA_ERR_UNSUPPORTED;
-}
-
-// enough short segments to fill the machine with warps of 32 segments each?  (host-side choice, reduce.cu)
-bool warpseg_applies(int64_t N, int64_t S) {
-  static const int64_t min_s = [] { const char* e = getenv("RUA_WARPSEG_MIN_S"); return e ? atoll(e) : 32768ll; }();
-  static const int64_t max_avg = [] { const char* e = getenv("RUA_WARPSEG_MAX_AVG"); return e ? atoll(e) : 256ll; }();
-  return S >= min_s && N <= max_avg * S;
-}
-
 int warpseg_launch(int32_t dtype, int64_t H, int32_t op, const void* data, const int64_t* off, int64_t N, int64_t S,
                    void* out, void* hdr, cudaStream_t st) {
-  RedHeader* h = (RedHeader*)hdr;
-  switch (dtype) {
-    case RUA_F32: return ws_launch1<float>((int)H, op, data, off, N, S, out, h, st);
-    case RUA_F64: return ws_launch1<double>((int)H, op, data, off, N, S, out, h, st);
-    case RUA_F16: return ws_launch1<__half>((int)H, op, data, off, N, S, out, h, st);
-    default: return ws_launch1<__nv_bfloat16>((int)H, op, data, off, N, S, out, h, st);
-  }
+  const int64_t blocks = ceil_div(S, (int64_t)kWsWarps * 32);
+  if (blocks >= (1ll << 31)) return RUA_ERR_UNSUPPORTED;
+  return with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    return with_row_elems<T>(H, [&](auto he) {
+      return with_op(op, [&](auto o) {
+        segreduce_warpseg_kernel<T, decltype(he)::value, decltype(o)::value><<<(unsigned)blocks, kWsThreads, 0, st>>>(
+            (const T*)data, off, N, S, (T*)out, (RedHeader*)hdr);
+        return check_launch();
+      });
+    });
+  });
 }
 
 }  // namespace rua

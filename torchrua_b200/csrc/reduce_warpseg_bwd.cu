@@ -1,6 +1,4 @@
 // K4w' -- backward twin of reduce_warpseg.cu (its own translation unit: the two files are ~160 kernel instances each).
-#include <cstdlib>
-
 #include "warpseg_common.cuh"
 
 namespace rua {
@@ -186,45 +184,23 @@ segreduce_bwd_warpseg_kernel(const T* __restrict__ gout, const T* __restrict__ o
   }
 }
 
-template <typename T, int HE>
-static int wsb_launch2(int op, const void* gout, const void* out, const void* data, const int64_t* off, int64_t N, int64_t S,
-                       void* grad, cudaStream_t st) {
-  const int64_t blocks = ceil_div(S, (int64_t)kWsWarps * 32);
-  if (blocks >= (1ll << 31)) return RUA_ERR_UNSUPPORTED;
-  const unsigned nb = (unsigned)blocks;
-#define RUA_WSB(OP_) segreduce_bwd_warpseg_kernel<T, HE, OP_><<<nb, kWsThreads, 0, st>>>((const T*)gout, (const T*)out, (const T*)data, off, N, S, (T*)grad)
-  switch (op) {
-    case RUA_SUM: RUA_WSB(RUA_SUM); break;
-    case RUA_MEAN: RUA_WSB(RUA_MEAN); break;
-    case RUA_PROD: RUA_WSB(RUA_PROD); break;
-    case RUA_MAX: RUA_WSB(RUA_MAX); break;
-    case RUA_MIN: RUA_WSB(RUA_MIN); break;
-    case RUA_LOGSUMEXP: RUA_WSB(RUA_LOGSUMEXP); break;
-    default: return RUA_ERR_INVALID;
-  }
-#undef RUA_WSB
-  return check_launch();
-}
-
-template <typename T>
-static int wsb_launch1(int he, int op, const void* gout, const void* out, const void* data, const int64_t* off, int64_t N,
-                       int64_t S, void* grad, cudaStream_t st) {
+// The kernel writes only the rows of [0, off[S]): rows past the last segment (sum of sizes < N) are left as they were.
+int warpseg_bwd_launch(int32_t dtype, int64_t H, int32_t op, const void* gout, const void* out, const void* data,
+                       const int64_t* off, int64_t N, int64_t S, void* grad, cudaStream_t st) {
   // per-token SCALARS only (H == 1: log-probabilities, losses, scores -- the config-5 shape).  Rows of 2..8 elements
   // keep the chunk kernel of reduce_bwd.cu: instantiating this kernel for them as well costs minutes of compile time
   // for a shape nothing on the path produces.
-  if (he == 1) return wsb_launch2<T, 1>(op, gout, out, data, off, N, S, grad, st);
-  return RUA_ERR_UNSUPPORTED;
-}
-
-// rows past the last segment (sum of sizes < N) receive no gradient: the caller zero-fills `grad` first in that case
-int warpseg_bwd_launch(int32_t dtype, int64_t H, int32_t op, const void* gout, const void* out, const void* data,
-                       const int64_t* off, int64_t N, int64_t S, void* grad, cudaStream_t st) {
-  switch (dtype) {
-    case RUA_F32: return wsb_launch1<float>((int)H, op, gout, out, data, off, N, S, grad, st);
-    case RUA_F64: return wsb_launch1<double>((int)H, op, gout, out, data, off, N, S, grad, st);
-    case RUA_F16: return wsb_launch1<__half>((int)H, op, gout, out, data, off, N, S, grad, st);
-    default: return wsb_launch1<__nv_bfloat16>((int)H, op, gout, out, data, off, N, S, grad, st);
-  }
+  if (H != 1) return RUA_ERR_UNSUPPORTED;
+  const int64_t blocks = ceil_div(S, (int64_t)kWsWarps * 32);
+  if (blocks >= (1ll << 31)) return RUA_ERR_UNSUPPORTED;
+  return with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    return with_op(op, [&](auto o) {
+      segreduce_bwd_warpseg_kernel<T, 1, decltype(o)::value><<<(unsigned)blocks, kWsThreads, 0, st>>>(
+          (const T*)gout, (const T*)out, (const T*)data, off, N, S, (T*)grad);
+      return check_launch();
+    });
+  });
 }
 
 }  // namespace rua

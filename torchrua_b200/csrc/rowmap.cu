@@ -14,10 +14,10 @@
 // lane.  Padding is written by the same pass, so every output byte is stored exactly once and no
 // payload byte is read twice: traffic = N*D read + rows_dst*D written (+ metadata).
 // HBM-bound; no shared memory (no reuse) and no tensor cores (nothing to contract).
-#include <cstdlib>
 #include <cstring>
 
 #include "common.cuh"
+#include "dispatch.cuh"
 #include "tile_decode.cuh"
 #include "tma.cuh"
 
@@ -216,11 +216,8 @@ __device__ __forceinline__ int64_t source_row(const RowMapParams& p, int64_t i, 
 template <typename V> __device__ __forceinline__ V ld_stream(const V* p) { return __ldcs(p); }
 template <typename V> __device__ __forceinline__ void st_stream(V* p, V v) { __stcs(p, v); }
 
-// 256-bit global accesses are new with sm_100 (SASS LDG.E.ENL2.256 / STG.E.ENL2.256): one full 32-byte
+// 256-bit global accesses (V256) are new with sm_100 (SASS LDG.E.ENL2.256 / STG.E.ENL2.256): one full 32-byte
 // sector per lane and half the LSU instructions of the 128-bit form.  Used when rows are 32-byte multiples.
-struct alignas(32) V256 {
-  unsigned long long x, y, z, w;
-};
 template <> __device__ __forceinline__ V256 ld_stream<V256>(const V256* p) {
   V256 v;
   asm volatile("ld.global.cs.v4.b64 {%0, %1, %2, %3}, [%4];" : "=l"(v.x), "=l"(v.y), "=l"(v.z), "=l"(v.w) : "l"(p));
@@ -1276,18 +1273,19 @@ static void launch_narrow(RowMapParams& p, int64_t rows, cudaStream_t st) {
     if (p.row_vecs == 1) {
       // one-vector rows: KT time tiles of 32 steps per CTA, all of their row loads in flight together
       constexpr int kMaxKT = sizeof(V) >= 16 ? 2 : 4;   // 48 KB of static shared memory
-      static const int kt_env = [] { const char* e = getenv("RUA_T1_KT"); return e ? atoi(e) : 0; }();
+      static const int64_t kt_env = knob("RUA_T1_KT", 0);
       int kt = gy <= 1 ? 1 : ((gy <= 2 || kMaxKT == 2) ? 2 : 4);
       if (sizeof(V) >= 16 && !from_pack) kt = 1;   // 16-byte rows into P: one tile per CTA measured 4.5 vs 4.1 TB/s (T = 512)
-      if (kt_env > 0 && kt_env <= kMaxKT) kt = kt_env;
+      if (kt_env > 0 && kt_env <= kMaxKT) kt = (int)kt_env;
       dim3 g1((unsigned)ceil_div(p.rg.B, 32), (unsigned)ceil_div(gy, kt));
-#define RUA_T1(FP_, KT_) row_map_transpose1_kernel<V, FP_, KT_><<<g1, 256, 0, st>>>(p)
-      if (from_pack) { if (kt == 1) RUA_T1(true, 1); else if (kt == 2) RUA_T1(true, 2); else RUA_T1(true, kMaxKT); }
-      else { if (kt == 1) RUA_T1(false, 1); else if (kt == 2) RUA_T1(false, 2); else RUA_T1(false, kMaxKT); }
-#undef RUA_T1
+      with_bool(from_pack, [&](auto fp) {
+        constexpr bool FP = decltype(fp)::value;
+        if (kt == 1) row_map_transpose1_kernel<V, FP, 1><<<g1, 256, 0, st>>>(p);
+        else if (kt == 2) row_map_transpose1_kernel<V, FP, 2><<<g1, 256, 0, st>>>(p);
+        else row_map_transpose1_kernel<V, FP, kMaxKT><<<g1, 256, 0, st>>>(p);
+      });
     } else {
-      if (from_pack) row_map_transpose_kernel<V, true, 0><<<grid, 256, 0, st>>>(p, tt);
-      else row_map_transpose_kernel<V, false, 0><<<grid, 256, 0, st>>>(p, tt);
+      with_bool(from_pack, [&](auto fp) { row_map_transpose_kernel<V, decltype(fp)::value, 0><<<grid, 256, 0, st>>>(p, tt); });
     }
     return;
   }
@@ -1304,9 +1302,8 @@ static void launch_narrow(RowMapParams& p, int64_t rows, cudaStream_t st) {
   const unsigned nb = (unsigned)blocks;
   if (searched) {
     // ... with many short sequences: a warp per 32 sequences (no per-tile decode chain)
-    static const int64_t ws_min = [] { const char* e = getenv("RUA_WARPSEG_MIN_S"); return e ? atoll(e) : 32768ll; }();
-    if (p.d.layout == RUA_CAT && p.row_vecs == 1 && ((uintptr_t)p.dst & (4 * sizeof(V) - 1)) == 0 && p.rg.B >= ws_min &&
-        rows <= 256 * p.rg.B && (srck == RUA_LEFT || srck == RUA_RIGHT || srck == kSrcCatRev || srck == kSrcCatRoll)) {
+    if (p.d.layout == RUA_CAT && p.row_vecs == 1 && ((uintptr_t)p.dst & (4 * sizeof(V) - 1)) == 0 &&
+        warpseg_applies(rows, p.rg.B) && (srck == RUA_LEFT || srck == RUA_RIGHT || srck == kSrcCatRev || srck == kSrcCatRoll)) {
       const unsigned wb = (unsigned)ceil_div(p.rg.B, (int64_t)kWcWarps * 32);
       switch (srck) {
         case RUA_LEFT: row_map_warpseg_cat1_kernel<V, RUA_LEFT><<<wb, kWcThreads, 0, st>>>(p); break;
@@ -1364,14 +1361,39 @@ static void launch_narrow(RowMapParams& p, int64_t rows, cudaStream_t st) {
   }
 }
 
+// widest vector of at most `max_vec` bytes that divides every address and size OR-ed into `align`
+static int vec_width(uintptr_t align, int max_vec) {
+  int vec = max_vec;
+  while (vec > 1 && (align & (uintptr_t)(vec - 1))) vec >>= 1;
+  return vec;
+}
+
+// Launch plan of the wide-row kernels (row_map / list / multi): the vector width (up to max_vec bytes, 256-bit words only
+// for rows of 128 bytes or more), lanes per row (short rows share a warp, 32 / lanes_per_row rows move concurrently),
+// and rows per warp / column splits that keep ~32 warps per SM in flight when the problem allows it.  Fills those fields
+// of p and returns the vector width in bytes; *blocks gets the number of kRowMapThreads-thread CTAs.
+static int plan_wide(RowMapParams& p, uintptr_t align, int64_t row_bytes, int64_t rows, int max_vec, int64_t* blocks) {
+  const int vec = vec_width(align, row_bytes >= 128 ? max_vec : 16);
+  p.row_vecs = row_bytes / vec;
+  int lpr = 1;
+  while (lpr < 32 && lpr < p.row_vecs) lpr <<= 1;  // smallest power of two covering the row, <= 32
+  p.lanes_per_row = lpr;
+  const int64_t target_warps = (int64_t)kNumSMs * 32;
+  int rpw = 32;
+  while (rpw > 32 / lpr && rpw > 1 && ceil_div(rows, rpw) < target_warps) rpw >>= 1;
+  p.rows_per_warp = rpw;
+  const int64_t warps = ceil_div(rows, rpw);
+  int splits = 1;
+  while (warps * splits < target_warps && p.row_vecs / (splits * 2) >= 32 * kUnroll && splits < 64) splits *= 2;
+  p.col_splits = splits;
+  *blocks = ceil_div(warps, kRowMapThreads / 32);
+  return vec;
+}
+
 static int launch_row_map(RowMapParams& p, int64_t row_bytes, int64_t rows, cudaStream_t st) {
   if (rows <= 0 || row_bytes <= 0) return RUA_OK;
-  // widest vector that divides the row size and both base addresses
-  uintptr_t a = (uintptr_t)p.src | (uintptr_t)p.dst | (uintptr_t)row_bytes;
-  static const bool use256 = [] { const char* e = getenv("RUA_VEC256"); return !(e && e[0] == '0'); }();
-  int vec = (use256 && row_bytes >= 128) ? 32 : 16;   // 256-bit accesses only in the wide-row kernel
-  while (vec > 1 && (a & (uintptr_t)(vec - 1))) vec >>= 1;
-  p.row_vecs = row_bytes / vec;
+  // the vector must divide the row size and both base addresses
+  const uintptr_t a = (uintptr_t)p.src | (uintptr_t)p.dst | (uintptr_t)row_bytes;
 
   // C <-> L/R conversions of 128..255-byte rows also take the narrow path: its four-vectors-per-thread kernels treat a
   // sequence as one contiguous run of vectors and beat the row-per-lane-group kernel there (128-byte rows: L -> C
@@ -1382,81 +1404,37 @@ static int launch_row_map(RowMapParams& p, int64_t row_bytes, int64_t rows, cuda
                            (p.d.layout == RUA_CAT && (p.s.layout == RUA_LEFT || p.s.layout == RUA_RIGHT));
   const bool run_copy = simple_map && padded_side && row_bytes < 512 && (a & 15u) == 0 && ((uintptr_t)p.dst & 63u) == 0 &&
                         !p.mask_out;   // the fused mask lives in the wide-row kernel
-  if (run_copy && row_bytes >= 128) {
-    vec = 16;
-    p.row_vecs = row_bytes / vec;
-  }
   if (row_bytes < 128 || run_copy) {  // narrow rows: tile kernels (segment offsets staged in shared memory)
     if (p.mask_out) return RUA_ERR_UNSUPPORTED;   // callers launch rua_mask separately for narrow rows
+    const int vec = vec_width(a, 16);
+    p.row_vecs = row_bytes / vec;
     if (ceil_div(rows * p.row_vecs, kTileVecs) >= (1ll << 31)) return RUA_ERR_UNSUPPORTED;
-    switch (vec) {
-      case 16: launch_narrow<uint4>(p, rows, st); break;
-      case 8: launch_narrow<uint2>(p, rows, st); break;
-      case 4: launch_narrow<unsigned int>(p, rows, st); break;
-      case 2: launch_narrow<unsigned short>(p, rows, st); break;
-      default: launch_narrow<unsigned char>(p, rows, st); break;
-    }
+    with_word(vec, [&](auto w) {
+      using W = typename decltype(w)::type;
+      if constexpr (sizeof(W) <= 16) launch_narrow<W>(p, rows, st);   // 256-bit words only in the wide-row kernel
+    });
     return check_launch();
   }
 
-  // lanes per row: short rows share a warp (32/lpr rows move concurrently)
-  int lpr = 1;
-  while (lpr < 32 && lpr < p.row_vecs) lpr <<= 1;  // smallest power of two covering the row, <= 32
-  p.lanes_per_row = lpr;
-
-  // rows per warp / column splits: keep >= ~32 warps per SM in flight when the problem allows it
-  const int64_t target_warps = (int64_t)kNumSMs * 32;
-  int rpw = 32;
-  while (rpw > 32 / lpr && rpw > 1 && ceil_div(rows, rpw) < target_warps) rpw >>= 1;
-  p.rows_per_warp = rpw;
-  int64_t warps = ceil_div(rows, rpw);
-  int splits = 1;
-  while (warps * splits < target_warps && p.row_vecs / (splits * 2) >= 32 * kUnroll && splits < 64) splits *= 2;
-  p.col_splits = splits;
-
-  int64_t blocks = ceil_div(warps, kRowMapThreads / 32);
+  static const bool use256 = knob("RUA_VEC256", 1) != 0;
+  int64_t blocks;
+  const int vec = plan_wide(p, a, row_bytes, rows, use256 ? 32 : 16, &blocks);
   if (blocks >= (1ll << 31)) return RUA_ERR_UNSUPPORTED;
-  dim3 grid((unsigned)blocks, (unsigned)splits);
-  switch (vec) {
-    case 32: row_map_kernel<V256><<<grid, kRowMapThreads, 0, st>>>(p); break;
-    case 16: row_map_kernel<uint4><<<grid, kRowMapThreads, 0, st>>>(p); break;
-    case 8: row_map_kernel<uint2><<<grid, kRowMapThreads, 0, st>>>(p); break;
-    case 4: row_map_kernel<unsigned int><<<grid, kRowMapThreads, 0, st>>>(p); break;
-    case 2: row_map_kernel<unsigned short><<<grid, kRowMapThreads, 0, st>>>(p); break;
-    default: row_map_kernel<unsigned char><<<grid, kRowMapThreads, 0, st>>>(p); break;
-  }
+  const dim3 grid((unsigned)blocks, (unsigned)p.col_splits);
+  with_word(vec, [&](auto w) { row_map_kernel<typename decltype(w)::type><<<grid, kRowMapThreads, 0, st>>>(p); });
   return check_launch();
 }
 
 static int launch_row_map_list(RowMapParams& p, const uint8_t* const* src_list, int src_align, int64_t row_bytes,
                                int64_t rows, cudaStream_t st, const int64_t* bases = nullptr, int n_src = 0) {
   if (rows <= 0 || row_bytes <= 0) return RUA_OK;
-  uintptr_t a = (uintptr_t)p.dst | (uintptr_t)row_bytes | (uintptr_t)src_align;
-  int vec = row_bytes >= 128 ? 32 : 16;
-  while (vec > 1 && (a & (uintptr_t)(vec - 1))) vec >>= 1;
-  p.row_vecs = row_bytes / vec;
-  int lpr = 1;
-  while (lpr < 32 && lpr < p.row_vecs) lpr <<= 1;
-  p.lanes_per_row = lpr;
-  const int64_t target_warps = (int64_t)kNumSMs * 32;
-  int rpw = 32;
-  while (rpw > 32 / lpr && rpw > 1 && ceil_div(rows, rpw) < target_warps) rpw >>= 1;
-  p.rows_per_warp = rpw;
-  const int64_t warps = ceil_div(rows, rpw);
-  int splits = 1;
-  while (warps * splits < target_warps && p.row_vecs / (splits * 2) >= 32 * kUnroll && splits < 64) splits *= 2;
-  p.col_splits = splits;
-  const int64_t blocks = ceil_div(warps, kRowMapThreads / 32);
+  int64_t blocks;
+  const int vec = plan_wide(p, (uintptr_t)p.dst | (uintptr_t)row_bytes | (uintptr_t)src_align, row_bytes, rows, 32, &blocks);
   if (blocks >= (1ll << 31)) return RUA_ERR_UNSUPPORTED;
-  dim3 grid((unsigned)blocks, (unsigned)splits);
-  switch (vec) {
-    case 32: row_map_list_kernel<V256><<<grid, kRowMapThreads, 0, st>>>(p, src_list, row_bytes, bases, n_src); break;
-    case 16: row_map_list_kernel<uint4><<<grid, kRowMapThreads, 0, st>>>(p, src_list, row_bytes, bases, n_src); break;
-    case 8: row_map_list_kernel<uint2><<<grid, kRowMapThreads, 0, st>>>(p, src_list, row_bytes, bases, n_src); break;
-    case 4: row_map_list_kernel<unsigned int><<<grid, kRowMapThreads, 0, st>>>(p, src_list, row_bytes, bases, n_src); break;
-    case 2: row_map_list_kernel<unsigned short><<<grid, kRowMapThreads, 0, st>>>(p, src_list, row_bytes, bases, n_src); break;
-    default: row_map_list_kernel<unsigned char><<<grid, kRowMapThreads, 0, st>>>(p, src_list, row_bytes, bases, n_src); break;
-  }
+  const dim3 grid((unsigned)blocks, (unsigned)p.col_splits);
+  with_word(vec, [&](auto w) {
+    row_map_list_kernel<typename decltype(w)::type><<<grid, kRowMapThreads, 0, st>>>(p, src_list, row_bytes, bases, n_src);
+  });
   return check_launch();
 }
 
@@ -1466,35 +1444,15 @@ static int launch_row_map_multi(RowMapParams& p, const MultiDst& m, int64_t row_
   for (int k = 0; k < m.n; ++k) a |= (uintptr_t)m.dst[k];
   // (a TMA bulk-copy variant of this kernel -- one cp.async.bulk per row and destination -- measured 25.6-26.3 ms vs 25.3 ms
   //  at 8 GPUs: the wire, not the store shape, bounds it; profiles/r2_gather_sweep.md)
-  int vec = row_bytes >= 128 ? 32 : 16;
-  while (vec > 1 && (a & (uintptr_t)(vec - 1))) vec >>= 1;
-  p.row_vecs = row_bytes / vec;
-  int lpr = 1;
-  while (lpr < 32 && lpr < p.row_vecs) lpr <<= 1;
-  p.lanes_per_row = lpr;
-  const int64_t target_warps = (int64_t)kNumSMs * 32;
-  int rpw = 32;
-  while (rpw > 32 / lpr && rpw > 1 && ceil_div(rows, rpw) < target_warps) rpw >>= 1;
-  p.rows_per_warp = rpw;
-  const int64_t warps = ceil_div(rows, rpw);
-  int splits = 1;
-  while (warps * splits < target_warps && p.row_vecs / (splits * 2) >= 32 * kUnroll && splits < 64) splits *= 2;
-  p.col_splits = splits;
-  int64_t blocks = ceil_div(warps, kRowMapThreads / 32);
+  int64_t blocks;
+  const int vec = plan_wide(p, a, row_bytes, rows, 32, &blocks);
   // wire-bound (>= 4 destinations, i.e. >= 2 peers beside the local window and copy): cap the grid so that other streams'
   // kernels find free CTA slots on every SM; RUA_MULTI_CTAS_PER_SM overrides (0 = no cap)
-  static const int cap_per_sm = [] { const char* e = getenv("RUA_MULTI_CTAS_PER_SM"); return e ? atoi(e) : 4; }();
+  static const int64_t cap_per_sm = knob("RUA_MULTI_CTAS_PER_SM", 4);
   if (m.n >= 4 && cap_per_sm > 0 && blocks > (int64_t)kNumSMs * cap_per_sm) blocks = (int64_t)kNumSMs * cap_per_sm;
   if (blocks >= (1ll << 31)) return RUA_ERR_UNSUPPORTED;
-  dim3 grid((unsigned)blocks, (unsigned)splits);
-  switch (vec) {
-    case 32: row_map_multi_kernel<V256><<<grid, kRowMapThreads, 0, st>>>(p, m); break;
-    case 16: row_map_multi_kernel<uint4><<<grid, kRowMapThreads, 0, st>>>(p, m); break;
-    case 8: row_map_multi_kernel<uint2><<<grid, kRowMapThreads, 0, st>>>(p, m); break;
-    case 4: row_map_multi_kernel<unsigned int><<<grid, kRowMapThreads, 0, st>>>(p, m); break;
-    case 2: row_map_multi_kernel<unsigned short><<<grid, kRowMapThreads, 0, st>>>(p, m); break;
-    default: row_map_multi_kernel<unsigned char><<<grid, kRowMapThreads, 0, st>>>(p, m); break;
-  }
+  const dim3 grid((unsigned)blocks, (unsigned)p.col_splits);
+  with_word(vec, [&](auto w) { row_map_multi_kernel<typename decltype(w)::type><<<grid, kRowMapThreads, 0, st>>>(p, m); });
   return check_launch();
 }
 
@@ -1504,6 +1462,18 @@ static bool valid_side(const rua_side_t* s) {
   if (s->len_xform < RUA_LEN_SAME || s->len_xform > RUA_LEN_MINUS) return false;
   if ((s->layout == RUA_LEFT || s->layout == RUA_RIGHT) && s->width <= 0 && s->rows > 0) return false;
   return s->rows >= 0;
+}
+
+// the padding value: fill_bytes = 0 (zeros), or a pattern of 1, 2, 4, 8 or 16 bytes at fill_host that divides the row,
+// replicated over 16 bytes into p.fill
+static int set_fill(RowMapParams& p, const void* fill_host, int32_t fill_bytes, int64_t row_bytes) {
+  if (fill_bytes != 0 && fill_bytes != 1 && fill_bytes != 2 && fill_bytes != 4 && fill_bytes != 8 && fill_bytes != 16)
+    return RUA_ERR_INVALID;
+  if (fill_bytes > 0 && (!fill_host || row_bytes % fill_bytes != 0)) return RUA_ERR_INVALID;
+  uint8_t pat[16] = {0};
+  for (int k = 0; fill_bytes > 0 && k < 16; ++k) pat[k] = ((const uint8_t*)fill_host)[k % fill_bytes];
+  memcpy(&p.fill, pat, sizeof(pat));
+  return RUA_OK;
 }
 
 }  // namespace rua
@@ -1523,12 +1493,8 @@ int rua_row_map(const void* src, void* dst, int64_t row_bytes, const rua_ragged_
   bool uses_pack = src_side->layout == RUA_PACK || dst_side->layout == RUA_PACK;
   if (uses_pack && (!ragged->poff || !ragged->sorted || !ragged->unsorted)) return RUA_ERR_INVALID;
   if (!src && src_side->rows > 0) return RUA_ERR_INVALID;
-  if (fill_bytes != 0 && fill_bytes != 1 && fill_bytes != 2 && fill_bytes != 4 && fill_bytes != 8 &&
-      fill_bytes != 16)
-    return RUA_ERR_INVALID;
-  if (fill_bytes > 0 && (!fill_host || row_bytes % fill_bytes != 0)) return RUA_ERR_INVALID;
-
   RowMapParams p{};
+  if (int rc = set_fill(p, fill_host, fill_bytes, row_bytes)) return rc;
   p.src = (const uint8_t*)src;
   p.dst = (uint8_t*)dst;
   p.rg = *ragged;
@@ -1537,10 +1503,6 @@ int rua_row_map(const void* src, void* dst, int64_t row_bytes, const rua_ragged_
   p.tmap = tmap;
   p.tmap_arg = tmap_arg;
   p.pad_mode = pad_mode;
-  uint8_t pat[16] = {0};
-  if (fill_bytes > 0)
-    for (int k = 0; k < 16; ++k) pat[k] = ((const uint8_t*)fill_host)[k % fill_bytes];
-  p.fill = make_uint4(((uint32_t*)pat)[0], ((uint32_t*)pat)[1], ((uint32_t*)pat)[2], ((uint32_t*)pat)[3]);
   p.gather_index = nullptr;
   p.scatter_index = nullptr;
   return launch_row_map(p, row_bytes, dst_side->rows, (cudaStream_t)stream);
@@ -1559,10 +1521,8 @@ int rua_row_map_mask(const void* src, void* dst, int64_t row_bytes, const rua_ra
   bool uses_pack = src_side->layout == RUA_PACK;
   if (uses_pack && (!ragged->poff || !ragged->sorted || !ragged->unsorted)) return RUA_ERR_INVALID;
   if (!src && src_side->rows > 0) return RUA_ERR_INVALID;
-  if (fill_bytes != 0 && fill_bytes != 1 && fill_bytes != 2 && fill_bytes != 4 && fill_bytes != 8 && fill_bytes != 16)
-    return RUA_ERR_INVALID;
-  if (fill_bytes > 0 && (!fill_host || row_bytes % fill_bytes != 0)) return RUA_ERR_INVALID;
   RowMapParams p{};
+  if (int rc = set_fill(p, fill_host, fill_bytes, row_bytes)) return rc;
   p.src = (const uint8_t*)src;
   p.dst = (uint8_t*)dst;
   p.rg = *ragged;
@@ -1570,10 +1530,6 @@ int rua_row_map_mask(const void* src, void* dst, int64_t row_bytes, const rua_ra
   p.d = *dst_side;
   p.tmap = RUA_MAP_SHIFT;
   p.pad_mode = RUA_PAD_FILL;
-  uint8_t pat[16] = {0};
-  if (fill_bytes > 0)
-    for (int k = 0; k < 16; ++k) pat[k] = ((const uint8_t*)fill_host)[k % fill_bytes];
-  p.fill = make_uint4(((uint32_t*)pat)[0], ((uint32_t*)pat)[1], ((uint32_t*)pat)[2], ((uint32_t*)pat)[3]);
   p.mask_out = mask_out;
   p.mask_elem = mask_elem_bytes;
   memcpy(&p.mask_zero, zero_host, mask_elem_bytes);
@@ -1664,18 +1620,12 @@ int rua_row_map_list(const void* const* src_list, int32_t src_align, void* dst, 
   if (src_align < 1 || (src_align & (src_align - 1))) return RUA_ERR_INVALID;
   if (dst_side->len_xform != RUA_LEN_SAME) return RUA_ERR_INVALID;
   if (dst_side->layout == RUA_PACK && (!ragged->poff || !ragged->sorted)) return RUA_ERR_INVALID;
-  if (fill_bytes != 0 && fill_bytes != 1 && fill_bytes != 2 && fill_bytes != 4 && fill_bytes != 8 && fill_bytes != 16)
-    return RUA_ERR_INVALID;
-  if (fill_bytes > 0 && (!fill_host || row_bytes % fill_bytes != 0)) return RUA_ERR_INVALID;
   RowMapParams p{};
+  if (int rc = set_fill(p, fill_host, fill_bytes, row_bytes)) return rc;
   p.dst = (uint8_t*)dst;
   p.rg = *ragged;
   p.d = *dst_side;
   p.s.layout = RUA_CAT;
-  uint8_t pat[16] = {0};
-  if (fill_bytes > 0)
-    for (int k = 0; k < 16; ++k) pat[k] = ((const uint8_t*)fill_host)[k % fill_bytes];
-  p.fill = make_uint4(((uint32_t*)pat)[0], ((uint32_t*)pat)[1], ((uint32_t*)pat)[2], ((uint32_t*)pat)[3]);
   return launch_row_map_list(p, (const uint8_t* const*)src_list, src_align, row_bytes, dst_side->rows, (cudaStream_t)stream);
 }
 

@@ -487,34 +487,39 @@ struct Plan {
   size_t state_bytes, flag_bytes, total;
 };
 
-template <typename T> int vec_of() { return sizeof(T) == 8 ? 2 : (sizeof(T) == 4 ? 4 : 8); }
-int elem_bytes(int32_t dtype) { return dtype == RUA_F64 ? 8 : (dtype == RUA_F32 ? 4 : 2); }
-
-template <class Op> size_t state_size() { return sizeof(typename Op::S); }
-
-size_t state_bytes_of(Kind kind, int32_t dtype) {
-  const bool dbl = dtype == RUA_F64;
-  switch (kind) {
-    case K_SUM: case K_LSE: return dbl ? 8 : 4;
-    case K_MAX: case K_MIN: return dbl ? 16 : 8;
-    case K_LSE_BWD: return dbl ? 16 : 8;
-    default: return dbl ? 16 : 8;
-  }
+// f(Type<Op>{}) for the operator of `kind` on `dtype`, at the full 16-byte vector when `vec` allows it and H is a
+// multiple of it, else one element per thread
+template <typename F> int with_scan_op(Kind kind, int32_t dtype, bool vec, int64_t H, F&& f) {
+  return with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    auto at = [&](auto v) {
+      constexpr int V = decltype(v)::value;
+      switch (kind) {
+        case K_SUM: return f(Type<OpSum<T, V>>{});
+        case K_LSE: return f(Type<OpLse<T, V>>{});
+        case K_MAX: return f(Type<OpExt<T, V, true>>{});
+        case K_MIN: return f(Type<OpExt<T, V, false>>{});
+        case K_LSE_BWD: return f(Type<OpLseBwd<T, V>>{});
+        default: return f(Type<OpRunBwd<T, V>>{});
+      }
+    };
+    constexpr int VV = 16 / sizeof(T);
+    if (!vec || H % VV != 0) return at(Int<1>{});
+    return at(Int<VV>{});
+  });
 }
-int rows_per_group(Kind kind) { return kind == K_LSE_BWD ? 4 : (kind == K_SUM || kind == K_LSE ? 16 : 8); }
 
-Plan make_plan(Kind kind, int32_t dtype, int64_t rows, int64_t H, bool vec) {
+template <class Op> Plan make_plan(int64_t rows, int64_t H) {
   Plan p{};
-  const int vmax = 16 / elem_bytes(dtype);
-  p.V = vec && H % vmax == 0 ? vmax : 1;
+  p.V = Op::V;
   const int64_t vecs = ceil_div(H, p.V);
   int tpc = 1;
   while (tpc < kMaxTPC && tpc < vecs) tpc <<= 1;
   p.tpc_log2 = __builtin_ctz(tpc);
-  p.R = (kScanThreads / tpc) * rows_per_group(kind);
+  p.R = (kScanThreads / tpc) * Op::kRG;
   p.ncb = (int)ceil_div(vecs, tpc);
   p.chunks = ceil_div(rows, p.R);
-  p.state_bytes = state_bytes_of(kind, dtype);
+  p.state_bytes = sizeof(typename Op::S);
   p.flag_bytes = (size_t)ceil_div(16 + 4 * p.chunks * p.ncb, 256) * 256;
   const size_t slots = (size_t)p.chunks * p.ncb * tpc * p.V;
   p.total = p.flag_bytes + 2 * slots * p.state_bytes;
@@ -524,7 +529,6 @@ Plan make_plan(Kind kind, int32_t dtype, int64_t rows, int64_t H, bool vec) {
 bool aligned16(const void* p) { return p == nullptr || ((uintptr_t)p & 15) == 0; }
 
 template <class Op> int launch_op(const ScanArgs& a0, const Plan& p, cudaStream_t st) {
-  static_assert(sizeof(typename Op::S) <= 16, "state slots are sized by state_bytes_of");
   ScanArgs a = a0;
   a.tpc_log2 = p.tpc_log2;
   a.R = p.R;
@@ -538,22 +542,6 @@ template <class Op> int launch_op(const ScanArgs& a0, const Plan& p, cudaStream_
   const int64_t blocks = p.chunks * p.ncb;
   segscan_kernel<Op><<<(unsigned)blocks, kScanThreads, smem, st>>>(a);
   return check_launch();
-}
-
-template <typename T, int V> int launch_kind(Kind kind, const ScanArgs& a, const Plan& p, cudaStream_t st) {
-  switch (kind) {
-    case K_SUM: return launch_op<OpSum<T, V>>(a, p, st);
-    case K_LSE: return launch_op<OpLse<T, V>>(a, p, st);
-    case K_MAX: return launch_op<OpExt<T, V, true>>(a, p, st);
-    case K_MIN: return launch_op<OpExt<T, V, false>>(a, p, st);
-    case K_LSE_BWD: return launch_op<OpLseBwd<T, V>>(a, p, st);
-    default: return launch_op<OpRunBwd<T, V>>(a, p, st);
-  }
-}
-
-template <typename T> int launch_t(Kind kind, const ScanArgs& a, const Plan& p, cudaStream_t st) {
-  constexpr int VV = 16 / sizeof(T);
-  return p.V == 1 ? launch_kind<T, 1>(kind, a, p, st) : launch_kind<T, VV>(kind, a, p, st);
 }
 
 int validate(int64_t H, int32_t dtype, int32_t op, const rua_ragged_t* rg, const rua_side_t* side) {
@@ -577,32 +565,30 @@ int run(Kind kind, int32_t dtype, int64_t H, int32_t reverse, const rua_ragged_t
         ScanArgs a, bool vec, void* ws, size_t ws_bytes, rua_stream_t stream) {
   const int64_t rows = side->rows;
   if (rows == 0 || H == 0) return RUA_OK;
-  const Plan p = make_plan(kind, dtype, rows, H, vec);
-  if (!ws || ws_bytes < p.total) return RUA_ERR_WORKSPACE;
-  if (p.chunks * p.ncb > 0x7fffffffLL) return RUA_ERR_UNSUPPORTED;
-  a.H = H;
-  a.B = rg->B;
-  a.off = rg->off;
-  a.poff = rg->poff;
-  a.unsorted = rg->unsorted;
-  a.layout = side->layout;
-  a.reverse = reverse ? 1 : 0;
-  a.W = side->width;
-  a.rows = rows;
-  unsigned char* w = static_cast<unsigned char*>(ws);
-  a.ticket = reinterpret_cast<unsigned long long*>(w);
-  a.flags = reinterpret_cast<int*>(w + 16);
-  const size_t slots = p.total - p.flag_bytes;
-  a.agg = w + p.flag_bytes;
-  a.inc = w + p.flag_bytes + slots / 2;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (int rc = check_cuda(cudaMemsetAsync(ws, 0, p.flag_bytes, st))) return rc;
-  switch (dtype) {
-    case RUA_F32: return launch_t<float>(kind, a, p, st);
-    case RUA_F64: return launch_t<double>(kind, a, p, st);
-    case RUA_F16: return launch_t<__half>(kind, a, p, st);
-    default: return launch_t<__nv_bfloat16>(kind, a, p, st);
-  }
+  return with_scan_op(kind, dtype, vec, H, [&](auto op) {
+    using Op = typename decltype(op)::type;
+    const Plan p = make_plan<Op>(rows, H);
+    if (!ws || ws_bytes < p.total) return (int)RUA_ERR_WORKSPACE;
+    if (p.chunks * p.ncb > 0x7fffffffLL) return (int)RUA_ERR_UNSUPPORTED;
+    a.H = H;
+    a.B = rg->B;
+    a.off = rg->off;
+    a.poff = rg->poff;
+    a.unsorted = rg->unsorted;
+    a.layout = side->layout;
+    a.reverse = reverse ? 1 : 0;
+    a.W = side->width;
+    a.rows = rows;
+    unsigned char* w = static_cast<unsigned char*>(ws);
+    a.ticket = reinterpret_cast<unsigned long long*>(w);
+    a.flags = reinterpret_cast<int*>(w + 16);
+    const size_t slots = p.total - p.flag_bytes;
+    a.agg = w + p.flag_bytes;
+    a.inc = w + p.flag_bytes + slots / 2;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (int rc = check_cuda(cudaMemsetAsync(ws, 0, p.flag_bytes, st))) return rc;
+    return launch_op<Op>(a, p, st);
+  });
 }
 
 Kind forward_kind(int32_t op) {
@@ -622,8 +608,14 @@ extern "C" size_t rua_segment_scan_workspace_bytes(int64_t rows, int64_t H, int3
   if (rows < 0 || H < 0 || dtype < RUA_F32 || dtype > RUA_BF16 || op < RUA_SCAN_SUM || op > RUA_SCAN_MIN) return 0;
   if (rows == 0 || H == 0) return 0;
   const Kind kind = backward ? backward_kind(op) : forward_kind(op);
-  const Plan a = make_plan(kind, dtype, rows, H, true), b = make_plan(kind, dtype, rows, H, false);
-  return a.total > b.total ? a.total : b.total;
+  size_t total = 0;
+  for (bool vec : {true, false})
+    with_scan_op(kind, dtype, vec, H, [&](auto o) {
+      const size_t t = make_plan<typename decltype(o)::type>(rows, H).total;
+      total = t > total ? t : total;
+      return RUA_OK;
+    });
+  return total;
 }
 
 extern "C" int rua_segment_scan(const void* src, void* dst, int64_t* idx_out, int64_t H, int32_t dtype, int32_t op,
