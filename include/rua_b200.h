@@ -327,6 +327,40 @@ int rua_segment_scan_backward(const void* grad_out, const void* x, const void* y
                               const rua_side_t* side, void* ws, size_t ws_bytes, rua_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------- */
+/* K8  per-sequence depthwise 1-D convolution (no counterpart in the reference; replaces the     */
+/* pad -> F.conv1d(groups=H) on (B, H, T) -> unpad composition, and F.conv1d straight on the     */
+/* storage, which mixes every sequence's first and last K-1 outputs with its neighbours)         */
+/* ------------------------------------------------------------------------------------------- */
+/* workspace of rua_segment_conv (backward = 0: always 0) / rua_segment_conv_backward (backward = 1) over rows = side->rows
+ * rows of H elements with K taps: a fixed number of per-CTA slots of partial weight / bias gradients, capped whatever
+ * rows is (monotone in rows, bounded).  Host only; 0 when an argument is invalid. */
+size_t rua_segment_conv_workspace_bytes(int64_t rows, int64_t H, int32_t K, int32_t dtype, int32_t backward);
+
+/* src / dst: side->rows rows of H elements in the storage of `side` (C, L, P or R over `ragged`; len_xform must be
+ * RUA_LEN_SAME); weight (H, K) row-major, bias (H) or NULL, both of the payload dtype.  For token (i, t) of sequence i with
+ * length len[i] (rows from the "Row of token" formulas above), 1 <= K <= 32, 0 <= pad <= K - 1:
+ *   dst(i, t, h) = bias[h] + sum_{k<K} weight[h, k] * src(i, t + k - pad, h),   src(i, s, .) = 0 for s outside [0, len[i])
+ * pad = K - 1 is causal (weight[:, K-1] multiplies the current token), pad = (K - 1) / 2 is torch's padding='same'.
+ * Rows that hold no token (L / R padding, C rows at or past off[B]) are copied through.  fp32 accumulation (fp64 for
+ * RUA_F64), one rounding.  No workspace (ws may be NULL). */
+int rua_segment_conv(const void* src, const void* weight, const void* bias, void* dst, int64_t H, int32_t dtype, int32_t K,
+                     int32_t pad, const rua_ragged_t* ragged, const rua_side_t* side, void* ws, size_t ws_bytes,
+                     rua_stream_t stream);
+
+/* gradients of rua_segment_conv with the same weight / H / dtype / K / pad / ragged / side; x = the forward input.
+ *   grad_in: the same convolution of grad_out with the taps flipped and pad' = K - 1 - pad; rows that hold no token pass
+ *            grad_out through (every row written);
+ *   grad_weight[h, k] = sum over tokens (i, t) with 0 <= t + k - pad < len[i] of grad_out(i, t, h) * x(i, t + k - pad, h);
+ *   grad_bias[h] = sum over tokens of grad_out(i, t, h).
+ * Any of grad_in / grad_weight / grad_bias may be NULL and is then not computed (x may be NULL without grad_weight).
+ * Deterministic: every CTA sums its chunks into its own workspace slot in a fixed order (no atomics), and a second kernel
+ * sums the slots in slot order, so grad_weight / grad_bias are bit-identical run to run.  ws:
+ * rua_segment_conv_workspace_bytes(side->rows, H, K, dtype, 1) bytes when grad_weight or grad_bias is wanted. */
+int rua_segment_conv_backward(const void* grad_out, const void* x, const void* weight, void* grad_in, void* grad_weight,
+                              void* grad_bias, int64_t H, int32_t dtype, int32_t K, int32_t pad, const rua_ragged_t* ragged,
+                              const rua_side_t* side, void* ws, size_t ws_bytes, rua_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------- */
 /* K5  multi-GPU output gather over NVLink peer memory (SURVEY.md 8e-3; the reference is         */
 /* single-device).  One process per GPU; the batch is sharded by sequence; every rank stores its */
 /* rows directly into the output buffers ("windows") of all ranks of the node.                   */

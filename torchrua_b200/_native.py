@@ -1307,6 +1307,127 @@ def segment_scan(data: Tensor, rg: Ragged, side: SideSpec, op: str, reverse: boo
 
 
 # ------------------------------------------------------------------------------------------------
+# K8: per-sequence depthwise 1-D convolution (+ autograd)
+# ------------------------------------------------------------------------------------------------
+CONV_MAX_K = 32
+
+
+def conv_check(data: Tensor, weight: Tensor, bias: Optional[Tensor], feat: Tuple[int, ...], padding) -> int:
+    """validate a depthwise convolution of rows with features ``feat`` -> pad (positions before the current token)."""
+    if data.dtype not in _DTYPES:
+        raise RuntimeError(f'torchrua_b200: depthwise_conv1d supports float16/bfloat16/float32/float64, got {data.dtype}')
+    for name, t in (('weight', weight), ('bias', bias)):
+        if t is not None and t.dtype != data.dtype:
+            raise RuntimeError(f'torchrua_b200: depthwise_conv1d {name} has dtype {t.dtype}, the input {data.dtype}')
+    if weight.dim() != len(feat) + 1 or tuple(weight.shape[:-1]) != tuple(feat):
+        raise ValueError(f'torchrua_b200: depthwise_conv1d weight must be (*feat, K) = {tuple(feat)} + (K,), '
+                         f'got {tuple(weight.shape)}')
+    K = weight.shape[-1]
+    if not 1 <= K <= CONV_MAX_K:
+        raise ValueError(f'torchrua_b200: depthwise_conv1d supports kernel sizes 1..{CONV_MAX_K}, got {K}')
+    if bias is not None and tuple(bias.shape) != tuple(feat):
+        raise ValueError(f'torchrua_b200: depthwise_conv1d bias must be {tuple(feat)}, got {tuple(bias.shape)}')
+    if padding == 'causal':
+        padding = K - 1
+    elif padding == 'same':
+        padding = (K - 1) // 2
+    elif isinstance(padding, bool) or not isinstance(padding, int) or not 0 <= padding <= K - 1:
+        raise ValueError(f"torchrua_b200: depthwise_conv1d padding must be 'causal', 'same' or an int in [0, {K - 1}], "
+                         f'got {padding!r}')
+    require_cuda(data, weight, bias)
+    return padding
+
+
+def _conv_raw(data: Tensor, weight: Tensor, bias: Optional[Tensor], pad: int, rg: Ragged, side: SideSpec) -> Tensor:
+    """y laid out like data; data (side.rows, *feat), weight (H, K), bias (H,) or None, all contiguous."""
+    lib = _lib.load()
+    out = torch.empty_like(data)
+    if out.numel() == 0:
+        return out
+    H, K = weight.shape
+    dt = _DTYPES[data.dtype]
+    c_rg, c_side = rg.c_struct(), side.c_struct()
+    with _on(data.device):
+        prof = _profile_begin()
+        _lib.check(lib.rua_segment_conv(data.data_ptr(), weight.data_ptr(), _ptr(bias), out.data_ptr(), H, dt, K, pad,
+                                        ctypes.byref(c_rg), ctypes.byref(c_side), None, 0, _stream()), 'rua_segment_conv')
+        if prof is not None:
+            # every row read once and written once + the taps (and bias) + the metadata consulted
+            e = data.element_size()
+            nb = 2 * data.numel() * e + (K + (bias is not None)) * H * e
+            _profile_end(prof, 'segment_conv', nb + 8 * rg.B + (8 * (rg.Tp + rg.B) if side.layout == PACK else 0))
+    return out
+
+
+def _conv_backward_raw(g: Tensor, x: Tensor, weight: Tensor, pad: int, rg: Ragged, side: SideSpec, want_in: bool,
+                       want_w: bool, want_b: bool):
+    """(grad_in, grad_weight, grad_bias), None where not wanted; g, x (side.rows, *feat) contiguous."""
+    lib = _lib.load()
+    H, K = weight.shape
+    gi = torch.empty_like(g) if want_in else None
+    gw = torch.empty_like(weight) if want_w else None
+    gb = torch.empty(H, dtype=g.dtype, device=g.device) if want_b else None
+    if g.numel() == 0:
+        if gw is not None:
+            gw.zero_()
+        if gb is not None:
+            gb.zero_()
+        return gi, gw, gb
+    dt = _DTYPES[g.dtype]
+    c_rg, c_side = rg.c_struct(), side.c_struct()
+    with _on(g.device):
+        nbytes = lib.rua_segment_conv_workspace_bytes(side.rows, H, K, dt, 1) if (want_w or want_b) else 0
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=g.device)
+        prof = _profile_begin()
+        _lib.check(lib.rua_segment_conv_backward(g.data_ptr(), _ptr(x) if want_w else None, weight.data_ptr(), _ptr(gi),
+                                                 _ptr(gw), _ptr(gb), H, dt, K, pad, ctypes.byref(c_rg),
+                                                 ctypes.byref(c_side), ws.data_ptr() if nbytes else None, nbytes,
+                                                 _stream()), 'rua_segment_conv_backward')
+        if prof is not None:
+            # grad_out read once, x read once (grad_weight), grad_in written once + taps and their gradients
+            e = g.element_size()
+            nb = g.numel() * e * (1 + want_w + want_in) + (2 * K + 1) * H * e
+            _profile_end(prof, 'segment_conv_backward', nb + 8 * rg.B + (8 * (rg.Tp + rg.B) if side.layout == PACK else 0))
+    return gi, gw, gb
+
+
+class _SegmentConv(torch.autograd.Function):
+    """once-differentiable: the backward is a native kernel, double backward is not supported."""
+
+    @staticmethod
+    def forward(ctx, data: Tensor, weight: Tensor, bias: Optional[Tensor], pad: int, rg: Ragged, side: SideSpec):
+        x = data.detach().contiguous()
+        w = weight.detach().reshape(-1, weight.shape[-1]).contiguous()
+        b = None if bias is None else bias.detach().reshape(-1).contiguous()
+        ctx.meta = (pad, rg, side, weight.shape, None if bias is None else bias.shape)
+        ctx.save_for_backward(x if ctx.needs_input_grad[1] else None, w)   # x only feeds grad_weight
+        return _conv_raw(x, w, b, pad, rg, side)
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_out: Tensor):
+        pad, rg, side, wshape, bshape = ctx.meta
+        x, w = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        gi, gw, gb = _conv_backward_raw(grad_out.contiguous(), x, w, pad, rg, side, need[0], need[1],
+                                        need[2] and bshape is not None)
+        return (gi, None if gw is None else gw.view(wshape), None if gb is None else gb.view(bshape),
+                None, None, None)
+
+
+def segment_conv(data: Tensor, weight: Tensor, bias: Optional[Tensor], padding, rg: Ragged, side: SideSpec) -> Tensor:
+    """per-sequence depthwise convolution of the flattened storage ``data`` (side.rows, *feat); weight (*feat, K)."""
+    pad = conv_check(data, weight, bias, tuple(data.shape[1:]), padding)
+    grad = torch.is_grad_enabled() and (data.requires_grad or weight.requires_grad or
+                                        (bias is not None and bias.requires_grad))
+    if grad:
+        return _SegmentConv.apply(data, weight, bias, pad, rg, side)
+    w = weight.reshape(-1, weight.shape[-1]).contiguous()
+    b = None if bias is None else bias.reshape(-1).contiguous()
+    return _conv_raw(data if data.is_contiguous() else data.contiguous(), w, b, pad, rg, side)
+
+
+# ------------------------------------------------------------------------------------------------
 # scatter_*: stable sort of the index + bucket boundaries + segment reduce over GATHERED rows
 # ------------------------------------------------------------------------------------------------
 def sort_keys(keys: Tensor, max_key: int) -> Tuple[Tensor, Tensor]:

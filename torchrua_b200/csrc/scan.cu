@@ -33,6 +33,7 @@
 //   cummax / cummin backward, in reverse scan order: grad x_k = sum of g_j over the run of positions whose index is k
 //              (the run starts at j = k).  S = (acc, pass) with pass = 0 at a run start: an affine map with slope 0/1.
 #include "reduce_common.cuh"
+#include "seq_decode.cuh"
 
 namespace rua {
 namespace {
@@ -257,28 +258,11 @@ __device__ __forceinline__ void st_release(int* p, int v) {
 // row decode of virtual position j: storage row, position within the sequence, flags
 __device__ __forceinline__ void decode_row(const ScanArgs& a, int64_t j, int64_t n_tok, int64_t lo, int64_t hi,
                                            int64_t& srow, int64_t& t, uint8_t& fl) {
-  srow = j;
-  t = 0;
   fl = 0;
-  int64_t len;
-  if (a.layout == RUA_LEFT || a.layout == RUA_RIGHT) {
-    const int64_t i = j / a.W, c = j - i * a.W;
-    len = __ldg(a.off + i + 1) - __ldg(a.off + i);
-    t = a.layout == RUA_LEFT ? c : c - (a.W - len);
-    if (t < 0 || t >= len) return;
-  } else {
-    if (j >= n_tok) return;
-    while (hi - lo > 1) {   // owner of j among the sequences [lo, hi) that meet this chunk
-      const int64_t mid = (lo + hi) >> 1;
-      if (__ldg(a.off + mid) <= j) lo = mid; else hi = mid;
-    }
-    const int64_t o = __ldg(a.off + lo);
-    len = __ldg(a.off + lo + 1) - o;
-    t = j - o;
-    if (a.layout == RUA_PACK) srow = __ldg(a.poff + t) + __ldg(a.unsorted + lo);
-  }
-  const int64_t first = a.reverse ? len - 1 : 0, last = a.reverse ? 0 : len - 1;
-  fl = kTok | (t == first ? kStart : 0) | (t == last ? kEnd : 0);
+  decode_position(a, j, n_tok, lo, hi, srow, t, [&](int64_t len) {
+    const int64_t first = a.reverse ? len - 1 : 0, last = a.reverse ? 0 : len - 1;
+    fl = kTok | (t == first ? kStart : 0) | (t == last ? kEnd : 0);
+  });
 }
 
 template <class Op>
@@ -309,14 +293,8 @@ __global__ void __launch_bounds__(kScanThreads, Op::kMinBlocks) segscan_kernel(S
   const int64_t n_tok = __ldg(a.off + a.B);
   const int64_t jlo = a.reverse ? a.rows - q0 - nq : q0;
   const int64_t jhi = a.reverse ? a.rows - 1 - q0 : q0 + nq - 1;
-  const bool search = (a.layout == RUA_CAT || a.layout == RUA_PACK) && jlo < n_tok;
-  if (search && warp < 2) {
-    const int64_t j = warp == 0 ? jlo : min(jhi, n_tok - 1);
-    const int64_t s = warp_owner_search(GlobalOff{a.off}, a.B, j, lane);
-    if (lane == 0) s_bounds[warp] = s;
-  }
-  __syncthreads();
-  const int64_t lo = search ? s_bounds[0] : 0, hi = search ? s_bounds[1] + 1 : 0;
+  int64_t lo, hi;
+  owner_bounds(a, n_tok, jlo, jhi, lane, warp, s_bounds, lo, hi);
   for (int q = tid; q < nq; q += kScanThreads) {
     const int64_t j = a.reverse ? a.rows - 1 - (q0 + q) : q0 + q;
     int64_t srow, t;
