@@ -326,6 +326,38 @@ int rua_segment_scan_backward(const void* grad_out, const void* x, const void* y
                               int64_t H, int32_t dtype, int32_t op, int32_t reverse, const rua_ragged_t* ragged,
                               const rua_side_t* side, void* ws, size_t ws_bytes, rua_stream_t stream);
 
+/* per-sequence gated linear recurrence, on the same kernel as the scans (an affine scan with state (m, b)).
+ * workspace of rua_segment_linrec (backward = 0) / rua_segment_linrec_backward (backward = 1) over side->rows = rows rows
+ * of H elements; 0 when there is nothing to do or an argument is invalid. */
+size_t rua_segment_linrec_workspace_bytes(int64_t rows, int64_t H, int32_t dtype, int32_t backward);
+
+/* x / gate / dst: side->rows rows of H elements in the storage of `side` (as rua_segment_scan), all of `dtype`; h0: B rows
+ * of H elements in sequence order (for P the index in ragged->off, not the sorted one), or NULL for a zero state.  For
+ * token (i, t) of sequence i with length len[i]:
+ *   dst(i, t) = gate(i, t) * dst(i, t-1) + x(i, t),  dst(i, -1)     = h0[i]     (reverse = 0)
+ *   dst(i, t) = gate(i, t) * dst(i, t+1) + x(i, t),  dst(i, len[i]) = h0[i]     (reverse = 1)
+ * Any real gate: 0 resets the state, 1 gives cumsum.  Rows that hold no token are copied through from x.  fp32
+ * accumulation (fp64 for RUA_F64), one rounding.  Deterministic: chunk carries are combined in chunk order.  Specified
+ * for finite inputs; non-finite values propagate, in a pattern that may differ from a sequential loop (0 * inf).
+ * ws: rua_segment_linrec_workspace_bytes(side->rows, H, dtype, 0) bytes; it is cleared by a memset on `stream`. */
+int rua_segment_linrec(const void* x, const void* gate, const void* h0, void* dst, int64_t H, int32_t dtype,
+                       int32_t reverse, const rua_ragged_t* ragged, const rua_side_t* side, void* ws, size_t ws_bytes,
+                       rua_stream_t stream);
+
+/* gradients of rua_segment_linrec with the same gate / h0 / reverse / ragged / side; y = the forward output, g = grad_out.
+ * In forward order, with g~(t) = g(t) + gate(t+1) g~(t+1) the whole adjoint of dst(t) (g~ = g at the last position):
+ *   grad_x(t)    = g~(t);
+ *   grad_gate(t) = g~(t) * y(t-1), with y(-1) = h0[i] (0 when h0 is NULL);
+ *   grad_h0[i]   = gate(0) * g~(0), 0 for an empty sequence.
+ * The kernel scans z(t) = gate(t) g~(t) against the forward direction; y(t-1) is read from its own row of the same
+ * sequence.  grad_x, grad_gate and grad_h0 may each be NULL and are then not computed; y is needed for grad_gate only.
+ * Rows that hold no token pass grad_out through to grad_x and get 0 in grad_gate.  Deterministic like the forward.
+ * ws: rua_segment_linrec_workspace_bytes(side->rows, H, dtype, 1) bytes. */
+int rua_segment_linrec_backward(const void* grad_out, const void* gate, const void* h0, const void* y, void* grad_x,
+                                void* grad_gate, void* grad_h0, int64_t H, int32_t dtype, int32_t reverse,
+                                const rua_ragged_t* ragged, const rua_side_t* side, void* ws, size_t ws_bytes,
+                                rua_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------- */
 /* K8  per-sequence depthwise 1-D convolution (no counterpart in the reference; replaces the     */
 /* pad -> F.conv1d(groups=H) on (B, H, T) -> unpad composition, and F.conv1d straight on the     */

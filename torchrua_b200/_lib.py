@@ -82,6 +82,12 @@ SIGNATURES = {
                                    POINTER(Side), c_void_p, c_size_t, c_void_p]),
     'rua_segment_scan_backward': (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32,
                                             c_int32, POINTER(Ragged), POINTER(Side), c_void_p, c_size_t, c_void_p]),
+    'rua_segment_linrec_workspace_bytes': (c_size_t, [c_int64, c_int64, c_int32, c_int32]),
+    'rua_segment_linrec': (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, POINTER(Ragged),
+                                     POINTER(Side), c_void_p, c_size_t, c_void_p]),
+    'rua_segment_linrec_backward': (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                              c_int64, c_int32, c_int32, POINTER(Ragged), POINTER(Side), c_void_p,
+                                              c_size_t, c_void_p]),
     'rua_segment_conv_workspace_bytes': (c_size_t, [c_int64, c_int64, c_int32, c_int32, c_int32]),
     'rua_segment_conv': (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32,
                                    POINTER(Ragged), POINTER(Side), c_void_p, c_size_t, c_void_p]),

@@ -1306,6 +1306,109 @@ def segment_scan(data: Tensor, rg: Ragged, side: SideSpec, op: str, reverse: boo
     return _ScanExtreme.apply(data, rg, side, code, reverse)
 
 
+def linrec_check(data: Tensor, gate: Tensor, initial: Optional[Tensor], B: int, feat: Tuple[int, ...]) -> None:
+    """validate a linear recurrence over rows with features ``feat`` of B sequences, before any device work."""
+    if data.dtype not in _DTYPES:
+        raise RuntimeError(f'torchrua_b200: linear_recurrence supports float16/bfloat16/float32/float64, got {data.dtype}')
+    for name, t in (('gate', gate), ('initial', initial)):
+        if t is not None and t.dtype != data.dtype:
+            raise RuntimeError(f'torchrua_b200: linear_recurrence {name} has dtype {t.dtype}, the input {data.dtype}')
+    if tuple(gate.shape) != tuple(data.shape):
+        raise ValueError(f'torchrua_b200: linear_recurrence gate must have the shape of the input {tuple(data.shape)}, '
+                         f'got {tuple(gate.shape)}')
+    if initial is not None and tuple(initial.shape) != (B,) + tuple(feat):
+        raise ValueError(f'torchrua_b200: linear_recurrence initial must be (B, *feat) = {(B,) + tuple(feat)}, '
+                         f'got {tuple(initial.shape)}')
+    require_cuda(data, gate, initial)
+
+
+def _linrec_raw(data: Tensor, gate: Tensor, h0: Optional[Tensor], rg: Ragged, side: SideSpec, reverse: bool) -> Tensor:
+    """y laid out like data; data, gate (side.rows, *feat) and h0 (B, *feat) or None, all contiguous."""
+    lib = _lib.load()
+    out = torch.empty_like(data)
+    if out.numel() == 0:
+        return out
+    H = data[0].numel()
+    dt = _DTYPES[data.dtype]
+    c_rg, c_side = rg.c_struct(), side.c_struct()
+    with _on(data.device):
+        nbytes = lib.rua_segment_linrec_workspace_bytes(side.rows, H, dt, 0)
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=data.device)
+        prof = _profile_begin()
+        _lib.check(lib.rua_segment_linrec(data.data_ptr(), gate.data_ptr(), _ptr(h0), out.data_ptr(), H, dt, int(reverse),
+                                          ctypes.byref(c_rg), ctypes.byref(c_side), ws.data_ptr(), nbytes, _stream()),
+                   'rua_segment_linrec')
+        if prof is not None:
+            # x and the gate read once, y written once + the initial states + the metadata consulted
+            nb = 3 * data.numel() * data.element_size() + (h0.numel() * h0.element_size() if h0 is not None else 0)
+            _profile_end(prof, 'segment_linrec', nb + 8 * rg.B + (8 * (rg.Tp + rg.B) if side.layout == PACK else 0))
+    return out
+
+
+def _linrec_backward_raw(g: Tensor, gate: Tensor, h0: Optional[Tensor], y: Optional[Tensor], rg: Ragged, side: SideSpec,
+                         reverse: bool, want_x: bool, want_gate: bool, want_h0: bool):
+    """(grad_x, grad_gate, grad_h0), None where not wanted; g, gate, y (side.rows, *feat) contiguous, y needed for
+    grad_gate only."""
+    lib = _lib.load()
+    gx = torch.empty_like(g) if want_x else None
+    gg = torch.empty_like(g) if want_gate else None
+    gh = torch.empty((rg.B,) + tuple(g.shape[1:]), dtype=g.dtype, device=g.device) if want_h0 else None
+    H = int(np.prod(g.shape[1:]))
+    if not (want_x or want_gate or want_h0) or H == 0:
+        return gx, gg, gh
+    dt = _DTYPES[g.dtype]
+    c_rg, c_side = rg.c_struct(), side.c_struct()
+    with _on(g.device):
+        nbytes = lib.rua_segment_linrec_workspace_bytes(side.rows, H, dt, 1)
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=g.device)
+        prof = _profile_begin()
+        _lib.check(lib.rua_segment_linrec_backward(g.data_ptr(), gate.data_ptr(), _ptr(h0), _ptr(y) if want_gate else None,
+                                                   _ptr(gx), _ptr(gg), _ptr(gh), H, dt, int(reverse), ctypes.byref(c_rg),
+                                                   ctypes.byref(c_side), ws.data_ptr() if nbytes else None, nbytes,
+                                                   _stream()), 'rua_segment_linrec_backward')
+        if prof is not None:
+            # grad_out, the gate and y read once, grad_x and grad_gate written once
+            e = g.element_size()
+            nb = g.numel() * e * (2 + 2 * want_gate + want_x) + (gh.numel() * e if gh is not None else 0)
+            _profile_end(prof, 'segment_linrec_backward', nb + 8 * rg.B + (8 * (rg.Tp + rg.B) if side.layout == PACK else 0))
+    return gx, gg, gh
+
+
+class _LinearRecurrence(torch.autograd.Function):
+    """once-differentiable: the backward is a native kernel, double backward is not supported."""
+
+    @staticmethod
+    def forward(ctx, data: Tensor, gate: Tensor, initial: Optional[Tensor], rg: Ragged, side: SideSpec, reverse: bool):
+        x = data.detach().contiguous()
+        a = gate.detach().contiguous()
+        h0 = None if initial is None else initial.detach().contiguous()
+        y = _linrec_raw(x, a, h0, rg, side, reverse)
+        ctx.meta = (rg, side, reverse)
+        ctx.save_for_backward(a, h0, y if ctx.needs_input_grad[1] else None)   # y only feeds grad_gate
+        return y
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_out: Tensor):
+        rg, side, reverse = ctx.meta
+        a, h0, y = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        gx, gg, gh = _linrec_backward_raw(grad_out.contiguous(), a, h0, y, rg, side, reverse, need[0], need[1],
+                                          need[2] and h0 is not None)
+        return gx, gg, gh, None, None, None
+
+
+def linear_recurrence(data: Tensor, gate: Tensor, initial: Optional[Tensor], rg: Ragged, side: SideSpec,
+                      reverse: bool) -> Tensor:
+    """per-sequence h_t = gate_t * h_(t-1) + x_t over the flattened storage ``data`` (side.rows, *feat); gate like data,
+    initial (B, *feat) or None; checked by the caller (linrec_check)."""
+    grad = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (data, gate, initial))
+    if grad:
+        return _LinearRecurrence.apply(data, gate, initial, rg, side, reverse)
+    return _linrec_raw(data.contiguous(), gate.contiguous(), None if initial is None else initial.contiguous(), rg, side,
+                       reverse)
+
+
 # ------------------------------------------------------------------------------------------------
 # K8: per-sequence depthwise 1-D convolution (+ autograd)
 # ------------------------------------------------------------------------------------------------

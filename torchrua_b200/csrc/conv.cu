@@ -176,7 +176,7 @@ __global__ void __launch_bounds__(kConvThreads, 2) segconv_kernel(ConvArgs a) {
       int64_t srow = -1, t;
       int clo = 0, chi = -1, flo = 0, fhi = -1;
       if (j >= 0 && j < a.rows) {
-        decode_position(a, j, n_tok, lo, hi, srow, t, [&](int64_t len) {
+        decode_position(a, j, n_tok, lo, hi, srow, t, [&](int64_t, int64_t len) {
           clo = (int)max((int64_t)0, pad - t);
           chi = (int)min((int64_t)K, len - t + pad);
           flo = (int)max((int64_t)0, a.fpad - t);

@@ -32,6 +32,14 @@
 //              (y is monotone in scan order), so nothing overflows
 //   cummax / cummin backward, in reverse scan order: grad x_k = sum of g_j over the run of positions whose index is k
 //              (the run starts at j = k).  S = (acc, pass) with pass = 0 at a run start: an affine map with slope 0/1.
+//   linear recurrence h_t = a_t h_{t-1} + x_t: S = (m, b), the affine map h -> m h + b; an element lifts to (a_t, x_t),
+//              (a_t, a_t h0[i] + x_t) at the first position of sequence i when an initial state is given;
+//              p (+) q = (p.m q.m, q.m p.b + q.b); the output is b
+//   linear recurrence backward, in reverse scan order: with g~_t = g_t + a_{t+1} g~_{t+1} (the whole adjoint of h_t),
+//              z_t = a_t g~_t is the same affine scan over the elements (a_t, a_t g_t).  grad x_t = g~_t = g_t + z_{t+1}
+//              (the exclusive state), grad a_t = g~_t h_{t-1} (h_{t-1} = the forward output at the previous position, or
+//              h0[i] / 0 at the first), grad h0[i] = z at the first position.  h_{t-1} lies at a closed-form row of the
+//              same sequence (C / L / R srow -+ 1, P srow -+ the batch size between the two steps), so no halo is staged
 #include "reduce_common.cuh"
 #include "seq_decode.cuh"
 
@@ -65,6 +73,9 @@ struct ScanArgs {
   int* flags;
   void* agg;
   void* inc;
+  const void* h0;           // linear recurrence: initial states (B x H), NULL for zero
+  void* out_gate;           // linear recurrence backward: grad gate (NULL: not wanted)
+  void* out_h0;             // linear recurrence backward: grad h0 (NULL: not wanted)
 };
 
 template <typename A> __device__ __forceinline__ bool is_nan(A v) { return v != v; }
@@ -106,7 +117,7 @@ template <typename T, int V> __device__ __forceinline__ void copy_row(const Scan
 template <typename T, int V_> struct OpSum {
   static constexpr int V = V_, kRG = 16;
   static constexpr int kMinBlocks = 2;
-  static constexpr bool kIdx = false;
+  static constexpr bool kIdx = false, kSeq = false;
   using Tp = T;
   using A = typename Store<T>::Acc;
   struct S { A v; };
@@ -137,7 +148,7 @@ template <typename T, int V_> struct OpLse : OpSum<T, V_> {
 template <typename T, int V_, bool kMax> struct OpExt {
   static constexpr int V = V_, kRG = 8;   // the (value, index) state doubles the registers per column
   static constexpr int kMinBlocks = 2;
-  static constexpr bool kIdx = true;
+  static constexpr bool kIdx = true, kSeq = false;
   using Tp = T;
   using A = typename Store<T>::Acc;
   struct S { A v; int32_t i; };   // a position within a sequence: the host refuses >= 2^31 rows
@@ -166,7 +177,7 @@ template <typename T, int V_, bool kMax> struct OpExt {
 template <typename T, int V_> struct OpLseBwd {
   static constexpr int V = V_, kRG = 4;   // three inputs held per row
   static constexpr int kMinBlocks = sizeof(T) == 2 ? 1 : 2;   // eight fp32 (v, y) states per thread: 128 registers spill
-  static constexpr bool kIdx = false;
+  static constexpr bool kIdx = false, kSeq = false;
   static constexpr bool kFast = sizeof(T) == 2;
   using Tp = T;
   using A = typename Store<T>::Acc;
@@ -201,7 +212,7 @@ template <typename T, int V_> struct OpLseBwd {
 template <typename T, int V_> struct OpRunBwd {
   static constexpr int V = V_, kRG = 8;
   static constexpr int kMinBlocks = 2;
-  static constexpr bool kIdx = false;
+  static constexpr bool kIdx = false, kSeq = false;
   using Tp = T;
   using A = typename Store<T>::Acc;
   struct S { A v; int pass; };
@@ -230,6 +241,120 @@ template <typename T, int V_> struct OpRunBwd {
   }
 };
 
+// Operators with kSeq also receive, per row, the decode flags and the offset ho = i * H + col0 of the row's column vector
+// in the per-sequence (B x H) arrays (lift also gets act: a thread past the row end must not read there); their non-token
+// rows go through pass() instead of copy_row.
+template <typename T, int V> __device__ __forceinline__ Raw<T, V> zero_raw() {
+  Raw<T, V> w;
+  if constexpr (V == 1) w.r = Store<T>::from_acc(typename Store<T>::Acc(0));
+  else w.r = make_uint4(0, 0, 0, 0);
+  return w;
+}
+
+template <typename T, int V_> struct OpLinRec {
+  static constexpr int V = V_, kRG = 6;   // two register images per row: kRG = 8 spills at 128 registers
+  static constexpr int kMinBlocks = 2;
+  static constexpr bool kSeq = true;
+  using Tp = T;
+  using A = typename Store<T>::Acc;
+  struct S { A m; A b; };
+  struct E { Raw<T, V> x, g; };
+  __device__ static void load(E& e, const ScanArgs& a, int64_t o, int64_t, uint8_t, int64_t) {
+    load_raw<T, V>(static_cast<const T*>(a.in0) + o, e.x);
+    load_raw<T, V>(static_cast<const T*>(a.in1) + o, e.g);
+  }
+  // h0[i] is read here, at a sequence's first position only, rather than held with the row: a third register image per
+  // row would force kRG = 4, and chunks that small cost a multiple of the time (the latency chain per chunk)
+  __device__ static void lift(const E& e, const ScanArgs& a, bool act, uint8_t fl, int64_t ho, S* s) {
+    A x[V], g[V];
+    unpack_raw<T, V>(e.x, x);
+    unpack_raw<T, V>(e.g, g);
+    if (act && (fl & kStart) && a.h0) {   // act: this thread's columns exist (h0 ends at row B-1, column H-1)
+      Raw<T, V> w;
+      if constexpr (V == 1) w.r = __ldg(static_cast<const T*>(a.h0) + ho);
+      else w.r = __ldg(reinterpret_cast<const uint4*>(static_cast<const T*>(a.h0) + ho));
+      A h[V];
+      unpack_raw<T, V>(w, h);
+#pragma unroll
+      for (int k = 0; k < V; ++k) x[k] = fma(g[k], h[k], x[k]);
+    }
+#pragma unroll
+    for (int k = 0; k < V; ++k) s[k] = {g[k], x[k]};
+  }
+  __device__ static S compose(const S& p, const S& q) { return {p.m * q.m, fma(q.m, p.b, q.b)}; }
+  __device__ static void emit(const ScanArgs& a, int64_t o, const E&, int64_t, bool, const S*, const S* s, uint8_t,
+                              int64_t) {
+    A y[V];
+#pragma unroll
+    for (int k = 0; k < V; ++k) y[k] = s[k].b;
+    store_vec<T, V>(static_cast<T*>(a.out) + o, y);
+  }
+  __device__ static void pass(const ScanArgs& a, int64_t o) { copy_row<T, V>(a, o, false); }
+};
+
+template <typename T, int V_> struct OpLinRecBwd {
+  static constexpr int V = V_, kRG = 8;   // three inputs held per row: one CTA per SM, but chunks of 8 rows per group
+  static constexpr int kMinBlocks = 1;
+  static constexpr bool kSeq = true;
+  using Tp = T;
+  using A = typename Store<T>::Acc;
+  struct S { A m; A b; };
+  struct E { Raw<T, V> g, a, h; };   // h = h_{t-1}, loaded only when grad gate is wanted
+  __device__ static void load(E& e, const ScanArgs& a, int64_t o, int64_t t, uint8_t fl, int64_t ho) {
+    load_raw<T, V>(static_cast<const T*>(a.in0) + o, e.g);
+    load_raw<T, V>(static_cast<const T*>(a.in1) + o, e.a);
+    if (!a.out_gate) return;
+    if (fl & kEnd) {   // the first forward position: h_{-1} = h0[i] or 0
+      if (a.h0) load_raw<T, V>(static_cast<const T*>(a.h0) + ho, e.h);
+      else e.h = zero_raw<T, V>();
+      return;
+    }
+    // the previous forward position of the same sequence; this launch runs against the forward direction
+    int64_t d;
+    if (a.layout == RUA_PACK) d = a.reverse ? __ldg(a.poff + t - 1) - __ldg(a.poff + t) : __ldg(a.poff + t + 1) - __ldg(a.poff + t);
+    else d = a.reverse ? -1 : 1;
+    load_raw<T, V>(static_cast<const T*>(a.in2) + o + d * a.H, e.h);
+  }
+  __device__ static void lift(const E& e, const ScanArgs&, bool, uint8_t, int64_t, S* s) {
+    A g[V], m[V];
+    unpack_raw<T, V>(e.g, g);
+    unpack_raw<T, V>(e.a, m);
+#pragma unroll
+    for (int k = 0; k < V; ++k) s[k] = {m[k], m[k] * g[k]};
+  }
+  __device__ static S compose(const S& p, const S& q) { return {p.m * q.m, fma(q.m, p.b, q.b)}; }
+  __device__ static void emit(const ScanArgs& a, int64_t o, const E& e, int64_t, bool has_before, const S* before,
+                              const S* s, uint8_t fl, int64_t ho) {
+    A g[V];
+    unpack_raw<T, V>(e.g, g);
+#pragma unroll
+    for (int k = 0; k < V; ++k) g[k] = has_before ? g[k] + before[k].b : g[k];
+    if (a.out) store_vec<T, V>(static_cast<T*>(a.out) + o, g);
+    if (a.out_gate) {
+      A h[V], r[V];
+      unpack_raw<T, V>(e.h, h);
+#pragma unroll
+      for (int k = 0; k < V; ++k) r[k] = g[k] * h[k];
+      store_vec<T, V>(static_cast<T*>(a.out_gate) + o, r);
+    }
+    if ((fl & kEnd) && a.out_h0) {
+      A z[V];
+#pragma unroll
+      for (int k = 0; k < V; ++k) z[k] = s[k].b;
+      store_vec<T, V>(static_cast<T*>(a.out_h0) + ho, z);
+    }
+  }
+  __device__ static void pass(const ScanArgs& a, int64_t o) {   // grad_out passes through, the gate gets 0
+    if (a.out) copy_row<T, V>(a, o, false);
+    if (a.out_gate) {
+      A z[V];
+#pragma unroll
+      for (int k = 0; k < V; ++k) z[k] = A(0);
+      store_vec<T, V>(static_cast<T*>(a.out_gate) + o, z);
+    }
+  }
+};
+
 // ---------------------------------------------------------------------------------------------------------------------
 // workspace access: bypass L1 (values are written by other CTAs)
 // ---------------------------------------------------------------------------------------------------------------------
@@ -255,13 +380,15 @@ __device__ __forceinline__ void st_release(int* p, int v) {
   asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
 }
 
-// row decode of virtual position j: storage row, position within the sequence, flags
+// row decode of virtual position j: storage row, position within the sequence, flags (and with kSeq the sequence index)
+template <bool kSeq>
 __device__ __forceinline__ void decode_row(const ScanArgs& a, int64_t j, int64_t n_tok, int64_t lo, int64_t hi,
-                                           int64_t& srow, int64_t& t, uint8_t& fl) {
+                                           int64_t& srow, int64_t& t, uint8_t& fl, int64_t& seq) {
   fl = 0;
-  decode_position(a, j, n_tok, lo, hi, srow, t, [&](int64_t len) {
+  decode_position(a, j, n_tok, lo, hi, srow, t, [&](int64_t i, int64_t len) {
     const int64_t first = a.reverse ? len - 1 : 0, last = a.reverse ? 0 : len - 1;
     fl = kTok | (t == first ? kStart : 0) | (t == last ? kEnd : 0);
+    if constexpr (kSeq) seq = i;
   });
 }
 
@@ -274,7 +401,8 @@ __global__ void __launch_bounds__(kScanThreads, Op::kMinBlocks) segscan_kernel(S
   const int R = a.R;
   int64_t* s_row = reinterpret_cast<int64_t*>(smem);
   int64_t* s_t = s_row + R;
-  S* s_buf = reinterpret_cast<S*>(s_t + R);                       // kScanThreads x V states
+  int64_t* s_seq = s_t + R;                                       // kSeq operators only
+  S* s_buf = reinterpret_cast<S*>(s_t + (Op::kSeq ? 2 : 1) * R);  // kScanThreads x V states
   int* s_flag = reinterpret_cast<int*>(s_buf + kScanThreads * V);  // kScanThreads segment-start flags
   uint8_t* s_fl = reinterpret_cast<uint8_t*>(s_flag + kScanThreads);
   __shared__ unsigned long long s_ticket;
@@ -299,10 +427,12 @@ __global__ void __launch_bounds__(kScanThreads, Op::kMinBlocks) segscan_kernel(S
     const int64_t j = a.reverse ? a.rows - 1 - (q0 + q) : q0 + q;
     int64_t srow, t;
     uint8_t fl;
-    decode_row(a, j, n_tok, lo, hi, srow, t, fl);
+    int64_t seq = 0;
+    decode_row<Op::kSeq>(a, j, n_tok, lo, hi, srow, t, fl, seq);
     s_row[q] = srow;
     s_t[q] = t;
     s_fl[q] = fl;
+    if constexpr (Op::kSeq) s_seq[q] = seq;
   }
   __syncthreads();
 
@@ -316,7 +446,10 @@ __global__ void __launch_bounds__(kScanThreads, Op::kMinBlocks) segscan_kernel(S
 #pragma unroll
   for (int r = 0; r < RG; ++r) {
     const int q = qb + r;
-    if (act && q < nq && (s_fl[q] & kTok)) Op::load(e[r], a, s_row[q] * a.H + col0, s_t[q]);
+    if (act && q < nq && (s_fl[q] & kTok)) {
+      if constexpr (Op::kSeq) Op::load(e[r], a, s_row[q] * a.H + col0, s_t[q], s_fl[q], s_seq[q] * a.H + col0);
+      else Op::load(e[r], a, s_row[q] * a.H + col0, s_t[q]);
+    }
   }
   S s[V];
   bool started = false, have = false;
@@ -330,7 +463,8 @@ __global__ void __launch_bounds__(kScanThreads, Op::kMinBlocks) segscan_kernel(S
         have = false;
       } else {
         S l[V];
-        Op::lift(e[r], s_t[q], l);
+        if constexpr (Op::kSeq) Op::lift(e[r], a, act, f, s_seq[q] * a.H + col0, l);
+        else Op::lift(e[r], s_t[q], l);
         if ((f & kStart) || !have) {
 #pragma unroll
           for (int k = 0; k < V; ++k) s[k] = l[k];
@@ -438,17 +572,26 @@ __global__ void __launch_bounds__(kScanThreads, Op::kMinBlocks) segscan_kernel(S
       const uint8_t f = s_fl[q];
       const int64_t o = s_row[q] * a.H + col0;
       if (!(f & kTok)) {
-        if (act) copy_row<T, V>(a, o, Op::kIdx);
+        if constexpr (Op::kSeq) {
+          if (act) Op::pass(a, o);
+        } else {
+          if (act) copy_row<T, V>(a, o, Op::kIdx);
+        }
       } else {
         S l[V], before[V];
-        Op::lift(e[r], s_t[q], l);
+        if constexpr (Op::kSeq) Op::lift(e[r], a, act, f, s_seq[q] * a.H + col0, l);
+        else Op::lift(e[r], s_t[q], l);
         const bool hb = !(f & kStart);
 #pragma unroll
         for (int k = 0; k < V; ++k) {
           before[k] = gin[k];
           gin[k] = hb ? Op::compose(gin[k], l[k]) : l[k];
         }
-        if (act) Op::emit(a, o, e[r], s_t[q], hb, before, gin);
+        if constexpr (Op::kSeq) {
+          if (act) Op::emit(a, o, e[r], s_t[q], hb, before, gin, f, s_seq[q] * a.H + col0);
+        } else {
+          if (act) Op::emit(a, o, e[r], s_t[q], hb, before, gin);
+        }
       }
     }
   }
@@ -457,7 +600,7 @@ __global__ void __launch_bounds__(kScanThreads, Op::kMinBlocks) segscan_kernel(S
 // ---------------------------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------------------------
-enum Kind { K_SUM, K_LSE, K_MAX, K_MIN, K_LSE_BWD, K_RUN_BWD };
+enum Kind { K_SUM, K_LSE, K_MAX, K_MIN, K_LSE_BWD, K_RUN_BWD, K_LINREC, K_LINREC_BWD };
 
 struct Plan {
   int V, tpc_log2, R, ncb;
@@ -478,6 +621,8 @@ template <typename F> int with_scan_op(Kind kind, int32_t dtype, bool vec, int64
         case K_MAX: return f(Type<OpExt<T, V, true>>{});
         case K_MIN: return f(Type<OpExt<T, V, false>>{});
         case K_LSE_BWD: return f(Type<OpLseBwd<T, V>>{});
+        case K_LINREC: return f(Type<OpLinRec<T, V>>{});
+        case K_LINREC_BWD: return f(Type<OpLinRecBwd<T, V>>{});
         default: return f(Type<OpRunBwd<T, V>>{});
       }
     };
@@ -511,7 +656,7 @@ template <class Op> int launch_op(const ScanArgs& a0, const Plan& p, cudaStream_
   a.tpc_log2 = p.tpc_log2;
   a.R = p.R;
   a.ncb = p.ncb;
-  const size_t smem = (size_t)p.R * 17 + sizeof(typename Op::S) * kScanThreads * Op::V + 4 * kScanThreads;
+  const size_t smem = (size_t)p.R * (Op::kSeq ? 25 : 17) + sizeof(typename Op::S) * kScanThreads * Op::V + 4 * kScanThreads;
   if (smem > 48 * 1024) {   // narrow rows: up to 4096 positions per chunk (~72 KB)
     if (int rc = check_cuda(cudaFuncSetAttribute(segscan_kernel<Op>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                                  (int)smem)))
@@ -522,8 +667,8 @@ template <class Op> int launch_op(const ScanArgs& a0, const Plan& p, cudaStream_
   return check_launch();
 }
 
-int validate(int64_t H, int32_t dtype, int32_t op, const rua_ragged_t* rg, const rua_side_t* side) {
-  if (H < 0 || dtype < RUA_F32 || dtype > RUA_BF16 || op < RUA_SCAN_SUM || op > RUA_SCAN_MIN) return RUA_ERR_INVALID;
+int validate(int64_t H, int32_t dtype, const rua_ragged_t* rg, const rua_side_t* side) {
+  if (H < 0 || dtype < RUA_F32 || dtype > RUA_BF16) return RUA_ERR_INVALID;
   if (!rg || !side || rg->B < 0 || !rg->off || side->rows < 0 || side->width < 0) return RUA_ERR_INVALID;
   if (side->len_xform != RUA_LEN_SAME) return RUA_ERR_UNSUPPORTED;
   switch (side->layout) {
@@ -537,6 +682,10 @@ int validate(int64_t H, int32_t dtype, int32_t op, const rua_ragged_t* rg, const
     default: return RUA_ERR_INVALID;
   }
   return RUA_OK;
+}
+int validate(int64_t H, int32_t dtype, int32_t op, const rua_ragged_t* rg, const rua_side_t* side) {
+  if (op < RUA_SCAN_SUM || op > RUA_SCAN_MIN) return RUA_ERR_INVALID;
+  return validate(H, dtype, rg, side);
 }
 
 int run(Kind kind, int32_t dtype, int64_t H, int32_t reverse, const rua_ragged_t* rg, const rua_side_t* side,
@@ -576,6 +725,18 @@ Kind backward_kind(int32_t op) {
   return op == RUA_SCAN_SUM ? K_SUM : (op == RUA_SCAN_LOGSUMEXP ? K_LSE_BWD : K_RUN_BWD);
 }
 
+// the larger workspace of the two vector widths `kind` may run at
+size_t workspace_bytes(Kind kind, int64_t rows, int64_t H, int32_t dtype) {
+  size_t total = 0;
+  for (bool vec : {true, false})
+    with_scan_op(kind, dtype, vec, H, [&](auto o) {
+      const size_t t = make_plan<typename decltype(o)::type>(rows, H).total;
+      total = t > total ? t : total;
+      return RUA_OK;
+    });
+  return total;
+}
+
 }  // namespace
 }  // namespace rua
 
@@ -585,15 +746,7 @@ extern "C" size_t rua_segment_scan_workspace_bytes(int64_t rows, int64_t H, int3
                                                    int32_t backward) {
   if (rows < 0 || H < 0 || dtype < RUA_F32 || dtype > RUA_BF16 || op < RUA_SCAN_SUM || op > RUA_SCAN_MIN) return 0;
   if (rows == 0 || H == 0) return 0;
-  const Kind kind = backward ? backward_kind(op) : forward_kind(op);
-  size_t total = 0;
-  for (bool vec : {true, false})
-    with_scan_op(kind, dtype, vec, H, [&](auto o) {
-      const size_t t = make_plan<typename decltype(o)::type>(rows, H).total;
-      total = t > total ? t : total;
-      return RUA_OK;
-    });
-  return total;
+  return workspace_bytes(backward ? backward_kind(op) : forward_kind(op), rows, H, dtype);
 }
 
 extern "C" int rua_segment_scan(const void* src, void* dst, int64_t* idx_out, int64_t H, int32_t dtype, int32_t op,
@@ -632,4 +785,54 @@ extern "C" int rua_segment_scan_backward(const void* grad_out, const void* x, co
   const bool vec = aligned16(grad_out) && aligned16(grad_in) && aligned16(x) && aligned16(y) && aligned16(idx);
   // the gradient runs against the forward scan direction
   return run(backward_kind(op), dtype, H, !reverse, ragged, side, a, vec, ws, ws_bytes, stream);
+}
+
+extern "C" size_t rua_segment_linrec_workspace_bytes(int64_t rows, int64_t H, int32_t dtype, int32_t backward) {
+  if (rows < 0 || H < 0 || dtype < RUA_F32 || dtype > RUA_BF16) return 0;
+  if (rows == 0 || H == 0) return 0;
+  return workspace_bytes(backward ? K_LINREC_BWD : K_LINREC, rows, H, dtype);
+}
+
+extern "C" int rua_segment_linrec(const void* x, const void* gate, const void* h0, void* dst, int64_t H, int32_t dtype,
+                                  int32_t reverse, const rua_ragged_t* ragged, const rua_side_t* side, void* ws,
+                                  size_t ws_bytes, rua_stream_t stream) {
+  if (int rc = validate(H, dtype, ragged, side)) return rc;
+  const bool empty = side->rows == 0 || H == 0;
+  if (!empty && (!x || !gate || !dst)) return RUA_ERR_INVALID;
+  ScanArgs a{};
+  a.in0 = x;
+  a.in1 = gate;
+  a.h0 = h0;
+  a.out = dst;
+  const bool vec = aligned16(x) && aligned16(gate) && aligned16(h0) && aligned16(dst);
+  return run(K_LINREC, dtype, H, reverse, ragged, side, a, vec, ws, ws_bytes, stream);
+}
+
+extern "C" int rua_segment_linrec_backward(const void* grad_out, const void* gate, const void* h0, const void* y,
+                                           void* grad_x, void* grad_gate, void* grad_h0, int64_t H, int32_t dtype,
+                                           int32_t reverse, const rua_ragged_t* ragged, const rua_side_t* side,
+                                           void* ws, size_t ws_bytes, rua_stream_t stream) {
+  if (int rc = validate(H, dtype, ragged, side)) return rc;
+  const bool empty = side->rows == 0 || H == 0;
+  const bool any = grad_x || grad_gate || grad_h0;
+  if (!empty && any && (!grad_out || !gate || (grad_gate && !y))) return RUA_ERR_INVALID;
+  if (!any || H == 0) return RUA_OK;
+  if (!empty && (!ws || ws_bytes < workspace_bytes(K_LINREC_BWD, side->rows, H, dtype))) return RUA_ERR_WORKSPACE;
+  // an empty sequence has no first position to write its grad h0 at
+  if (grad_h0 && ragged->B > 0) {
+    const size_t bytes = (size_t)ragged->B * H * (16 / vec_elems(dtype));
+    if (int rc = check_cuda(cudaMemsetAsync(grad_h0, 0, bytes, static_cast<cudaStream_t>(stream)))) return rc;
+  }
+  ScanArgs a{};
+  a.in0 = grad_out;
+  a.in1 = gate;
+  a.in2 = y;
+  a.h0 = h0;
+  a.out = grad_x;
+  a.out_gate = grad_gate;
+  a.out_h0 = grad_h0;
+  const bool vec = aligned16(grad_out) && aligned16(gate) && aligned16(h0) && aligned16(y) && aligned16(grad_x) &&
+                   aligned16(grad_gate) && aligned16(grad_h0);
+  // the gradient runs against the forward scan direction
+  return run(K_LINREC_BWD, dtype, H, !reverse, ragged, side, a, vec, ws, ws_bytes, stream);
 }

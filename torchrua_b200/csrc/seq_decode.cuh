@@ -26,17 +26,19 @@ __device__ __forceinline__ void owner_bounds(const Args& a, int64_t n_tok, int64
 }
 
 // virtual position j -> storage row srow and position t within its sequence (srow = j, t = 0 for a row that holds no
-// token: L / R padding, C rows at or past n_tok = off[B]); on_token(len) runs for a token row only.  [lo, hi) from
-// owner_bounds.  Row of token (i, t): C off[i] + t, L i * W + t, R i * W + (W - len) + t, P poff[t] + unsorted[i].
+// token: L / R padding, C rows at or past n_tok = off[B]); on_token(i, len) runs for a token row only, with i the index of
+// its sequence in off (token_sizes order, also for P).  [lo, hi) from owner_bounds.  Row of token (i, t): C off[i] + t,
+// L i * W + t, R i * W + (W - len) + t, P poff[t] + unsorted[i].
 // `a` is the kernel's argument struct (fields layout, W, off, poff, unsorted), read where it lies.
 template <class Args, class OnToken>
 __device__ __forceinline__ void decode_position(const Args& a, int64_t j, int64_t n_tok, int64_t lo, int64_t hi,
                                                 int64_t& srow, int64_t& t, OnToken&& on_token) {
   srow = j;
   t = 0;
-  int64_t len;
+  int64_t i, len;
   if (a.layout == RUA_LEFT || a.layout == RUA_RIGHT) {
-    const int64_t i = j / a.W, c = j - i * a.W;
+    i = j / a.W;
+    const int64_t c = j - i * a.W;
     len = __ldg(a.off + i + 1) - __ldg(a.off + i);
     t = a.layout == RUA_LEFT ? c : c - (a.W - len);
     if (t < 0 || t >= len) return;
@@ -46,12 +48,13 @@ __device__ __forceinline__ void decode_position(const Args& a, int64_t j, int64_
       const int64_t mid = (lo + hi) >> 1;
       if (__ldg(a.off + mid) <= j) lo = mid; else hi = mid;
     }
-    const int64_t o = __ldg(a.off + lo);
-    len = __ldg(a.off + lo + 1) - o;
+    i = lo;
+    const int64_t o = __ldg(a.off + i);
+    len = __ldg(a.off + i + 1) - o;
     t = j - o;
-    if (a.layout == RUA_PACK) srow = __ldg(a.poff + t) + __ldg(a.unsorted + lo);
+    if (a.layout == RUA_PACK) srow = __ldg(a.poff + t) + __ldg(a.unsorted + i);
   }
-  on_token(len);
+  on_token(i, len);
 }
 
 }  // namespace rua
