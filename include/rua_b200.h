@@ -282,7 +282,9 @@ int rua_segment_reduce_strict(const void* data, const int64_t* off, int64_t N, i
 
 /* backward twin (ATen SegmentReduceBackward0 semantics, SURVEY.md 8a): sum -> broadcast, mean ->
  * broadcast / len, max/min -> split evenly among ties, prod -> grad*out/x (exact when x != 0, else
- * product of the others), logsumexp -> softmax weights. */
+ * product of the others), logsumexp -> softmax weights.  Writes all N rows of grad_data: rows no segment
+ * owns (at or past off[S]) get 0.  S == 0: grad_out, out, data and off may be NULL; grad_data is zeroed
+ * with cudaMemsetAsync and no kernel runs. */
 size_t rua_segment_reduce_backward_workspace_bytes(int64_t N, int64_t S, int64_t H, int32_t dtype,
                                                    int32_t op);
 int rua_segment_reduce_backward(const void* grad_out, const void* out, const void* data,

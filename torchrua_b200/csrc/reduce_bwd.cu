@@ -317,9 +317,12 @@ int rua_segment_reduce_backward(const void* grad_out, const void* out, const voi
                                 void* ws, size_t ws_bytes, rua_stream_t stream) {
   if (N < 0 || S < 0 || H < 0) return RUA_ERR_INVALID;
   if (N == 0 || H == 0) return RUA_OK;
-  if (!grad_out || !out || !data || !off || !grad_data) return RUA_ERR_INVALID;
   if (op < RUA_SUM || op > RUA_LOGSUMEXP) return RUA_ERR_INVALID;
   if (dtype < RUA_F32 || dtype > RUA_BF16) return RUA_ERR_UNSUPPORTED;
+  if (!grad_data) return RUA_ERR_INVALID;
+  if (S == 0)   // no segment owns a row: the gradient is zero, and nothing else is read (the forward's output is empty)
+    return check_cuda(cudaMemsetAsync(grad_data, 0, (size_t)N * H * (16 / vec_elems(dtype)), (cudaStream_t)stream));
+  if (!grad_out || !out || !data || !off) return RUA_ERR_INVALID;
   if (ws_bytes < rua_segment_reduce_backward_workspace_bytes(N, S, H, dtype, op) - 16) return RUA_ERR_WORKSPACE;
   if ((op == RUA_MAX || op == RUA_MIN) && !ws) return RUA_ERR_INVALID;
   uintptr_t a = (uintptr_t)grad_out | (uintptr_t)out | (uintptr_t)data | (uintptr_t)grad_data;

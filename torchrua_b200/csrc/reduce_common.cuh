@@ -296,7 +296,7 @@ __device__ __forceinline__ void lse_batch(const Raw<T, V>* raw, typename Store<T
       float m_new = max_nan(a[v], bm[v]);
       s[v] = s[v] == 0.f ? 0.f : s[v] * ex2_approx((a[v] - m_new) * kLog2e);
       a[v] = m_new;
-      mb[v] = m_new * kLog2e;
+      mb[v] = m_new == -inf_of<A>() ? 0.f : m_new * kLog2e;   // all -inf so far: each adds ex2(-inf) = 0, not ex2(NaN)
     }
 #pragma unroll
     for (int k = 0; k < kRows; ++k) {
@@ -317,7 +317,7 @@ __device__ __forceinline__ void lse_batch(const Raw<T, V>* raw, typename Store<T
       A x[V];
       unpack_raw<T, V>(raw[k], x);
 #pragma unroll
-      for (int v = 0; v < V; ++v) s[v] += exp(x[v] - a[v]);
+      for (int v = 0; v < V; ++v) s[v] += exp(x[v] - (a[v] == -inf_of<A>() ? A(0) : a[v]));
     }
   }
 }
@@ -362,10 +362,11 @@ struct State {
       else if (OP == RUA_PROD) a[v] *= x[v];
       else if (OP == RUA_MAX) a[v] = max_nan(a[v], x[v]);
       else if (OP == RUA_MIN) a[v] = min_nan(a[v], x[v]);
-      else {  // online logsumexp: one exp per element
+      else {  // online logsumexp: one exp per element.  A -inf element adds 0, also while the running max is still -inf
+              // (-inf - -inf = NaN, clamped to 0 by the fmax); a NaN element still poisons the result through a
         A d = x[v] - a[v];
         A e = exp_acc<kFast>(-abs_acc(d));
-        s[v] = d > A(0) ? s[v] * e + A(1) : s[v] + e;
+        s[v] = d > A(0) ? s[v] * e + A(1) : s[v] + fmax(e, A(0));
         a[v] = max_nan(a[v], x[v]);
       }
     }

@@ -98,7 +98,7 @@ segreduce_kernel(const T* __restrict__ data, const int64_t* __restrict__ ridx, c
             unpack_raw<T, V>(raw[kk], x);
             if (OpInfo<OP>::kIsLse && !pending) {          // first row of a piece: exp(x - x) = 1, no exponential needed
 #pragma unroll
-              for (int v = 0; v < V; ++v) { st.a[v] = x[v]; st.s[v] = A(1); }
+              for (int v = 0; v < V; ++v) { st.a[v] = x[v]; st.s[v] = x[v] == -inf_of<A>() ? A(0) : A(1); }   // -inf adds 0
             } else {
               st.template add<kFast>(x);
             }

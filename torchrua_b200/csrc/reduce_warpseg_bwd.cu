@@ -25,8 +25,13 @@ segreduce_bwd_warpseg_kernel(const T* __restrict__ gout, const T* __restrict__ o
   __shared__ __align__(8) uint64_t s_bar[kWsWarps];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int64_t s0 = ((int64_t)blockIdx.x * kWsWarps + warp) * 32;
-  if (s0 >= S) return;                                // warp-uniform; nothing block-wide below
   const int64_t covered = __ldg(off + S) < N ? __ldg(off + S) : N;
+  if (covered < N) {                                  // rows no segment owns (sum of sizes < N): zero gradient, every warp
+    const int64_t step = (int64_t)gridDim.x * kWsThreads;   // of the grid takes a strided share of them
+    for (int64_t e = covered * HE + (int64_t)blockIdx.x * kWsThreads + threadIdx.x; e < N * HE; e += step)
+      grad[e] = Store<T>::from_acc(A(0));
+  }
+  if (s0 >= S) return;                                // warp-uniform; nothing block-wide below
   const int64_t s = s0 + lane;
   int64_t beg = s < S ? __ldg(off + s) : covered, end = s < S ? __ldg(off + s + 1) : covered;
   const int64_t len = end - beg;
@@ -184,7 +189,7 @@ segreduce_bwd_warpseg_kernel(const T* __restrict__ gout, const T* __restrict__ o
   }
 }
 
-// The kernel writes only the rows of [0, off[S]): rows past the last segment (sum of sizes < N) are left as they were.
+// The kernel writes every one of the N rows: the segments' rows [0, off[S]) and zeros on the rows past the last segment.
 int warpseg_bwd_launch(int32_t dtype, int64_t H, int32_t op, const void* gout, const void* out, const void* data,
                        const int64_t* off, int64_t N, int64_t S, void* grad, cudaStream_t st) {
   // per-token SCALARS only (H == 1: log-probabilities, losses, scores -- the config-5 shape).  Rows of 2..8 elements
