@@ -395,6 +395,61 @@ int rua_segment_conv_backward(const void* grad_out, const void* x, const void* w
                               const rua_side_t* side, void* ws, size_t ws_bytes, rua_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------- */
+/* K9  per-sequence linear-chain CRF (no counterpart in the reference; replaces pad -> a Python   */
+/* loop over T of logsumexp(alpha[:, :, None] + W + x_t[:, None, :], 1) -> autograd, which keeps */
+/* a (B, K, K) temporary per step, and the same loop in max-plus + a backtrack for Viterbi)      */
+/* ------------------------------------------------------------------------------------------- */
+/* Emissions x: side->rows rows of K tag scores in the storage of `side` (C, L, P or R over `ragged`; len_xform must be
+ * RUA_LEN_SAME); W (K, K) row-major, W[a, b] scores tag a at t-1 followed by tag b at t; start, end (K) or NULL for 0; all of
+ * `dtype`.  1 <= K <= 64.  For a tag path y of sequence i with length len[i] (rows from the "Row of token" formulas):
+ *   score(y) = start[y_0] + sum_t x(i, t)[y_t] + sum_{t>=1} W[y_{t-1}, y_t] + end[y_{len-1}]
+ *   log Z_i  = logsumexp over all K^len paths of score(y)
+ * Per-sequence outputs (log_z, score, best_score and their gradients grad_log_z, grad_score) are B values of the
+ * ACCUMULATOR type (fp32, fp64 for RUA_F64) in sequence order (for P the index in ragged->off).  -inf anywhere means a
+ * forbidden tag or transition; behaviour is specified for inputs without NaN.  An empty sequence has log Z = score = best
+ * score = 0 and zero gradients.  ragged->sorted is required (B > 0): warp g of a fixed grid of G warps takes the sequences
+ * of ranks g, g + G, ... in that order (longest first for the package's own sort), so every result is bit-identical run
+ * to run and, for the same sequences, on every layout.  The running state is normalised per step with an fp64 offset. */
+enum rua_crf_mode { RUA_CRF_FORWARD = 0, RUA_CRF_BACKWARD = 1, RUA_CRF_DECODE = 2 };
+
+/* workspace of rua_crf_forward (0: none), rua_crf_backward (a fixed number of per-CTA slots of partial transition / start
+ * / end gradients: monotone in rows and bounded) and rua_crf_decode (rows x K bytes of uint8 backpointers).  Host only;
+ * 0 when an argument is invalid. */
+size_t rua_crf_workspace_bytes(int64_t rows, int32_t K, int32_t dtype, int32_t mode);
+/* bytes of the state rua_crf_forward keeps for rua_crf_backward: the normalised forward scores (rows x K, accumulator
+ * type) and the fp64 offset of every row. */
+size_t rua_crf_state_bytes(int64_t rows, int32_t K, int32_t dtype);
+
+/* log_z[i] = log Z_i.  tags != NULL (side->rows int64, read at token rows only): also score[i] = score(tags of i), NaN
+ * for a sequence with a tag outside [0, K) (that tag is not dereferenced); tags and score are given together or not at
+ * all.  state_out: rua_crf_state_bytes(side->rows, K, dtype) bytes for rua_crf_backward, or NULL.  No workspace. */
+int rua_crf_forward(const void* x, const int64_t* tags, const void* W, const void* start, const void* end, void* log_z,
+                    void* score, void* state_out, int32_t K, int32_t dtype, const rua_ragged_t* ragged,
+                    const rua_side_t* side, void* ws, size_t ws_bytes, rua_stream_t stream);
+
+/* gradients of gZ_i log Z_i + gS_i score_i (gZ = grad_log_z, gS = grad_score or NULL for 0) with the state and log_z of the
+ * rua_crf_forward call on the same x / W / start / end / ragged / side:
+ *   grad_x(i, t)[b] = gZ mu_t[b] + gS [b = y_t],   mu_t[b] = exp(alpha_t[b] + beta_t[b] - log Z_i) (the tag marginal);
+ *   grad_W[a, b]    = sum over tokens t >= 1 of gZ xi_t[a, b] + gS [y_{t-1} = a, y_t = b];
+ *   grad_start / grad_end: the same at the first / last token.
+ * A sequence with log Z = -inf contributes 0, and so do tags outside [0, K).  Rows that hold no token get 0 in grad_x.  Any
+ * of grad_x / grad_W / grad_start / grad_end may be NULL and is then not computed; tags are needed with grad_score only;
+ * start is not read (the state holds it).  Deterministic: every CTA sums its sequences into its own workspace slot, and a
+ * second kernel sums the slots in slot order.  ws: rua_crf_workspace_bytes(side->rows, K, dtype, RUA_CRF_BACKWARD) bytes
+ * when grad_W, grad_start or grad_end is wanted.  No token at all: the gradients are zeroed with cudaMemsetAsync. */
+int rua_crf_backward(const void* grad_log_z, const void* grad_score, const void* x, const int64_t* tags, const void* W,
+                     const void* start, const void* end, const void* state, const void* log_z, void* grad_x, void* grad_W,
+                     void* grad_start, void* grad_end, int32_t K, int32_t dtype, const rua_ragged_t* ragged,
+                     const rua_side_t* side, void* ws, size_t ws_bytes, rua_stream_t stream);
+
+/* Viterbi: tags_out (side->rows int64) = the best path of every sequence at its own rows, -1 at rows that hold no token;
+ * best_score[i] = its score.  Ties go to the smallest tag index, for the predecessor at every step and for the last tag.
+ * ws: rua_crf_workspace_bytes(side->rows, K, dtype, RUA_CRF_DECODE) bytes. */
+int rua_crf_decode(const void* x, const void* W, const void* start, const void* end, int64_t* tags_out, void* best_score,
+                   int32_t K, int32_t dtype, const rua_ragged_t* ragged, const rua_side_t* side, void* ws,
+                   size_t ws_bytes, rua_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------- */
 /* K5  multi-GPU output gather over NVLink peer memory (SURVEY.md 8e-3; the reference is         */
 /* single-device).  One process per GPU; the batch is sharded by sequence; every rank stores its */
 /* rows directly into the output buffers ("windows") of all ranks of the node.                   */

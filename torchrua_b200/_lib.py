@@ -18,6 +18,7 @@ PAD_FILL, PAD_ROW0, PAD_WRAP = 0, 1, 2
 F32, F64, F16, BF16 = 0, 1, 2, 3
 SUM, MEAN, PROD, MAX, MIN, LOGSUMEXP = 0, 1, 2, 3, 4, 5
 SCAN_SUM, SCAN_LOGSUMEXP, SCAN_MAX, SCAN_MIN = 0, 1, 2, 3
+CRF_FORWARD, CRF_BACKWARD, CRF_DECODE = 0, 1, 2
 
 
 class Ragged(Structure):
@@ -94,6 +95,15 @@ SIGNATURES = {
     'rua_segment_conv_backward': (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32,
                                             c_int32, c_int32, POINTER(Ragged), POINTER(Side), c_void_p, c_size_t,
                                             c_void_p]),
+    'rua_crf_workspace_bytes': (c_size_t, [c_int64, c_int32, c_int32, c_int32]),
+    'rua_crf_state_bytes': (c_size_t, [c_int64, c_int32, c_int32]),
+    'rua_crf_forward': (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32,
+                                  c_int32, POINTER(Ragged), POINTER(Side), c_void_p, c_size_t, c_void_p]),
+    'rua_crf_backward': (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                   c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, POINTER(Ragged), POINTER(Side),
+                                   c_void_p, c_size_t, c_void_p]),
+    'rua_crf_decode': (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, POINTER(Ragged),
+                                 POINTER(Side), c_void_p, c_size_t, c_void_p]),
     'rua_peer_window_alloc': (c_int32, [c_size_t, POINTER(c_void_p), c_char_p]),
     'rua_peer_window_open': (c_int32, [c_char_p, POINTER(c_void_p)]),
     'rua_peer_window_close': (c_int32, [c_void_p]),

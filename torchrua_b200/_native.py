@@ -1531,6 +1531,171 @@ def segment_conv(data: Tensor, weight: Tensor, bias: Optional[Tensor], padding, 
 
 
 # ------------------------------------------------------------------------------------------------
+# K9: per-sequence linear-chain CRF (+ autograd)
+# ------------------------------------------------------------------------------------------------
+CRF_MAX_K = 64
+
+
+def crf_check(emissions: Tensor, transitions: Tensor, start: Optional[Tensor], end: Optional[Tensor], lead: int,
+              tags: Optional[Tensor] = None) -> int:
+    """validate a CRF over emissions with ``lead`` row dimensions and one tag dimension -> K, before any device work;
+    ``tags`` must be int64 and shaped like the row dimensions."""
+    if emissions.dtype not in _DTYPES:
+        raise RuntimeError(f'torchrua_b200: crf supports float16/bfloat16/float32/float64 emissions, got {emissions.dtype}')
+    if emissions.dim() != lead + 1:
+        raise ValueError(f'torchrua_b200: crf emissions must have {lead} row dimension(s) and one tag dimension, '
+                         f'got shape {tuple(emissions.shape)}')
+    K = emissions.shape[-1]
+    if not 1 <= K <= CRF_MAX_K:
+        raise ValueError(f'torchrua_b200: crf supports 1..{CRF_MAX_K} tags, got {K}')
+    for name, t in (('transitions', transitions), ('start', start), ('end', end)):
+        if t is not None and t.dtype != emissions.dtype:
+            raise RuntimeError(f'torchrua_b200: crf {name} has dtype {t.dtype}, the emissions {emissions.dtype}')
+    if tuple(transitions.shape) != (K, K):
+        raise ValueError(f'torchrua_b200: crf transitions must be (K, K) = {(K, K)}, got {tuple(transitions.shape)}')
+    for name, t in (('start', start), ('end', end)):
+        if t is not None and tuple(t.shape) != (K,):
+            raise ValueError(f'torchrua_b200: crf {name} must be (K,) = {(K,)}, got {tuple(t.shape)}')
+    if tags is not None:
+        if tags.dtype != torch.long:
+            raise RuntimeError(f'torchrua_b200: crf tags must be int64, got {tags.dtype}')
+        if tuple(tags.shape) != tuple(emissions.shape[:-1]):
+            raise ValueError(f'torchrua_b200: crf tags must have the shape {tuple(emissions.shape[:-1])} of the emission '
+                             f'rows, got {tuple(tags.shape)}')
+    require_cuda(emissions, transitions, start, end, tags)
+    return K
+
+
+def _crf_acc_dtype(dtype: torch.dtype) -> torch.dtype:
+    return torch.float64 if dtype == torch.float64 else torch.float32
+
+
+def _crf_forward_raw(x: Tensor, tags: Optional[Tensor], W: Tensor, start: Optional[Tensor], end: Optional[Tensor],
+                     rg: Ragged, side: SideSpec, keep_state: bool):
+    """(log_z, score or None, state or None); x (side.rows, K), tags (side.rows,) or None, all contiguous."""
+    lib = _lib.load()
+    K = W.shape[0]
+    dt = _DTYPES[x.dtype]
+    acc = _crf_acc_dtype(x.dtype)
+    log_z = torch.empty(rg.B, dtype=acc, device=x.device)
+    score = torch.empty(rg.B, dtype=acc, device=x.device) if tags is not None else None
+    state = None
+    if keep_state:
+        state = torch.empty(lib.rua_crf_state_bytes(side.rows, K, dt), dtype=torch.uint8, device=x.device)
+    if rg.B == 0:
+        return log_z, score, state
+    c_rg, c_side = rg.c_struct(), side.c_struct()
+    with _on(x.device):
+        prof = _profile_begin()
+        _lib.check(lib.rua_crf_forward(x.data_ptr(), _ptr(tags), W.data_ptr(), _ptr(start), _ptr(end), log_z.data_ptr(),
+                                       _ptr(score), _ptr(state) if state is not None and state.numel() else None, K, dt,
+                                       ctypes.byref(c_rg), ctypes.byref(c_side), None, 0, _stream()), 'rua_crf_forward')
+        if prof is not None:
+            nb = x.numel() * x.element_size() + (state.numel() if state is not None else 0)
+            _profile_end(prof, 'crf_forward', nb + 8 * rg.B + (8 * (rg.Tp + rg.B) if side.layout == PACK else 0))
+    return log_z, score, state
+
+
+def _crf_backward_raw(g_z: Tensor, g_s: Optional[Tensor], x: Tensor, tags: Optional[Tensor], W: Tensor,
+                      end: Optional[Tensor], state: Tensor, log_z: Tensor, rg: Ragged, side: SideSpec, want_x: bool,
+                      want_w: bool, want_start: bool, want_end: bool):
+    """(grad_x, grad_W, grad_start, grad_end), None where not wanted; every input contiguous."""
+    lib = _lib.load()
+    K = W.shape[0]
+    dt = _DTYPES[x.dtype]
+    gx = torch.empty_like(x) if want_x else None
+    gw = torch.empty_like(W) if want_w else None
+    gst = torch.empty(K, dtype=x.dtype, device=x.device) if want_start else None
+    gen = torch.empty(K, dtype=x.dtype, device=x.device) if want_end else None
+    if not (want_x or want_w or want_start or want_end):
+        return gx, gw, gst, gen
+    c_rg, c_side = rg.c_struct(), side.c_struct()
+    with _on(x.device):
+        nbytes = lib.rua_crf_workspace_bytes(side.rows, K, dt, _lib.CRF_BACKWARD) if (want_w or want_start or want_end) else 0
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
+        prof = _profile_begin()
+        _lib.check(lib.rua_crf_backward(g_z.data_ptr(), _ptr(g_s), x.data_ptr(), _ptr(tags), W.data_ptr(), None, _ptr(end),
+                                        _ptr(state) if state.numel() else None, log_z.data_ptr(), _ptr(gx), _ptr(gw),
+                                        _ptr(gst), _ptr(gen), K, dt, ctypes.byref(c_rg), ctypes.byref(c_side),
+                                        ws.data_ptr() if nbytes else None, nbytes, _stream()), 'rua_crf_backward')
+        if prof is not None:
+            nb = x.numel() * x.element_size() * (1 + want_x) + state.numel()
+            _profile_end(prof, 'crf_backward', nb + 8 * rg.B + (8 * (rg.Tp + rg.B) if side.layout == PACK else 0))
+    return gx, gw, gst, gen
+
+
+class _SegmentCrf(torch.autograd.Function):
+    """log Z (tags is None) or score(tags) - log Z per sequence.  Once-differentiable: the backward is a native kernel,
+    double backward is not supported."""
+
+    @staticmethod
+    def forward(ctx, x: Tensor, W: Tensor, start: Optional[Tensor], end: Optional[Tensor], tags: Optional[Tensor],
+                rg: Ragged, side: SideSpec):
+        xs = x.detach().contiguous()
+        Ws = W.detach().contiguous()
+        ss = None if start is None else start.detach().contiguous()
+        es = None if end is None else end.detach().contiguous()
+        keep = any(ctx.needs_input_grad[:4])
+        log_z, score, state = _crf_forward_raw(xs, tags, Ws, ss, es, rg, side, keep)
+        ctx.meta = (rg, side, start is not None, end is not None)
+        if keep:
+            ctx.save_for_backward(xs, tags, Ws, es, state, log_z)
+        return log_z if tags is None else score - log_z
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, g: Tensor):
+        rg, side, has_start, has_end = ctx.meta
+        x, tags, W, end, state, log_z = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        g = g.contiguous()
+        g_z, g_s = (g, None) if tags is None else (-g, g)
+        gx, gw, gst, gen = _crf_backward_raw(g_z, g_s, x, tags, W, end, state, log_z, rg, side, need[0], need[1],
+                                             need[2] and has_start, need[3] and has_end)
+        return gx, gw, gst, gen, None, None, None
+
+
+def segment_crf(emissions: Tensor, tags: Optional[Tensor], transitions: Tensor, start: Optional[Tensor],
+                end: Optional[Tensor], rg: Ragged, side: SideSpec) -> Tensor:
+    """log Z (tags None) or the log-likelihood of ``tags`` per sequence over the flattened storage ``emissions``
+    (side.rows, K), tags (side.rows,); checked by the caller (crf_check); ``rg`` has its pack side."""
+    grad = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (emissions, transitions, start, end))
+    tags = None if tags is None else tags.contiguous()
+    if grad:
+        return _SegmentCrf.apply(emissions, transitions, start, end, tags, rg, side)
+    log_z, score, _ = _crf_forward_raw(emissions.contiguous(), tags, transitions.contiguous(),
+                                       None if start is None else start.contiguous(),
+                                       None if end is None else end.contiguous(), rg, side, False)
+    return log_z if tags is None else score - log_z
+
+
+def crf_decode(emissions: Tensor, transitions: Tensor, start: Optional[Tensor], end: Optional[Tensor], rg: Ragged,
+               side: SideSpec) -> Tuple[Tensor, Tensor]:
+    """(tags (side.rows,) int64 with -1 at rows that hold no token, best score (B,)); no gradient."""
+    lib = _lib.load()
+    x = emissions.detach().contiguous()
+    W, start, end = (None if t is None else t.detach().contiguous() for t in (transitions, start, end))
+    K = x.shape[-1]
+    dt = _DTYPES[x.dtype]
+    tags = torch.empty(side.rows, dtype=torch.long, device=x.device)
+    best = torch.empty(rg.B, dtype=_crf_acc_dtype(x.dtype), device=x.device)
+    if rg.B == 0 and side.rows == 0:
+        return tags, best
+    c_rg, c_side = rg.c_struct(), side.c_struct()
+    with _on(x.device):
+        nbytes = lib.rua_crf_workspace_bytes(side.rows, K, dt, _lib.CRF_DECODE)
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
+        prof = _profile_begin()
+        _lib.check(lib.rua_crf_decode(x.data_ptr(), W.data_ptr(), _ptr(start), _ptr(end), tags.data_ptr(), best.data_ptr(),
+                                      K, dt, ctypes.byref(c_rg), ctypes.byref(c_side), ws.data_ptr() if nbytes else None,
+                                      nbytes, _stream()), 'rua_crf_decode')
+        if prof is not None:
+            nb = x.numel() * x.element_size() + 9 * side.rows + 2 * side.rows * K
+            _profile_end(prof, 'crf_decode', nb + 8 * rg.B + (8 * (rg.Tp + rg.B) if side.layout == PACK else 0))
+    return tags, best
+
+
+# ------------------------------------------------------------------------------------------------
 # scatter_*: stable sort of the index + bucket boundaries + segment reduce over GATHERED rows
 # ------------------------------------------------------------------------------------------------
 def sort_keys(keys: Tensor, max_key: int) -> Tuple[Tensor, Tensor]:

@@ -22,10 +22,11 @@
 //   * grad_in is the same convolution of grad_out with flipped taps and pad' = K - 1 - pad;
 //   * grad_weight[h, k] = sum grad_out(i, t, h) x(i, t + k - pad, h) over valid taps, grad_bias[h] = sum grad_out.  Each
 //     CTA accumulates its chunks in registers (thread = (tap, column vector) pair) and stores one fixed slot; the slots
-//     are summed in slot order by conv_finalize.  The grid, and so the number of slots, is a host function of (rows, H,
-//     K, dtype) capped at kGridCTAs: fixed assignment, no atomics, bit-identical run to run, bounded workspace.
+//     are summed in slot order by slot_sum (slot_sum.cuh).  The grid, and so the number of slots, is a host function of
+//     (rows, H, K, dtype) capped at kGridCTAs: fixed assignment, no atomics, bit-identical run to run, bounded workspace.
 #include "reduce_common.cuh"
 #include "seq_decode.cuh"
+#include "slot_sum.cuh"
 
 namespace rua {
 namespace {
@@ -303,25 +304,21 @@ __global__ void __launch_bounds__(kConvThreads, 2) segconv_kernel(ConvArgs a) {
   }
 }
 
-// grad_weight[h, k] (k < K) and grad_bias[h] (k = K): the slots summed in slot order
-template <typename T>
-__global__ void conv_finalize(const typename Store<T>::Acc* slots, T* gw, T* gb, int64_t H, int K, int64_t S, int ncb,
-                              int CW) {
-  using A = typename Store<T>::Acc;
-  const int64_t n = (int64_t)(K + 1) * H;
-  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+// columns of the slot sum: grad_weight[h, k] (k < K) and grad_bias[h] (k = K), column i = k * H + h
+template <typename T> struct ConvCols {
+  T* gw;
+  T* gb;
+  int64_t H;
+  int K, CW;
+  __device__ T* operator()(int64_t i, int64_t& src) const {
     const int k = (int)(i / H);
     const int64_t h = i - (int64_t)k * H;
-    if (k < K ? !gw : !gb) continue;
     const int64_t cb = h / CW, c = h - cb * CW;
-    const A* p = slots + (cb * (K + 1) + k) * CW + c;
-    const int64_t stride = (int64_t)ncb * (K + 1) * CW;
-    A s = 0;
-    for (int64_t sl = 0; sl < S; ++sl) s += __ldcg(p + sl * stride);
-    if (k < K) gw[h * K + k] = Store<T>::from_acc(s);
-    else gb[h] = Store<T>::from_acc(s);
+    src = (cb * (K + 1) + k) * CW + c;
+    if (k < K) return gw ? gw + h * K + k : nullptr;
+    return gb ? gb + h : nullptr;
   }
-}
+};
 
 // ---------------------------------------------------------------------------------------------------------------------
 // host side
@@ -428,11 +425,9 @@ int run(bool bwd, int32_t dtype, int64_t H, int32_t K, int32_t pad, const rua_ra
       return launch(segconv_kernel<T, V, kB, false>);
     });
     if (rc || !bwd || (!gw && !gb)) return rc;
-    const int64_t n = (int64_t)(K + 1) * H;
-    const unsigned blocks = (unsigned)(ceil_div(n, 256) < 4096 ? ceil_div(n, 256) : 4096);
-    conv_finalize<T><<<blocks, 256, 0, st>>>(static_cast<const typename Store<T>::Acc*>(ws), static_cast<T*>(gw),
-                                             static_cast<T*>(gb), H, K, p.S, p.ncb, (1 << p.tpc_log2) * V);
-    return check_launch();
+    const int CW = (1 << p.tpc_log2) * V;
+    return launch_slot_sum<T>(static_cast<const typename Store<T>::Acc*>(ws), p.S, (int64_t)p.ncb * (K + 1) * CW,
+                              (int64_t)(K + 1) * H, ConvCols<T>{static_cast<T*>(gw), static_cast<T*>(gb), H, K, CW}, st);
   });
 }
 
