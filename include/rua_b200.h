@@ -450,6 +450,63 @@ int rua_crf_decode(const void* x, const void* W, const void* start, const void* 
                    size_t ws_bytes, rua_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------- */
+/* K10 per-sequence selective state-space scan, Mamba-1 style (no counterpart in the reference;  */
+/* replaces pad -> a Python loop over T that autograd keeps a (B, H, N) state of per step, and   */
+/* the linear recurrence over H x N columns, which materialises (tokens, H, N) tensors)          */
+/* ------------------------------------------------------------------------------------------- */
+/* x, delta, y: side->rows rows of H elements in the storage of `side` (C, L, P or R over `ragged`; len_xform must be
+ * RUA_LEN_SAME); Bm, Cm: side->rows rows of N elements in the same storage; all of `dtype`.  A (H, N), h0 / h_final
+ * (B, H, N) in sequence order (for P the index in ragged->off) are of the ACCUMULATOR type (fp32, fp64 for RUA_F64).
+ * 1 <= N <= 16, H >= 0.  For token (i, t) of sequence i with length len[i] (rows from the "Row of token" formulas),
+ * channel h and state n:
+ *   dA_t[h, n] = exp(delta_t[h] A[h, n])
+ *   h_t[h, n]  = dA_t[h, n] h_{t-1}[h, n] + delta_t[h] Bm_t[n] x_t[h],   h_{-1} = h0[i] (0 when h0 is NULL)
+ *   y_t[h]     = sum_n Cm_t[n] h_t[h, n]
+ *   h_final[i] = h at the last token (h0[i], or 0, for an empty sequence)
+ * reverse = 1 runs from each sequence's end: h_t depends on h_{t+1}, h_{len} = h0[i], h_final[i] is the state at t = 0.
+ * fp32 accumulation (fp64 for RUA_F64), one rounding of y.  Rows that hold no token (L / R padding, C rows at or past
+ * off[B]) are copied through from x.  ragged->sorted is required (B > 0): CTA (cb, g) of a fixed grid takes channel
+ * block cb of the sequences of ranks g, g + G, ... in that order, so every result is bit-identical run to run and, for
+ * the same sequences, on every layout.  No float atomics anywhere. */
+
+/* bytes of the state rua_ssm_forward keeps for rua_ssm_backward: the state entering every chunk of 32 steps of every
+ * sequence, (rows / 32 + B) x H x N accumulator-type values (at most one H x N state per 32 tokens of each sequence plus
+ * one per sequence; with rows >= sum(len)).  Host only; 0 when an argument is invalid. */
+size_t rua_ssm_state_bytes(int64_t rows, int64_t B, int64_t H, int32_t N, int32_t dtype);
+/* workspace of rua_ssm_backward when grad_A, grad_B or grad_C is wanted (0 when rows, B or H is 0, or an argument is
+ * invalid), in accumulator-type values:
+ *   G x H x N grad_A slots, G = min(B, ceil(148 c / ceil(H / W))) with c <= 8 CTAs per SM, rounded up to 256 bytes,
+ *   + ceil(H / W) x rows x 2N partials of [grad_B | grad_C] per (token, channel block),
+ * with W = 128 channels per block (64 for RUA_F64).  Monotone in rows. */
+size_t rua_ssm_workspace_bytes(int64_t rows, int64_t B, int64_t H, int32_t N, int32_t dtype);
+
+/* y (and h_final when not NULL) as above.  state_out: rua_ssm_state_bytes(side->rows, B, H, N, dtype) bytes for
+ * rua_ssm_backward, or NULL.  No workspace (ws may be NULL). */
+int rua_ssm_forward(const void* x, const void* delta, const void* A, const void* Bm, const void* Cm, const void* h0,
+                    void* y, void* h_final, void* state_out, int64_t H, int32_t N, int32_t dtype, int32_t reverse,
+                    const rua_ragged_t* ragged, const rua_side_t* side, void* ws, size_t ws_bytes, rua_stream_t stream);
+
+/* gradients of sum g y with the state of the rua_ssm_forward call on the same x / delta / A / Bm / Cm / h0 / reverse /
+ * ragged / side.  In processing order, with dh_t the adjoint of h_t (0 past the last token):
+ *   dh_t[h, n]      = Cm_t[n] g_t[h] + dA_{t+1}[h, n] dh_{t+1}[h, n]
+ *   grad_x_t[h]     = delta_t[h] sum_n Bm_t[n] dh_t[h, n]
+ *   grad_delta_t[h] = sum_n dh_t[h, n] (A[h, n] dA_t[h, n] h_{t-1}[h, n] + Bm_t[n] x_t[h])
+ *   grad_A[h, n]    = sum over all tokens of dh_t[h, n] delta_t[h] dA_t[h, n] h_{t-1}[h, n]
+ *   grad_Bm_t[n]    = sum_h dh_t[h, n] delta_t[h] x_t[h]
+ *   grad_Cm_t[n]    = sum_h g_t[h] h_t[h, n]
+ *   grad_h0[i]      = dA_0 dh_0 (0 for an empty sequence)
+ * grad_A and grad_h0 are of the accumulator type, the others of `dtype`.  Any gradient pointer may be NULL and is then not
+ * computed.  Rows that hold no token pass grad_out through to grad_x and get 0 in grad_delta, grad_Bm and grad_Cm.  The
+ * kernel recomputes each chunk's states from its checkpoint.  Deterministic: grad_A is summed per CTA slot in slot order,
+ * grad_Bm / grad_Cm per token in a fixed warp / block order, by a second kernel.  ws: rua_ssm_workspace_bytes(side->rows,
+ * B, H, N, dtype) bytes when grad_A, grad_Bm or grad_Cm is wanted.  No token at all: grad_x is copied from grad_out and the
+ * other gradients are zeroed on `stream`. */
+int rua_ssm_backward(const void* grad_out, const void* x, const void* delta, const void* A, const void* Bm, const void* Cm,
+                     const void* state, void* grad_x, void* grad_delta, void* grad_A, void* grad_Bm, void* grad_Cm,
+                     void* grad_h0, int64_t H, int32_t N, int32_t dtype, int32_t reverse, const rua_ragged_t* ragged,
+                     const rua_side_t* side, void* ws, size_t ws_bytes, rua_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------- */
 /* K5  multi-GPU output gather over NVLink peer memory (SURVEY.md 8e-3; the reference is         */
 /* single-device).  One process per GPU; the batch is sharded by sequence; every rank stores its */
 /* rows directly into the output buffers ("windows") of all ranks of the node.                   */

@@ -1696,6 +1696,148 @@ def crf_decode(emissions: Tensor, transitions: Tensor, start: Optional[Tensor], 
 
 
 # ------------------------------------------------------------------------------------------------
+# K10: per-sequence selective state-space scan (+ autograd)
+# ------------------------------------------------------------------------------------------------
+SSM_MAX_N = 16
+
+
+def ssm_check(data: Tensor, delta: Tensor, A: Tensor, Bm: Tensor, Cm: Tensor, initial: Optional[Tensor], B: int,
+              lead: int) -> Tuple[Tuple[int, ...], int]:
+    """validate a selective scan over ``data`` with ``lead`` row dimensions -> (feat, N), before any device work."""
+    if data.dtype not in _DTYPES:
+        raise RuntimeError(f'torchrua_b200: selective_scan supports float16/bfloat16/float32/float64, got {data.dtype}')
+    acc = _crf_acc_dtype(data.dtype)
+    for name, t, want in (('delta', delta, data.dtype), ('B', Bm, data.dtype), ('C', Cm, data.dtype), ('A', A, acc),
+                          ('initial', initial, acc)):
+        if t is not None and t.dtype != want:
+            raise RuntimeError(f'torchrua_b200: selective_scan {name} must have dtype {want} for a {data.dtype} input, '
+                               f'got {t.dtype}')
+    if data.dim() < lead:
+        raise ValueError(f'torchrua_b200: selective_scan input must have {lead} row dimension(s), '
+                         f'got shape {tuple(data.shape)}')
+    rows, feat = tuple(data.shape[:lead]), tuple(data.shape[lead:])
+    if tuple(delta.shape) != tuple(data.shape):
+        raise ValueError(f'torchrua_b200: selective_scan delta must have the shape of the input {tuple(data.shape)}, '
+                         f'got {tuple(delta.shape)}')
+    if Bm.dim() != lead + 1 or tuple(Bm.shape[:lead]) != rows:
+        raise ValueError(f'torchrua_b200: selective_scan B must be {rows} + (N,), got {tuple(Bm.shape)}')
+    N = Bm.shape[-1]
+    if not 1 <= N <= SSM_MAX_N:
+        raise ValueError(f'torchrua_b200: selective_scan supports state sizes 1..{SSM_MAX_N}, got {N}')
+    if tuple(Cm.shape) != tuple(Bm.shape):
+        raise ValueError(f'torchrua_b200: selective_scan C must have the shape of B {tuple(Bm.shape)}, '
+                         f'got {tuple(Cm.shape)}')
+    if tuple(A.shape) != feat + (N,):
+        raise ValueError(f'torchrua_b200: selective_scan A must be (*feat, N) = {feat + (N,)}, got {tuple(A.shape)}')
+    if initial is not None and tuple(initial.shape) != (B,) + feat + (N,):
+        raise ValueError(f'torchrua_b200: selective_scan initial must be (batch, *feat, N) = {(B,) + feat + (N,)}, '
+                         f'got {tuple(initial.shape)}')
+    require_cuda(data, delta, A, Bm, Cm, initial)
+    return feat, N
+
+
+def _ssm_forward_raw(x: Tensor, dl: Tensor, A: Tensor, Bm: Tensor, Cm: Tensor, h0: Optional[Tensor], rg: Ragged,
+                     side: SideSpec, reverse: bool, want_final: bool, keep_state: bool):
+    """(y, final or None, state or None); x, dl (side.rows, H), A (H, N), Bm, Cm (side.rows, N), h0 (B, H, N) or None,
+    all contiguous."""
+    lib = _lib.load()
+    H, N = A.shape
+    dt = _DTYPES[x.dtype]
+    y = torch.empty_like(x)
+    fin = torch.empty((rg.B, H, N), dtype=A.dtype, device=x.device) if want_final else None
+    state = None
+    if keep_state:
+        state = torch.empty(lib.rua_ssm_state_bytes(side.rows, rg.B, H, N, dt), dtype=torch.uint8, device=x.device)
+    c_rg, c_side = rg.c_struct(), side.c_struct()
+    with _on(x.device):
+        prof = _profile_begin()
+        _lib.check(lib.rua_ssm_forward(x.data_ptr(), dl.data_ptr(), A.data_ptr(), Bm.data_ptr(), Cm.data_ptr(), _ptr(h0),
+                                       y.data_ptr(), _ptr(fin), _ptr(state) if state is not None and state.numel() else None,
+                                       H, N, dt, int(reverse), ctypes.byref(c_rg), ctypes.byref(c_side), None, 0,
+                                       _stream()), 'rua_ssm_forward')
+        if prof is not None:
+            # x and delta read once, y written once, B and C read once per channel block + checkpoints
+            nb = 3 * x.numel() * x.element_size() + 2 * Bm.numel() * Bm.element_size() + \
+                (state.numel() if state is not None else 0)
+            _profile_end(prof, 'ssm_forward', nb + 8 * rg.B + (8 * (rg.Tp + rg.B) if side.layout == PACK else 0))
+    return y, fin, state
+
+
+def _ssm_backward_raw(g: Tensor, x: Tensor, dl: Tensor, A: Tensor, Bm: Tensor, Cm: Tensor, state: Tensor, rg: Ragged,
+                      side: SideSpec, reverse: bool, want):
+    """(grad_x, grad_delta, grad_A, grad_B, grad_C, grad_initial), None where ``want`` is False; inputs contiguous."""
+    lib = _lib.load()
+    H, N = A.shape
+    dt = _DTYPES[x.dtype]
+    outs = (torch.empty_like(x) if want[0] else None, torch.empty_like(x) if want[1] else None,
+            torch.empty_like(A) if want[2] else None, torch.empty_like(Bm) if want[3] else None,
+            torch.empty_like(Cm) if want[4] else None,
+            torch.empty((rg.B, H, N), dtype=A.dtype, device=x.device) if want[5] else None)
+    if not any(want):
+        return outs
+    c_rg, c_side = rg.c_struct(), side.c_struct()
+    with _on(x.device):
+        nbytes = lib.rua_ssm_workspace_bytes(side.rows, rg.B, H, N, dt) if any(want[2:5]) else 0
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
+        prof = _profile_begin()
+        _lib.check(lib.rua_ssm_backward(g.data_ptr(), x.data_ptr(), dl.data_ptr(), A.data_ptr(), Bm.data_ptr(),
+                                        Cm.data_ptr(), _ptr(state) if state.numel() else None, *(_ptr(t) for t in outs),
+                                        H, N, dt, int(reverse), ctypes.byref(c_rg), ctypes.byref(c_side),
+                                        ws.data_ptr() if nbytes else None, nbytes, _stream()), 'rua_ssm_backward')
+        if prof is not None:
+            # grad_out, x and delta read twice (recompute + adjoint), grad_x and grad_delta written once + checkpoints
+            e = x.element_size()
+            nb = x.numel() * e * (6 + want[0] + want[1]) + state.numel() + 2 * nbytes
+            _profile_end(prof, 'ssm_backward', nb + 8 * rg.B + (8 * (rg.Tp + rg.B) if side.layout == PACK else 0))
+    return outs
+
+
+class _SelectiveScan(torch.autograd.Function):
+    """(y, final or None); final is not differentiable.  Once-differentiable: the backward is a native kernel, double
+    backward is not supported."""
+
+    @staticmethod
+    def forward(ctx, x: Tensor, dl: Tensor, A: Tensor, Bm: Tensor, Cm: Tensor, h0: Optional[Tensor], rg: Ragged,
+                side: SideSpec, reverse: bool, want_final: bool):
+        xs, ds, As, Bs, Cs = (t.detach().contiguous() for t in (x, dl, A, Bm, Cm))
+        hs = None if h0 is None else h0.detach().contiguous()
+        y, fin, state = _ssm_forward_raw(xs, ds, As, Bs, Cs, hs, rg, side, reverse, want_final, True)
+        if fin is not None:
+            ctx.mark_non_differentiable(fin)
+        ctx.meta = (rg, side, reverse, h0 is not None)
+        ctx.save_for_backward(xs, ds, As, Bs, Cs, state)
+        return y, fin
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_y: Optional[Tensor], grad_fin: Optional[Tensor]):
+        rg, side, reverse, has_h0 = ctx.meta
+        x, dl, A, Bm, Cm, state = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        want = (need[0], need[1], need[2], need[3], need[4], need[5] and has_h0)
+        g = grad_y.contiguous() if grad_y is not None else torch.zeros_like(x)
+        return (*_ssm_backward_raw(g, x, dl, A, Bm, Cm, state, rg, side, reverse, want), None, None, None, None)
+
+
+def selective_scan(data: Tensor, delta: Tensor, A: Tensor, Bm: Tensor, Cm: Tensor, initial: Optional[Tensor],
+                   rg: Ragged, side: SideSpec, reverse: bool, want_final: bool) -> Tuple[Tensor, Optional[Tensor]]:
+    """(y like data, final (B, *feat, N) or None) of the selective scan over the flattened storage: data, delta
+    (side.rows, *feat), Bm, Cm (side.rows, N), A (*feat, N), initial (B, *feat, N) or None; checked by the caller
+    (ssm_check); ``rg`` has its pack side."""
+    rows, feat, N = data.shape[0], tuple(data.shape[1:]), A.shape[-1]
+    H = int(np.prod(feat))
+    args = (data.reshape(rows, H), delta.reshape(rows, H), A.reshape(H, N), Bm, Cm,
+            None if initial is None else initial.reshape(rg.B, H, N))
+    grad = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (data, delta, A, Bm, Cm, initial))
+    if grad:
+        y, fin = _SelectiveScan.apply(*args, rg, side, reverse, want_final)
+    else:
+        y, fin, _ = _ssm_forward_raw(*(None if t is None else t.contiguous() for t in args), rg, side, reverse,
+                                     want_final, False)
+    return y.view(data.shape), None if fin is None else fin.view((rg.B,) + feat + (N,))
+
+
+# ------------------------------------------------------------------------------------------------
 # scatter_*: stable sort of the index + bucket boundaries + segment reduce over GATHERED rows
 # ------------------------------------------------------------------------------------------------
 def sort_keys(keys: Tensor, max_key: int) -> Tuple[Tensor, Tensor]:

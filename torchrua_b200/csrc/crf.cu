@@ -30,6 +30,7 @@
 //     K = 64), the CTA sums its warps in warp order into its own workspace slot, and slot_sum adds the slots in slot
 //     order: no atomics, bit-identical run to run.  The grid is a host function of (B, K, dtype).
 #include "reduce_common.cuh"
+#include "seq_rows.cuh"
 #include "slot_sum.cuh"
 
 namespace rua {
@@ -70,35 +71,6 @@ struct CrfArgs {
   int64_t Wd;             // L / R width
   int64_t rows;
 };
-
-struct Seq {
-  int64_t i, o, len, prow;
-};
-
-__device__ __forceinline__ Seq seq_of(const CrfArgs& a, int64_t rank) {
-  Seq s;
-  s.i = __ldg(a.sorted + rank);
-  s.o = __ldg(a.off + s.i);
-  s.len = __ldg(a.off + s.i + 1) - s.o;
-  s.prow = a.layout == RUA_PACK ? __ldg(a.unsorted + s.i) : 0;
-  return s;
-}
-
-__device__ __forceinline__ int64_t row_of(const CrfArgs& a, const Seq& s, int64_t t) {
-  switch (a.layout) {
-    case RUA_CAT: return s.o + t;
-    case RUA_LEFT: return s.i * a.Wd + t;
-    case RUA_RIGHT: return s.i * a.Wd + (a.Wd - s.len) + t;
-    default: return __ldg(a.poff + t) + s.prow;
-  }
-}
-
-// f(row) for every row of sequence s's L / R storage that holds no token, spread over the lanes
-template <class F> __device__ __forceinline__ void for_padding_rows(const CrfArgs& a, const Seq& s, int lane, F&& f) {
-  if (a.layout != RUA_LEFT && a.layout != RUA_RIGHT) return;
-  const int64_t base = s.i * a.Wd + (a.layout == RUA_LEFT ? s.len : 0);
-  for (int64_t q = lane; q < a.Wd - s.len; q += 32) f(base + q);
-}
 
 template <typename A> __device__ __forceinline__ A neg_inf() { return (A)(-INFINITY); }
 __device__ __forceinline__ float fexp(float v) { return __expf(v); }
@@ -182,7 +154,7 @@ __global__ void __launch_bounds__(kFwdWarps * 32, 2) crf_forward_kernel(CrfArgs 
   const int64_t G = (int64_t)gridDim.x * kFwdWarps;
   for (int64_t rank = blockIdx.x * (int64_t)kFwdWarps + warp; rank < a.B; rank += G) {
     const Seq s = seq_of(a, rank);
-    if constexpr (kMax) for_padding_rows(a, s, lane, [&](int64_t r) { a.tags_out[r] = -1; });
+    if constexpr (kMax) for_padding_rows(a, s, lane, 32, [&](int64_t r) { a.tags_out[r] = -1; });
     if (s.len == 0) {
       if (lane == 0) {
         if constexpr (kMax) static_cast<A*>(a.score)[s.i] = A(0);
@@ -375,7 +347,7 @@ __global__ void __launch_bounds__(kBwdWarps * 32, 4) crf_backward_kernel(CrfArgs
   const int64_t G = (int64_t)gridDim.x * kBwdWarps;
   for (int64_t rank = blockIdx.x * (int64_t)kBwdWarps + warp; rank < a.B; rank += G) {
     const Seq s = seq_of(a, rank);
-    if (gx) for_padding_rows(a, s, lane, [&](int64_t r) {
+    if (gx) for_padding_rows(a, s, lane, 32, [&](int64_t r) {
       for (int b = 0; b < K; ++b) gx[r * K + b] = zero;
     });
     if (s.len == 0) continue;
