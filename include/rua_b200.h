@@ -507,6 +507,65 @@ int rua_ssm_backward(const void* grad_out, const void* x, const void* delta, con
                      const rua_side_t* side, void* ws, size_t ws_bytes, rua_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------- */
+/* K11 per-sequence Mamba-2 (SSD) state-space scan: a scalar decay per head, a P x N state per   */
+/* head, B / C shared by the heads of a group (no counterpart in the reference; replaces pad ->  */
+/* a pure-torch chunked einsum that materialises (B, chunks, Q, Q, H) decay tensors)              */
+/* ------------------------------------------------------------------------------------------- */
+/* x, y: side->rows rows of H x P elements; delta: side->rows rows of H; Bm, Cm: side->rows rows of G x N; all in the
+ * storage of `side` (C, L, P or R over `ragged`; len_xform must be RUA_LEN_SAME) and of `dtype`.  A (H), h0 / h_final
+ * (B, H, P, N) in sequence order (for P the index in ragged->off) are of the ACCUMULATOR type (fp32, fp64 for RUA_F64).
+ * 1 <= P <= 64, 1 <= N <= 128, G >= 1, H >= 0, H % G == 0.  For token (i, t), head h, channel p, state n and group
+ * g = h / (H / G):
+ *   dA_t      = exp(delta_t[h] A[h])
+ *   h_t[p, n] = dA_t h_{t-1}[p, n] + delta_t[h] x_t[h, p] Bm_t[g, n],   h_{-1} = h0[i, h] (0 when h0 is NULL)
+ *   y_t[h, p] = sum_n Cm_t[g, n] h_t[p, n]
+ *   h_final[i, h] = h at the last token (h0[i, h], or 0, for an empty sequence)
+ * reverse = 1 runs from each sequence's end.  Chunked form over Q = 64 tokens of one sequence (16 for RUA_F64); the
+ * carried state is kept in the accumulator type and never rounded.  For fp16 / bf16 the operands of the tensor-core
+ * products are rounded to `dtype` once each (delta x, the decay-masked scores exp(cum_t - cum_s) (C_t . B_s), the
+ * decay-weighted B of the state update and the copy of the state that C reads); fp32 / fp64 round only y.  Rows that
+ * hold no token (L / R padding, C rows at or past off[B]) are copied through from x.  ragged->sorted is required
+ * (B > 0); the sequence-to-CTA assignment is fixed, so every result is bit-identical run to run and, for the same
+ * sequences, on every layout.  No float atomics; every sum runs in a fixed order. */
+
+/* workspace of rua_ssd_backward (0 when rows, B or H is 0, or an argument is invalid), in accumulator-type values, with
+ * grid = min(B G, 296), Q = 64 (16 for RUA_F64) and Tmax = ragged->Tp (at least the longest sequence):
+ *   grid x H grad_A slots, rounded up to 256 bytes,
+ *   + grid x (ceil(Tmax / Q) P N + Tmax 2N): per CTA, the chunk-start states of one head and [grad_B | grad_C] of one
+ *     sequence.
+ * Host only; monotone in every size argument. */
+size_t rua_ssd_workspace_bytes(int64_t rows, int64_t B, int64_t Tmax, int64_t H, int32_t P, int32_t G, int32_t N,
+                               int32_t dtype);
+
+/* y (and h_final when not NULL) as above.  No workspace (ws may be NULL), and nothing is kept for the backward, which
+ * recomputes the states it needs. */
+int rua_ssd_forward(const void* x, const void* delta, const void* A, const void* Bm, const void* Cm, const void* h0,
+                    void* y, void* h_final, int64_t H, int32_t P, int32_t G, int32_t N, int32_t dtype, int32_t reverse,
+                    const rua_ragged_t* ragged, const rua_side_t* side, void* ws, size_t ws_bytes, rua_stream_t stream);
+
+/* gradients of sum g y for the rua_ssd_forward call on the same x / delta / A / Bm / Cm / h0 / reverse / ragged / side.
+ * In processing order, with dh_t the adjoint of h_t (0 past the last token):
+ *   dh_t          = Cm_t[g] (x) g_t[h] + dA_{t+1} dh_{t+1}
+ *   grad_x_t[h]   = delta_t[h] sum_n Bm_t[g, n] dh_t[., n]
+ *   grad_delta_t  = A dA_t <dh_t, h_{t-1}> + <dh_t, x_t[h] (x) Bm_t[g]>
+ *   grad_A[h]     = sum over all tokens of delta_t dA_t <dh_t, h_{t-1}>
+ *   grad_Bm_t[g]  = sum_{h in g} delta_t[h] sum_p x_t[h, p] dh_t[p, .]
+ *   grad_Cm_t[g]  = sum_{h in g} sum_p g_t[h, p] h_t[p, .]
+ *   grad_h0[i, h] = dA_0 dh_0 (0 for an empty sequence)
+ * grad_A and grad_h0 are of the accumulator type, the others of `dtype`.  Any gradient pointer may be NULL and is then not
+ * written.  Rows that hold no token pass grad_out through to grad_x and get 0 in grad_delta, grad_Bm and grad_Cm.  The
+ * unit of work is (sequence, group); per head it recomputes the chunk-start states, then walks the chunks from the end.
+ * grad_Bm / grad_Cm are summed over a group's heads in head order, grad_A per CTA slot in slot order.  ws:
+ * rua_ssd_workspace_bytes(side->rows, B, ragged->Tp, H, P, G, N, dtype) bytes; ragged->Tp must be at least the longest
+ * sequence (the lengths live on the device): a longer sequence gets NaN in every gradient it reaches (its rows of
+ * grad_x, grad_delta, grad_Bm, grad_Cm, its grad_h0 and grad_A of its heads).  No token at all: grad_x is copied from
+ * grad_out and the other gradients are zeroed on `stream`. */
+int rua_ssd_backward(const void* grad_out, const void* x, const void* delta, const void* A, const void* Bm, const void* Cm,
+                     const void* h0, void* grad_x, void* grad_delta, void* grad_A, void* grad_Bm, void* grad_Cm,
+                     void* grad_h0, int64_t H, int32_t P, int32_t G, int32_t N, int32_t dtype, int32_t reverse,
+                     const rua_ragged_t* ragged, const rua_side_t* side, void* ws, size_t ws_bytes, rua_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------- */
 /* K5  multi-GPU output gather over NVLink peer memory (SURVEY.md 8e-3; the reference is         */
 /* single-device).  One process per GPU; the batch is sharded by sequence; every rank stores its */
 /* rows directly into the output buffers ("windows") of all ranks of the node.                   */

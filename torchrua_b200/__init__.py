@@ -17,6 +17,7 @@ from torchrua_b200.reduce import *  # noqa: F401,F403
 from torchrua_b200.scan import *  # noqa: F401,F403
 from torchrua_b200.segment import *  # noqa: F401,F403
 from torchrua_b200.ssm import *  # noqa: F401,F403
+from torchrua_b200.ssd import *  # noqa: F401,F403
 from torchrua_b200.select import *  # noqa: F401,F403
 
 __version__ = '0.1.0'

@@ -112,6 +112,13 @@ SIGNATURES = {
     'rua_ssm_backward': (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                    c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32,
                                    POINTER(Ragged), POINTER(Side), c_void_p, c_size_t, c_void_p]),
+    'rua_ssd_workspace_bytes': (c_size_t, [c_int64, c_int64, c_int64, c_int64, c_int32, c_int32, c_int32, c_int32]),
+    'rua_ssd_forward': (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                  c_int64, c_int32, c_int32, c_int32, c_int32, c_int32, POINTER(Ragged), POINTER(Side),
+                                  c_void_p, c_size_t, c_void_p]),
+    'rua_ssd_backward': (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                   c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, c_int32,
+                                   c_int32, POINTER(Ragged), POINTER(Side), c_void_p, c_size_t, c_void_p]),
     'rua_peer_window_alloc': (c_int32, [c_size_t, POINTER(c_void_p), c_char_p]),
     'rua_peer_window_open': (c_int32, [c_char_p, POINTER(c_void_p)]),
     'rua_peer_window_close': (c_int32, [c_void_p]),

@@ -1838,6 +1838,144 @@ def selective_scan(data: Tensor, delta: Tensor, A: Tensor, Bm: Tensor, Cm: Tenso
 
 
 # ------------------------------------------------------------------------------------------------
+# K11: per-sequence Mamba-2 (SSD) state-space scan (+ autograd)
+# ------------------------------------------------------------------------------------------------
+SSD_MAX_P = 64
+SSD_MAX_N = 128
+
+
+def ssd_check(data: Tensor, delta: Tensor, A: Tensor, Bm: Tensor, Cm: Tensor, initial: Optional[Tensor], B: int,
+              lead: int) -> Tuple[int, int, int, int]:
+    """validate an SSD scan over ``data`` (*rows, H, P) with ``lead`` row dimensions -> (H, P, G, N), before any device
+    work."""
+    if data.dtype not in _DTYPES:
+        raise RuntimeError(f'torchrua_b200: ssd supports float16/bfloat16/float32/float64, got {data.dtype}')
+    acc = _crf_acc_dtype(data.dtype)
+    for name, t, want in (('delta', delta, data.dtype), ('B', Bm, data.dtype), ('C', Cm, data.dtype), ('A', A, acc),
+                          ('initial', initial, acc)):
+        if t is not None and t.dtype != want:
+            raise RuntimeError(f'torchrua_b200: ssd {name} must have dtype {want} for a {data.dtype} input, '
+                               f'got {t.dtype}')
+    if data.dim() != lead + 2:
+        raise ValueError(f'torchrua_b200: ssd input must be {lead} row dimension(s) + (H, P), '
+                         f'got shape {tuple(data.shape)}')
+    rows, (H, P) = tuple(data.shape[:lead]), tuple(data.shape[lead:])
+    if tuple(delta.shape) != rows + (H,):
+        raise ValueError(f'torchrua_b200: ssd delta must be {rows + (H,)}, got {tuple(delta.shape)}')
+    if Bm.dim() != lead + 2 or tuple(Bm.shape[:lead]) != rows:
+        raise ValueError(f'torchrua_b200: ssd B must be {rows} + (G, N), got {tuple(Bm.shape)}')
+    G, N = Bm.shape[lead:]
+    if tuple(Cm.shape) != tuple(Bm.shape):
+        raise ValueError(f'torchrua_b200: ssd C must have the shape of B {tuple(Bm.shape)}, got {tuple(Cm.shape)}')
+    if G < 1 or H % G:
+        raise ValueError(f'torchrua_b200: ssd needs the heads H = {H} to split into G = {G} groups')
+    if not 1 <= P <= SSD_MAX_P:
+        raise ValueError(f'torchrua_b200: ssd supports head dims 1..{SSD_MAX_P}, got {P}')
+    if not 1 <= N <= SSD_MAX_N:
+        raise ValueError(f'torchrua_b200: ssd supports state sizes 1..{SSD_MAX_N}, got {N}')
+    if tuple(A.shape) != (H,):
+        raise ValueError(f'torchrua_b200: ssd A must be (H,) = {(H,)}, got {tuple(A.shape)}')
+    if initial is not None and tuple(initial.shape) != (B, H, P, N):
+        raise ValueError(f'torchrua_b200: ssd initial must be (batch, H, P, N) = {(B, H, P, N)}, '
+                         f'got {tuple(initial.shape)}')
+    require_cuda(data, delta, A, Bm, Cm, initial)
+    return H, P, G, N
+
+
+def _ssd_forward_raw(x: Tensor, dl: Tensor, A: Tensor, Bm: Tensor, Cm: Tensor, h0: Optional[Tensor], rg: Ragged,
+                     side: SideSpec, reverse: bool, want_final: bool):
+    """(y, final or None); x (side.rows, H, P), dl (side.rows, H), A (H,), Bm, Cm (side.rows, G, N), h0 (B, H, P, N) or
+    None, all contiguous."""
+    lib = _lib.load()
+    H, P = x.shape[1:]
+    G, N = Bm.shape[1:]
+    y = torch.empty_like(x)
+    fin = torch.empty((rg.B, H, P, N), dtype=A.dtype, device=x.device) if want_final else None
+    c_rg, c_side = rg.c_struct(), side.c_struct()
+    with _on(x.device):
+        prof = _profile_begin()
+        _lib.check(lib.rua_ssd_forward(x.data_ptr(), dl.data_ptr(), A.data_ptr(), Bm.data_ptr(), Cm.data_ptr(), _ptr(h0),
+                                       y.data_ptr(), _ptr(fin), H, P, G, N, _DTYPES[x.dtype], int(reverse),
+                                       ctypes.byref(c_rg), ctypes.byref(c_side), None, 0, _stream()), 'rua_ssd_forward')
+        if prof is not None:
+            # x and y once, delta once, B and C once per head
+            nb = 2 * x.numel() * x.element_size() + dl.numel() * dl.element_size() + \
+                2 * Bm.numel() * Bm.element_size() * (H // G)
+            _profile_end(prof, 'ssd_forward', nb + 8 * rg.B + (8 * (rg.Tp + rg.B) if side.layout == PACK else 0))
+    return y, fin
+
+
+def _ssd_backward_raw(g: Tensor, x: Tensor, dl: Tensor, A: Tensor, Bm: Tensor, Cm: Tensor, h0: Optional[Tensor],
+                      rg: Ragged, side: SideSpec, reverse: bool, want):
+    """(grad_x, grad_delta, grad_A, grad_B, grad_C, grad_initial), None where ``want`` is False; inputs contiguous."""
+    lib = _lib.load()
+    H, P = x.shape[1:]
+    G, N = Bm.shape[1:]
+    dt = _DTYPES[x.dtype]
+    outs = (torch.empty_like(x) if want[0] else None, torch.empty_like(dl) if want[1] else None,
+            torch.empty_like(A) if want[2] else None, torch.empty_like(Bm) if want[3] else None,
+            torch.empty_like(Cm) if want[4] else None,
+            torch.empty((rg.B, H, P, N), dtype=A.dtype, device=x.device) if want[5] else None)
+    if not any(want):
+        return outs
+    c_rg, c_side = rg.c_struct(), side.c_struct()
+    with _on(x.device):
+        nbytes = lib.rua_ssd_workspace_bytes(side.rows, rg.B, rg.Tp, H, P, G, N, dt)
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
+        prof = _profile_begin()
+        _lib.check(lib.rua_ssd_backward(g.data_ptr(), x.data_ptr(), dl.data_ptr(), A.data_ptr(), Bm.data_ptr(),
+                                        Cm.data_ptr(), _ptr(h0), *(_ptr(t) for t in outs), H, P, G, N, dt,
+                                        int(reverse), ctypes.byref(c_rg), ctypes.byref(c_side),
+                                        ws.data_ptr() if nbytes else None, nbytes, _stream()), 'rua_ssd_backward')
+        if prof is not None:
+            # x, delta, grad_out twice (recompute + reverse sweep), B and C twice per head, the gradients once
+            e = x.element_size()
+            nb = x.numel() * e * (3 + want[0]) + dl.numel() * e * (2 + want[1]) + \
+                Bm.numel() * e * (4 * (H // G) + want[3] + want[4])
+            _profile_end(prof, 'ssd_backward', nb + 8 * rg.B + (8 * (rg.Tp + rg.B) if side.layout == PACK else 0))
+    return outs
+
+
+class _SSD(torch.autograd.Function):
+    """(y, final or None); final is not differentiable.  Saves only its inputs: the backward recomputes the states.
+    Once-differentiable: the backward is a native kernel, double backward is not supported."""
+
+    @staticmethod
+    def forward(ctx, x: Tensor, dl: Tensor, A: Tensor, Bm: Tensor, Cm: Tensor, h0: Optional[Tensor], rg: Ragged,
+                side: SideSpec, reverse: bool, want_final: bool):
+        xs, ds, As, Bs, Cs = (t.detach().contiguous() for t in (x, dl, A, Bm, Cm))
+        hs = None if h0 is None else h0.detach().contiguous()
+        y, fin = _ssd_forward_raw(xs, ds, As, Bs, Cs, hs, rg, side, reverse, want_final)
+        if fin is not None:
+            ctx.mark_non_differentiable(fin)
+        ctx.meta = (rg, side, reverse, h0 is not None)
+        ctx.save_for_backward(xs, ds, As, Bs, Cs, hs)
+        return y, fin
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_y: Optional[Tensor], grad_fin: Optional[Tensor]):
+        rg, side, reverse, has_h0 = ctx.meta
+        x, dl, A, Bm, Cm, h0 = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        want = (need[0], need[1], need[2], need[3], need[4], need[5] and has_h0)
+        g = grad_y.contiguous() if grad_y is not None else torch.zeros_like(x)
+        return (*_ssd_backward_raw(g, x, dl, A, Bm, Cm, h0, rg, side, reverse, want), None, None, None, None)
+
+
+def ssd(data: Tensor, delta: Tensor, A: Tensor, Bm: Tensor, Cm: Tensor, initial: Optional[Tensor], rg: Ragged,
+        side: SideSpec, reverse: bool, want_final: bool) -> Tuple[Tensor, Optional[Tensor]]:
+    """(y like data, final (B, H, P, N) or None) of the SSD scan over the flattened storage: data (side.rows, H, P),
+    delta (side.rows, H), Bm, Cm (side.rows, G, N), A (H,), initial (B, H, P, N) or None; checked by the caller
+    (ssd_check); ``rg`` has its pack side."""
+    args = (data, delta, A, Bm, Cm, initial)
+    grad = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in args)
+    if grad:
+        return _SSD.apply(*args, rg, side, reverse, want_final)
+    return _ssd_forward_raw(*(None if t is None else t.contiguous() for t in args), rg, side, reverse, want_final)
+
+
+# ------------------------------------------------------------------------------------------------
 # scatter_*: stable sort of the index + bucket boundaries + segment reduce over GATHERED rows
 # ------------------------------------------------------------------------------------------------
 def sort_keys(keys: Tensor, max_key: int) -> Tuple[Tensor, Tensor]:
