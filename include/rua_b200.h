@@ -566,6 +566,67 @@ int rua_ssd_backward(const void* grad_out, const void* x, const void* delta, con
                      const rua_ragged_t* ragged, const rua_side_t* side, void* ws, size_t ws_bytes, rua_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------- */
+/* K12 per-sequence gated delta rule (Gated DeltaNet): a scalar log decay and write strength per  */
+/* token and value head, a K x V state per value head, q / k shared by the value heads of a key   */
+/* group (no counterpart in the reference; replaces pad -> a pure-torch chunked form)             */
+/* ------------------------------------------------------------------------------------------- */
+/* v, o: side->rows rows of H x V elements; q, k: side->rows rows of G x K; beta: side->rows rows of H; all in the
+ * storage of `side` (C, L, P or R over `ragged`; len_xform must be RUA_LEN_SAME) and of `dtype`.  g (side->rows rows of
+ * H, the log decay), h0 / h_final (B, H, K, V) in sequence order (for P the index in ragged->off) are of the ACCUMULATOR
+ * type (fp32, fp64 for RUA_F64).  1 <= K <= 128, 1 <= V <= 256, G >= 1, H >= 0, H % G == 0.  For token (i, t), value
+ * head h and key group c = h / (H / G), with S the K x V state of head h:
+ *   S'_t   = exp(g_t[h]) S_{t-1}                              S_{-1} = h0[i, h] (0 when h0 is NULL)
+ *   u_t    = beta_t[h] (v_t[h] - S'_t^T k_t[c])
+ *   S_t    = S'_t + k_t[c] (x) u_t
+ *   o_t[h] = scale S_t^T q_t[c]
+ *   h_final[i, h] = S at the last token (h0[i, h], or 0, for an empty sequence)
+ * reverse = 1 runs from each sequence's end.  Chunked form over Q tokens of one sequence (64 for fp16 / bf16, 32 for
+ * fp32, 16 for RUA_F64) and V blocks of 64 columns (32 for RUA_F64); the carried state, the per-chunk inverse
+ * T = (I + strict_tril(diag(beta) (K K^T) o exp(cum_t - cum_s)))^-1, cum and every exponential are kept in the
+ * accumulator type.  For fp16 / bf16 each operand of a tensor-core product is rounded to `dtype` once; fp32 / fp64
+ * round only o.  Rows that hold no token (L / R padding, C rows at or past off[B]) are copied through from v.
+ * ragged->sorted is required (B > 0); the sequence-to-CTA assignment is fixed, so every result is bit-identical run to
+ * run and, for the same sequences, on every layout.  No float atomics; every sum runs in a fixed order. */
+
+/* workspace of rua_gdn_backward (0 when rows, B or H is 0, or an argument is invalid), in accumulator-type values, with
+ * grid = min(B G, 296), Q and VB as above and Tmax = ragged->Tp (at least the longest sequence):
+ *   grid x (ceil(Tmax / Q) K VB + Tmax (2K + 2)): per CTA, the chunk-start states of one (head, V block) and
+ *   [grad_q | grad_k | grad_g | grad_beta] of one sequence.
+ * Host only; monotone in every size argument. */
+size_t rua_gdn_workspace_bytes(int64_t rows, int64_t B, int64_t Tmax, int64_t H, int32_t G, int32_t K, int32_t V,
+                               int32_t dtype);
+
+/* o (and h_final when not NULL) as above.  No workspace (ws may be NULL), and nothing is kept for the backward, which
+ * recomputes the states it needs. */
+int rua_gdn_forward(const void* v, const void* q, const void* k, const void* g, const void* beta, const void* h0, void* o,
+                    void* h_final, int64_t H, int32_t G, int32_t K, int32_t V, double scale, int32_t dtype,
+                    int32_t reverse, const rua_ragged_t* ragged, const rua_side_t* side, void* ws, size_t ws_bytes,
+                    rua_stream_t stream);
+
+/* gradients of sum grad_out o for the rua_gdn_forward call on the same v / q / k / g / beta / h0 / scale / reverse /
+ * ragged / side.  In processing order, with dS_t the adjoint of S_t (0 past the last token), p_t = S'_t^T k_t and
+ * du_t = dS_t^T k_t after dS_t = scale q_t (x) grad_out_t + exp(g_{t+1}) (I - beta_{t+1} k_{t+1} k_{t+1}^T) dS_{t+1}:
+ *   grad_v_t[h]      = beta_t du_t
+ *   grad_beta_t[h]   = <du_t, v_t - p_t>
+ *   grad_g_t[h]      = <dS_t - beta_t k_t (x) du_t, S'_t>
+ *   grad_q_t[c]      = scale sum_{h in c} S_t grad_out_t[h]
+ *   grad_k_t[c]      = sum_{h in c} (dS_t u_t - beta_t S'_t du_t)
+ *   grad_h0[i, h]    = exp(g_0) (I - beta_0 k_0 k_0^T) dS_0 (0 for an empty sequence)
+ * grad_g and grad_h0 are of the accumulator type, the others of `dtype`.  Any gradient pointer may be NULL and is then
+ * not written.  Rows that hold no token pass grad_out through to grad_v and get 0 in grad_q, grad_k, grad_g and
+ * grad_beta.  The unit of work is (sequence, key group); per (value head, V block) it recomputes the chunk-start states,
+ * then walks the chunks from the end.  grad_q / grad_k are summed over a group's heads and V blocks, grad_g / grad_beta
+ * over the V blocks, in that order.  ws: rua_gdn_workspace_bytes(side->rows, B, ragged->Tp, H, G, K, V, dtype) bytes;
+ * ragged->Tp must be at least the longest sequence (the lengths live on the device): a longer sequence gets NaN in every
+ * gradient it reaches (its rows of grad_v, grad_q, grad_k, grad_g, grad_beta and its grad_h0).  No token at all: grad_v
+ * is copied from grad_out and the other gradients are zeroed on `stream`. */
+int rua_gdn_backward(const void* grad_out, const void* v, const void* q, const void* k, const void* g, const void* beta,
+                     const void* h0, void* grad_v, void* grad_q, void* grad_k, void* grad_g, void* grad_beta,
+                     void* grad_h0, int64_t H, int32_t G, int32_t K, int32_t V, double scale, int32_t dtype,
+                     int32_t reverse, const rua_ragged_t* ragged, const rua_side_t* side, void* ws, size_t ws_bytes,
+                     rua_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------- */
 /* K5  multi-GPU output gather over NVLink peer memory (SURVEY.md 8e-3; the reference is         */
 /* single-device).  One process per GPU; the batch is sharded by sequence; every rank stores its */
 /* rows directly into the output buffers ("windows") of all ranks of the node.                   */

@@ -10,8 +10,8 @@ from torchrua_b200 import *  # noqa: F401,F403
 __version__ = _impl.__version__
 
 for _name in ('utils', 'layout', 'layout.cat', 'layout.left', 'layout.right', 'layout.pack', 'core', 'core.cast',
-              'core.get', 'core.set', 'core.view', 'conv', 'crf', 'mask', 'reduce', 'scan', 'segment', 'ssm', 'ssd',
-              'select', 'select.head', 'select.last', 'select.rev', 'select.roll', 'select.trunc', 'detach', 'compose',
+              'core.get', 'core.set', 'core.view', 'conv', 'crf', 'delta', 'mask', 'reduce', 'scan', 'segment', 'ssm',
+              'ssd', 'select', 'select.head', 'select.last', 'select.rev', 'select.roll', 'select.trunc', 'detach', 'compose',
               'shard'):
     sys.modules[f'{__name__}.{_name}'] = importlib.import_module(f'torchrua_b200.{_name}')
 for _name in ('utils', 'layout', 'core', 'reduce', 'segment', 'select', 'detach', 'shard'):

@@ -11,6 +11,7 @@ from torchrua_b200.core import *  # noqa: F401,F403
 from torchrua_b200.compose import *  # noqa: F401,F403
 from torchrua_b200.conv import *  # noqa: F401,F403
 from torchrua_b200.crf import *  # noqa: F401,F403
+from torchrua_b200.delta import *  # noqa: F401,F403
 from torchrua_b200.detach import *  # noqa: F401,F403
 from torchrua_b200.mask import *  # noqa: F401,F403
 from torchrua_b200.reduce import *  # noqa: F401,F403

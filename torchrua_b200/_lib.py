@@ -5,7 +5,7 @@ non-CUDA tensors are rejected by the callers in ``_native``.
 """
 import ctypes
 import os
-from ctypes import POINTER, Structure, c_char_p, c_int32, c_int64, c_size_t, c_void_p
+from ctypes import POINTER, Structure, c_char_p, c_double, c_int32, c_int64, c_size_t, c_void_p
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, 'lib', 'librua_b200.so')
@@ -119,6 +119,13 @@ SIGNATURES = {
     'rua_ssd_backward': (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                    c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, c_int32,
                                    c_int32, POINTER(Ragged), POINTER(Side), c_void_p, c_size_t, c_void_p]),
+    'rua_gdn_workspace_bytes': (c_size_t, [c_int64, c_int64, c_int64, c_int64, c_int32, c_int32, c_int32, c_int32]),
+    'rua_gdn_forward': (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                  c_int64, c_int32, c_int32, c_int32, c_double, c_int32, c_int32, POINTER(Ragged),
+                                  POINTER(Side), c_void_p, c_size_t, c_void_p]),
+    'rua_gdn_backward': (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                   c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, c_double,
+                                   c_int32, c_int32, POINTER(Ragged), POINTER(Side), c_void_p, c_size_t, c_void_p]),
     'rua_peer_window_alloc': (c_int32, [c_size_t, POINTER(c_void_p), c_char_p]),
     'rua_peer_window_open': (c_int32, [c_char_p, POINTER(c_void_p)]),
     'rua_peer_window_close': (c_int32, [c_void_p]),

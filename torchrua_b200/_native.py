@@ -1976,6 +1976,149 @@ def ssd(data: Tensor, delta: Tensor, A: Tensor, Bm: Tensor, Cm: Tensor, initial:
 
 
 # ------------------------------------------------------------------------------------------------
+# K12: per-sequence gated delta rule (Gated DeltaNet) (+ autograd)
+# ------------------------------------------------------------------------------------------------
+GDN_MAX_K = 128
+GDN_MAX_V = 256
+
+
+def gdn_check(data: Tensor, q: Tensor, k: Tensor, g: Tensor, beta: Tensor, initial: Optional[Tensor], B: int,
+              lead: int) -> Tuple[int, int, int, int]:
+    """validate a gated delta rule over ``data`` (*rows, H, V) with ``lead`` row dimensions -> (H, G, K, V), before any
+    device work."""
+    if data.dtype not in _DTYPES:
+        raise RuntimeError(f'torchrua_b200: gated_delta_rule supports float16/bfloat16/float32/float64, got {data.dtype}')
+    acc = _crf_acc_dtype(data.dtype)
+    for name, t, want in (('q', q, data.dtype), ('k', k, data.dtype), ('beta', beta, data.dtype), ('g', g, acc),
+                          ('initial', initial, acc)):
+        if t is not None and t.dtype != want:
+            raise RuntimeError(f'torchrua_b200: gated_delta_rule {name} must have dtype {want} for a {data.dtype} '
+                               f'input, got {t.dtype}')
+    if data.dim() != lead + 2:
+        raise ValueError(f'torchrua_b200: gated_delta_rule input must be {lead} row dimension(s) + (H, V), '
+                         f'got shape {tuple(data.shape)}')
+    rows, (H, V) = tuple(data.shape[:lead]), tuple(data.shape[lead:])
+    if q.dim() != lead + 2 or tuple(q.shape[:lead]) != rows:
+        raise ValueError(f'torchrua_b200: gated_delta_rule q must be {rows} + (G, K), got {tuple(q.shape)}')
+    G, K = q.shape[lead:]
+    if tuple(k.shape) != tuple(q.shape):
+        raise ValueError(f'torchrua_b200: gated_delta_rule k must have the shape of q {tuple(q.shape)}, '
+                         f'got {tuple(k.shape)}')
+    for name, t in (('g', g), ('beta', beta)):
+        if tuple(t.shape) != rows + (H,):
+            raise ValueError(f'torchrua_b200: gated_delta_rule {name} must be {rows + (H,)}, got {tuple(t.shape)}')
+    if G < 1 or H % G:
+        raise ValueError(f'torchrua_b200: gated_delta_rule needs the value heads H = {H} to split into G = {G} groups')
+    if not 1 <= K <= GDN_MAX_K:
+        raise ValueError(f'torchrua_b200: gated_delta_rule supports key dims 1..{GDN_MAX_K}, got {K}')
+    if not 1 <= V <= GDN_MAX_V:
+        raise ValueError(f'torchrua_b200: gated_delta_rule supports value dims 1..{GDN_MAX_V}, got {V}')
+    if initial is not None and tuple(initial.shape) != (B, H, K, V):
+        raise ValueError(f'torchrua_b200: gated_delta_rule initial must be (batch, H, K, V) = {(B, H, K, V)}, '
+                         f'got {tuple(initial.shape)}')
+    require_cuda(data, q, k, g, beta, initial)
+    return H, G, K, V
+
+
+def gdn_scale(scale: Optional[float], K: int) -> float:
+    """the output scale: K^-1/2 when None"""
+    return float(K) ** -0.5 if scale is None else float(scale)
+
+
+def _gdn_forward_raw(v: Tensor, q: Tensor, k: Tensor, g: Tensor, beta: Tensor, h0: Optional[Tensor], scale: float,
+                     rg: Ragged, side: SideSpec, reverse: bool, want_final: bool):
+    """(o, final or None); v (side.rows, H, V), q, k (side.rows, G, K), g, beta (side.rows, H), h0 (B, H, K, V) or None,
+    all contiguous."""
+    lib = _lib.load()
+    H, V = v.shape[1:]
+    G, K = q.shape[1:]
+    o = torch.empty_like(v)
+    fin = torch.empty((rg.B, H, K, V), dtype=g.dtype, device=v.device) if want_final else None
+    c_rg, c_side = rg.c_struct(), side.c_struct()
+    with _on(v.device):
+        prof = _profile_begin()
+        _lib.check(lib.rua_gdn_forward(v.data_ptr(), q.data_ptr(), k.data_ptr(), g.data_ptr(), beta.data_ptr(), _ptr(h0),
+                                       o.data_ptr(), _ptr(fin), H, G, K, V, scale, _DTYPES[v.dtype], int(reverse),
+                                       ctypes.byref(c_rg), ctypes.byref(c_side), None, 0, _stream()), 'rua_gdn_forward')
+        if prof is not None:
+            # v and o once, g and beta once, q and k once per value head block
+            nb = 2 * v.numel() * v.element_size() + g.numel() * g.element_size() + beta.numel() * beta.element_size() + \
+                2 * q.numel() * q.element_size() * (H // G) * ((V + 63) // 64)
+            _profile_end(prof, 'gdn_forward', nb + 8 * rg.B + (8 * (rg.Tp + rg.B) if side.layout == PACK else 0))
+    return o, fin
+
+
+def _gdn_backward_raw(go: Tensor, v: Tensor, q: Tensor, k: Tensor, g: Tensor, beta: Tensor, h0: Optional[Tensor],
+                      scale: float, rg: Ragged, side: SideSpec, reverse: bool, want):
+    """(grad_v, grad_q, grad_k, grad_g, grad_beta, grad_initial), None where ``want`` is False; inputs contiguous."""
+    lib = _lib.load()
+    H, V = v.shape[1:]
+    G, K = q.shape[1:]
+    dt = _DTYPES[v.dtype]
+    outs = (torch.empty_like(v) if want[0] else None, torch.empty_like(q) if want[1] else None,
+            torch.empty_like(k) if want[2] else None, torch.empty_like(g) if want[3] else None,
+            torch.empty_like(beta) if want[4] else None,
+            torch.empty((rg.B, H, K, V), dtype=g.dtype, device=v.device) if want[5] else None)
+    if not any(want):
+        return outs
+    c_rg, c_side = rg.c_struct(), side.c_struct()
+    with _on(v.device):
+        nbytes = lib.rua_gdn_workspace_bytes(side.rows, rg.B, rg.Tp, H, G, K, V, dt)
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=v.device)
+        prof = _profile_begin()
+        _lib.check(lib.rua_gdn_backward(go.data_ptr(), v.data_ptr(), q.data_ptr(), k.data_ptr(), g.data_ptr(),
+                                        beta.data_ptr(), _ptr(h0), *(_ptr(t) for t in outs), H, G, K, V, scale, dt,
+                                        int(reverse), ctypes.byref(c_rg), ctypes.byref(c_side),
+                                        ws.data_ptr() if nbytes else None, nbytes, _stream()), 'rua_gdn_backward')
+        if prof is not None:
+            # v and grad_out twice (recompute + reverse sweep), q and k three times per head block, the gradients once
+            e = v.element_size()
+            nb = v.numel() * e * (4 + want[0]) + q.numel() * e * (6 * (H // G) * ((V + 63) // 64) + want[1] + want[2])
+            _profile_end(prof, 'gdn_backward', nb + 8 * rg.B + (8 * (rg.Tp + rg.B) if side.layout == PACK else 0))
+    return outs
+
+
+class _GDN(torch.autograd.Function):
+    """(o, final or None); final is not differentiable.  Saves only its inputs: the backward recomputes the states.
+    Once-differentiable: the backward is a native kernel, double backward is not supported."""
+
+    @staticmethod
+    def forward(ctx, v: Tensor, q: Tensor, k: Tensor, g: Tensor, beta: Tensor, h0: Optional[Tensor], scale: float,
+                rg: Ragged, side: SideSpec, reverse: bool, want_final: bool):
+        vs, qs, ks, gs, bs = (t.detach().contiguous() for t in (v, q, k, g, beta))
+        hs = None if h0 is None else h0.detach().contiguous()
+        o, fin = _gdn_forward_raw(vs, qs, ks, gs, bs, hs, scale, rg, side, reverse, want_final)
+        if fin is not None:
+            ctx.mark_non_differentiable(fin)
+        ctx.meta = (scale, rg, side, reverse, h0 is not None)
+        ctx.save_for_backward(vs, qs, ks, gs, bs, hs)
+        return o, fin
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_o: Optional[Tensor], grad_fin: Optional[Tensor]):
+        scale, rg, side, reverse, has_h0 = ctx.meta
+        v, q, k, g, beta, h0 = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        want = (need[0], need[1], need[2], need[3], need[4], need[5] and has_h0)
+        go = grad_o.contiguous() if grad_o is not None else torch.zeros_like(v)
+        return (*_gdn_backward_raw(go, v, q, k, g, beta, h0, scale, rg, side, reverse, want),
+                None, None, None, None, None)
+
+
+def gdn(data: Tensor, q: Tensor, k: Tensor, g: Tensor, beta: Tensor, initial: Optional[Tensor], scale: float,
+        rg: Ragged, side: SideSpec, reverse: bool, want_final: bool) -> Tuple[Tensor, Optional[Tensor]]:
+    """(o like data, final (B, H, K, V) or None) of the gated delta rule over the flattened storage: data (side.rows, H,
+    V), q, k (side.rows, G, K), g, beta (side.rows, H), initial (B, H, K, V) or None; checked by the caller (gdn_check);
+    ``rg`` has its pack side."""
+    args = (data, q, k, g, beta, initial)
+    grad = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in args)
+    if grad:
+        return _GDN.apply(*args, scale, rg, side, reverse, want_final)
+    return _gdn_forward_raw(*(None if t is None else t.contiguous() for t in args), scale, rg, side, reverse, want_final)
+
+
+# ------------------------------------------------------------------------------------------------
 # scatter_*: stable sort of the index + bucket boundaries + segment reduce over GATHERED rows
 # ------------------------------------------------------------------------------------------------
 def sort_keys(keys: Tensor, max_key: int) -> Tuple[Tensor, Tensor]:
